@@ -61,7 +61,17 @@ def parse_args():
                     help="table = BASELINE configs[1] (headline); single_doc = configs[2]: SA+LCP+annotation build "
                          "throughput of ONE document of --doc-bytes (use 200000000), replicas only for N>1")
     ap.add_argument("--cpu-sample-docs", type=int, default=0, help="0 = 2 documents per host core (max 64)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the score table of the last "
+                    "device-timed step to DIR/scores.npy (float64; a seeded sample of its rows, listed in "
+                    "DIR/scores_rows.npy, when the table exceeds 64 MB), so that two builds can be compared output "
+                    "for output on identical inputs.  Headline workload only (--workload table, --impl b200): the "
+                    "reference arm's subprocess returns timings and a checksum, not the table")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.workload != "table"):
+        ap.error("--dump-outputs writes the table of --workload table with --impl b200")
+    return args
 
 
 def apply_env_options(_capi):
@@ -108,6 +118,23 @@ def oracle_check(sample, kp_codes, kp_off, normalized):
         out = subprocess.check_output([sys.executable, os.path.join(ROOT, "oracle", "check_rows.py"), path],
                                       stderr=subprocess.DEVNULL, timeout=1500)
     return json.loads(out.decode().strip().splitlines()[-1])
+
+
+DUMP_BYTES = 64 * 10**6 - 4096   # everything --dump-outputs writes, .npy headers included, stays within 64 MB
+
+
+def dump_table(out_dir, name, table):
+    """out_dir/<name>.npy = table (float64 [rows, cols]).  A table larger than DUMP_BYTES is replaced by the rows of a
+    fixed seeded sample, in increasing order, whose row numbers go to out_dir/<name>_rows.npy (float64)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    table = np.ascontiguousarray(table, dtype=np.float64)
+    if table.nbytes > DUMP_BYTES:
+        keep = max(1, DUMP_BYTES // (table.shape[1] * 8 + 8))
+        rows = np.sort(np.random.default_rng(0).choice(table.shape[0], size=keep, replace=False))
+        np.save(os.path.join(out_dir, name + "_rows.npy"), rows.astype(np.float64))
+        table = table[rows]
+    np.save(os.path.join(out_dir, name + ".npy"), table)
 
 
 def cpu_sample_size(args):
@@ -439,6 +466,10 @@ def run_b200(args):
     e1.record(stream)
     barrier()
     sampler.sample()
+    if args.dump_outputs:
+        if rank == 0:   # the [N * D, K] table as a caller of the last timed step receives it
+            dump_table(args.dump_outputs, "scores", (gathered if world > 1 else out_dev).view(-1, K).cpu().numpy())
+        barrier()       # the next pass's kernels of the other ranks store rows into rank 0's table: not before the copy
     launches = _capi.launch_count()
     kstats = _capi.kernel_stats()
     _capi.set_option("time_kernels", 0)

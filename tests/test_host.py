@@ -166,6 +166,28 @@ def test_narrow_packing_and_batch_planning():
     assert not ok("café") and not ok("x²") and not ok("中文") and not ok("Ѡ")
 
 
+def test_bench_dump_outputs_writes_the_table_or_a_fixed_sample(tmp_path, monkeypatch):
+    import importlib.util
+    spec = importlib.util.spec_from_file_location("bench_for_test", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    table = np.random.default_rng(3).random((50, 7))
+    bench.dump_table(str(tmp_path / "full"), "scores", table)
+    assert os.listdir(str(tmp_path / "full")) == ["scores.npy"]
+    got = np.load(str(tmp_path / "full" / "scores.npy"))
+    assert got.dtype == np.float64 and np.array_equal(got, table)
+    monkeypatch.setattr(bench, "DUMP_BYTES", 20 * (7 * 8 + 8))   # room for 20 rows and their row numbers
+    samples = []
+    for run in ("a", "b"):
+        bench.dump_table(str(tmp_path / run), "scores", table)
+        rows = np.load(str(tmp_path / run / "scores_rows.npy"))
+        got = np.load(str(tmp_path / run / "scores.npy"))
+        assert rows.dtype == got.dtype == np.float64 and got.shape == (20, 7)
+        assert np.all(np.diff(rows) > 0) and np.array_equal(got, table[rows.astype(np.int64)])
+        samples.append(rows)
+    assert np.array_equal(samples[0], samples[1])
+
+
 def test_graph_from_cooccurrence_matches_the_reference_graphs(golden):
     # the graph assembly (applications.py:115-149) from exact co-occurrence counts computed on the host from the golden table
     from east import applications
