@@ -1081,8 +1081,11 @@ static void score_enqueue(const east_index *idx, const KpPrepared *kp, const uin
                           int normalized, double *out_dev, int32_t doc_begin, int32_t doc_count, cudaStream_t s,
                           double *tmp, int32_t tile_docs, unsigned long long *probe_count,
                           double *const *peer_rows = nullptr /* sharded table: rows of document doc_begin in the peers' tables */,
-                          int32_t n_peers = 0) {
+                          int32_t n_peers = 0,
+                          const int32_t *group_off_dev = nullptr /* synonym-expanded scoring: G + 1 offsets of the variant groups */,
+                          int32_t G = 0) {
     ensure_suffix_keys(idx, s);
+    const int32_t cols = group_off_dev ? G : K;   // columns of out_dev
     ScoreInput in;
     in.text = idx->text; in.sa = idx->sa;
     in.doc_off = idx->d_doc_off + doc_begin; in.doc_m = idx->d_doc_m + doc_begin; in.n_docs = doc_count;
@@ -1096,6 +1099,7 @@ static void score_enqueue(const east_index *idx, const KpPrepared *kp, const uin
     }
     in.algorithmic_bytes = (double)get_option("score_bytes", 0);
     in.probe_count = probe_count;
+    in.group_off = group_off_dev; in.G = G;
     auto tile = [&](int32_t d0, int32_t cnt) {
         ScoreInput part = in;
         part.n_docs = cnt;
@@ -1112,7 +1116,7 @@ static void score_enqueue(const east_index *idx, const KpPrepared *kp, const uin
     if (n_tiles <= 2 || tile_docs < 2 || probe_count || get_option("score_no_overlap", 0)) {
         for (int32_t d0 = 0; d0 < doc_count; d0 += tile_docs) {
             const ScoreInput part = tile(d0, std::min(tile_docs, doc_count - d0));
-            score_table(part, tmp, out_dev + (size_t)d0 * K, s);
+            score_table(part, tmp, out_dev + (size_t)d0 * cols, s);
         }
         return;
     }
@@ -1135,7 +1139,7 @@ static void score_enqueue(const east_index *idx, const KpPrepared *kp, const uin
         score_suffixes(part, buf, s);
         EAST_CUDA(cudaEventRecord(walked[b], s));
         EAST_CUDA(cudaStreamWaitEvent(aux, walked[b], 0));
-        score_combine(part, buf, out_dev + (size_t)d0 * K, aux);
+        score_combine(part, buf, out_dev + (size_t)d0 * cols, aux);
         EAST_CUDA(cudaEventRecord(summed[b], aux));
     }
     for (int i = 0; i < 2; ++i) {
@@ -1149,7 +1153,9 @@ static void score_common(const east_index *idx, const uint32_t *kp_dev, const in
                          int normalized, double *out_dev, int32_t doc_begin, int32_t doc_count, cudaStream_t s,
                          double *suffix_out_dev /* optional: per-suffix results of the doc range */,
                          int64_t *probes_out = nullptr /* optional: run the probe-counting scorer */,
-                         const uint32_t *kp_host = nullptr /* optional: the same code points on the host */) {
+                         const uint32_t *kp_host = nullptr /* optional: the same code points on the host */,
+                         const int64_t *group_off = nullptr /* optional: the K queries are variants in G groups (host, G + 1) */,
+                         int32_t G = 0) {
     // per-suffix results wanted (return_suffix_scores): every suffix is its own "distinct" suffix
     const bool dedup = !suffix_out_dev && !get_option("score_no_dedup", 0);
     KpPrepared *kp = prepare_keyphrases(idx, kp_dev, kp_host, kp_off, K, dedup, s);
@@ -1166,6 +1172,12 @@ static void score_common(const east_index *idx, const uint32_t *kp_dev, const in
         tmp_own = DevBuf<double>((size_t)tile_docs * (size_t)n_uniq, s);
         tmp = tmp_own.p;
     }
+    DevBuf<int32_t> d_groups;
+    if (group_off) {   // < 2^31 variants: each has a code point of the keyphrase buffer (check_keyphrases)
+        const std::vector<int32_t> g32(group_off, group_off + G + 1);
+        d_groups = DevBuf<int32_t>((size_t)G + 1, s);
+        EAST_CUDA(cudaMemcpyAsync(d_groups.p, g32.data(), sizeof(int32_t) * ((size_t)G + 1), cudaMemcpyHostToDevice, s));
+    }
     DevBuf<unsigned long long> d_probes;
     if (probes_out) {
         d_probes = DevBuf<unsigned long long>(1, s);
@@ -1173,7 +1185,8 @@ static void score_common(const east_index *idx, const uint32_t *kp_dev, const in
     }
     StageTimer tm(s);
     tm.mark("score");
-    score_enqueue(idx, kp, kp_dev, total, K, normalized, out_dev, doc_begin, doc_count, s, tmp, tile_docs, d_probes.p);
+    score_enqueue(idx, kp, kp_dev, total, K, normalized, out_dev, doc_begin, doc_count, s, tmp, tile_docs, d_probes.p, nullptr, 0,
+                  d_groups.p, G);
     tm.finish();
     if (probes_out) {
         unsigned long long h = 0;
@@ -1210,6 +1223,49 @@ int east_score_probes_dev(const east_index *idx, const uint32_t *kp_dev, const i
     if (!idx || !kp_dev || !kp_off || !out_DxK_dev || !probes || K <= 0) throw Error(EAST_ERR_INVALID, "bad argument");
     EAST_CUDA(cudaSetDevice(idx->device));
     score_common(idx, kp_dev, kp_off, K, 1, out_DxK_dev, 0, idx->n_docs, (cudaStream_t)stream, nullptr, probes);
+    EAST_API_END
+}
+
+// synonym-expanded scoring: V variants in G groups, every group non-empty, the offsets ending at V
+static void check_groups(const int64_t *group_off, int32_t G, int32_t V) {
+    if (!group_off || G < 1) throw Error(EAST_ERR_INVALID, "no groups of variants");
+    if (group_off[0] != 0 || group_off[G] != V) throw Error(EAST_ERR_INVALID, "group offsets must run from 0 to the number of variants");
+    for (int32_t g = 0; g < G; ++g)
+        if (group_off[g + 1] <= group_off[g]) throw Error(EAST_ERR_INVALID, "empty group of variants");
+}
+
+static void check_groups_call(const east_index *idx, const int64_t *kp_off, int32_t V, const int64_t *group_off, int32_t G,
+                              int32_t doc_begin, int32_t doc_count) {
+    if (!idx || !kp_off || V <= 0) throw Error(EAST_ERR_INVALID, "bad argument");
+    if (doc_begin < 0 || doc_count <= 0 || (int64_t)doc_begin + doc_count > idx->n_docs) throw Error(EAST_ERR_INVALID, "bad document range");
+    check_groups(group_off, G, V);
+    check_keyphrases(kp_off, V);
+}
+
+int east_score_groups_dev(const east_index *idx, const uint32_t *kp_dev, const int64_t *kp_off, int32_t V,
+                          const int64_t *group_off, int32_t G, int32_t doc_begin, int32_t doc_count, double *out_dev,
+                          void *stream) {
+    EAST_API_BEGIN
+    check_groups_call(idx, kp_off, V, group_off, G, doc_begin, doc_count);
+    if (!kp_dev || !out_dev) throw Error(EAST_ERR_INVALID, "bad argument");
+    EAST_CUDA(cudaSetDevice(idx->device));
+    score_common(idx, kp_dev, kp_off, V, 1, out_dev, doc_begin, doc_count, (cudaStream_t)stream, nullptr, nullptr, nullptr,
+                 group_off, G);
+    EAST_API_END
+}
+
+int east_score_groups_host(const east_index *idx, const uint32_t *kp, const int64_t *kp_off, int32_t V,
+                           const int64_t *group_off, int32_t G, int32_t doc_begin, int32_t doc_count, double *out_host) {
+    EAST_API_BEGIN
+    check_groups_call(idx, kp_off, V, group_off, G, doc_begin, doc_count);
+    if (!kp || !out_host) throw Error(EAST_ERR_INVALID, "bad argument");
+    EAST_CUDA(cudaSetDevice(idx->device));
+    cudaStream_t s = 0;
+    DevBuf<uint32_t> d_kp((size_t)kp_off[V], s);
+    DevBuf<double> d_out((size_t)doc_count * G, s);
+    EAST_CUDA(cudaMemcpyAsync(d_kp.p, kp, sizeof(uint32_t) * (size_t)kp_off[V], cudaMemcpyHostToDevice, s));
+    score_common(idx, d_kp.p, kp_off, V, 1, d_out.p, doc_begin, doc_count, s, nullptr, nullptr, kp, group_off, G);
+    EAST_CUDA(cudaMemcpy(out_host, d_out.p, sizeof(double) * (size_t)doc_count * G, cudaMemcpyDeviceToHost));
     EAST_API_END
 }
 

@@ -196,8 +196,13 @@ struct ScoreInput {
     // memory, same offset as out_DxK): the all-gather of the batched scorer path
     double *peer_out[DocScore::MAX_PEERS] = {};
     int32_t n_peers = 0;
+    // synonym-expanded scoring: the K queries are variants, grouped by group_off[G + 1] (device); the combine step then
+    // stores out[doc][g] = the best variant of group g (k_score_combine_max).  nullptr: one column per query.
+    const int32_t *group_off = nullptr;
+    int32_t G = 0;
 };
 // the second half of score_table alone: tmp[doc][distinct suffix] (here: written by the per-document kernel) -> out[doc][k]
+// (out[doc][g] with groups)
 void score_combine(const ScoreInput &in, const double *suffix_tmp, double *out_DxK, cudaStream_t s);
 void score_table(const ScoreInput &in, double *suffix_tmp /*n_docs x n_uniq*/, double *out_DxK,
                  cudaStream_t s);

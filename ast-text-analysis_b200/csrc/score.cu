@@ -14,6 +14,7 @@
 //
 //   k_score_suffixes  one thread per (document, query suffix)   -> tmp[doc][suffix]
 //   k_score_combine   one thread per (document, keyphrase)      -> out[doc][k] = (sum in suffix order) / len
+//   k_score_combine_max  one thread per (document, group of variants) -> out[doc][g] = best variant of the group
 #include "sa_build.h"
 #include "score_walk.cuh"
 
@@ -77,6 +78,31 @@ k_score_combine(ScoreInput in, const double *__restrict__ tmp, double *__restric
     if (in.n_peers > 0) __threadfence_system();
 }
 
+// One thread per (document, group of variants) -- the synonym substitutions of one keyphrase (easa.py:27-34): every
+// variant's score is taken as k_score_combine takes it (suffix results in suffix order, divided by the variant's
+// length) and the best of the group is stored, so the document x variant table never exists.  The maximum starts from
+// the first variant's score: scores are >= 0 and never NaN, so it is one of the scores, bit for bit.
+__global__ void __launch_bounds__(SC_THREADS)
+k_score_combine_max(ScoreInput in, const double *__restrict__ tmp, double *__restrict__ out) {
+    const int64_t total = (int64_t)in.n_docs * in.G;
+    const int64_t stride = (int64_t)gridDim.x * SC_THREADS;
+    for (int64_t idx = (int64_t)blockIdx.x * SC_THREADS + threadIdx.x; idx < total; idx += stride) {
+        const int32_t doc = (int32_t)(idx / in.G);
+        const int32_t g = (int32_t)(idx - (int64_t)doc * in.G);
+        const int32_t v0 = __ldg(in.group_off + g), v1 = __ldg(in.group_off + g + 1);
+        const double *row = tmp + (int64_t)doc * in.n_uniq;
+        double best = 0.0;
+        for (int32_t v = v0; v < v1; ++v) {
+            const int32_t b = __ldg(in.kp_off + v), e = __ldg(in.kp_off + v + 1);
+            double result = 0.0;
+            for (int32_t s = b; s < e; ++s) result = result + row[__ldg(in.uniq_of + s)];
+            const double score = result / (double)(e - b);
+            if (v == v0 || score > best) best = score;
+        }
+        out[idx] = best;
+    }
+}
+
 __global__ void __launch_bounds__(256)
 k_fill_suffix_keys(const uint8_t *__restrict__ t8, const int32_t *__restrict__ sa, int32_t n, uint32_t *__restrict__ sk) {
     const int64_t stride = (int64_t)gridDim.x * blockDim.x;
@@ -92,6 +118,12 @@ void fill_suffix_keys(const uint8_t *t8, const int32_t *sa, int32_t n, uint32_t 
 }
 
 void score_combine(const ScoreInput &in, const double *suffix_tmp, double *out_DxK, cudaStream_t s) {
+    if (in.group_off) {
+        const int64_t cells = (int64_t)in.n_docs * in.G;
+        if (cells > 0)
+            EAST_LAUNCH(k_score_combine_max, grid_for(cells, SC_THREADS, 64), SC_THREADS, 0, s, in, suffix_tmp, out_DxK);
+        return;
+    }
     const int64_t cells = (int64_t)in.n_docs * in.K;
     if (cells > 0)
         EAST_LAUNCH(k_score_combine, grid_for(cells, SC_THREADS, 64), SC_THREADS, 0, s, in, suffix_tmp, out_DxK);

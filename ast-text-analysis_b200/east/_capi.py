@@ -34,6 +34,7 @@ EXPORTED_SYMBOLS = [
     "east_cooc_host", "east_last_timings", "east_launch_count", "east_set_option", "east_kernel_stats",
     "east_score_probes_dev", "east_index_stat", "east_score_range_dev", "east_table_host", "east_table_dev",
     "east_build_host_u8", "east_table_host_u8", "east_table_dev_gather", "east_trim", "east_table_host_gather", "east_index_save", "east_index_load", "east_texts_to_packed_host", "east_table_texts_host",
+    "east_score_groups_host", "east_score_groups_dev",
 ]
 
 _lib = None
@@ -88,6 +89,10 @@ def load():
     L.east_table_texts_host.argtypes = [_u8p, _i64p, ctypes.c_int32, ctypes.c_int, _u32p, _i64p, ctypes.c_int32, ctypes.c_int, _f64p,
                                         _i64p, _i32p, ctypes.POINTER(_vp)]
     L.east_score_range_dev.argtypes = [_vp, _vp, _i64p, ctypes.c_int32, ctypes.c_int, ctypes.c_int32, ctypes.c_int32, _vp, _vp]
+    L.east_score_groups_host.argtypes = [_vp, _u32p, _i64p, ctypes.c_int32, _i64p, ctypes.c_int32, ctypes.c_int32,
+                                         ctypes.c_int32, _f64p]
+    L.east_score_groups_dev.argtypes = [_vp, _vp, _i64p, ctypes.c_int32, _i64p, ctypes.c_int32, ctypes.c_int32,
+                                        ctypes.c_int32, _vp, _vp]
     L.east_score_probes_dev.argtypes = [_vp, _vp, _i64p, ctypes.c_int32, _vp, _vp, _i64p]
     L.east_score_one.argtypes = [_vp, ctypes.c_int32, _u32p, ctypes.c_int32, ctypes.c_int, _f64p, _f64p]
     L.east_cooc_dev.argtypes = [_vp, ctypes.c_int64, ctypes.c_int32, ctypes.c_double, _vp, ctypes.c_int, _vp]
@@ -171,6 +176,25 @@ def pack_keyphrases(queries):
     if codes.size != off[-1]:
         raise ValueError("keyphrases contain lone surrogates")
     return codes, off
+
+
+def pack_variant_groups(queries, synonyms):
+    """Synonym-expanded queries -> (uint32 codes, int64 variant offsets [V + 1], int64 group offsets [len(queries) + 1]):
+    the variants of query k (utils.synonym_variants) are variants group_off[k] .. group_off[k + 1] - 1, packed as they
+    are -- the reference scores them with _score, which does not strip spaces (easa.py:34)."""
+    from east import utils
+    from east.asts.utils import codepoints
+    variants = []
+    group_off = np.zeros(len(queries) + 1, dtype=np.int64)
+    for k, q in enumerate(queries):
+        variants.extend(utils.synonym_variants(q, synonyms))
+        group_off[k + 1] = len(variants)
+    off = np.zeros(len(variants) + 1, dtype=np.int64)
+    np.cumsum([len(v) for v in variants], out=off[1:])
+    codes = np.ascontiguousarray(codepoints("".join(variants)), dtype=np.uint32)
+    if codes.size != off[-1]:
+        raise ValueError("synonym variants contain lone surrogates")
+    return codes, off, group_off
 
 
 def concat_utf8(texts):
@@ -461,6 +485,36 @@ class DeviceIndex(object):
         kp_off = np.ascontiguousarray(kp_off, dtype=np.int64)
         _check(load().east_score_range_dev(self._h, _vp(kp_devptr), _ptr(kp_off, _i64p), len(kp_off) - 1,
                                            1 if normalized else 0, int(doc_begin), int(doc_count), _vp(out_devptr), _vp(stream)))
+        self.score_timings = last_timings()
+
+    def score_groups(self, kp_codes, kp_off, group_off, doc_begin=0, doc_count=None):
+        """Synonym-expanded scores (pack_variant_groups) of documents [doc_begin, doc_begin + doc_count): float64
+        [doc_count, G], the best normalized score over the variants of each group (east_score_groups_host)."""
+        kp_codes = np.ascontiguousarray(kp_codes, dtype=np.uint32)
+        kp_off = np.ascontiguousarray(kp_off, dtype=np.int64)
+        group_off = np.ascontiguousarray(group_off, dtype=np.int64)
+        if len(kp_off) and kp_codes.size < kp_off[-1]:
+            raise ValueError("variant offsets run past the code points")
+        if doc_count is None:
+            doc_count = self.n_docs - doc_begin
+        G = len(group_off) - 1
+        out = np.empty((max(int(doc_count), 0), max(G, 0)), dtype=np.float64)
+        if kp_codes.size == 0:
+            kp_codes = np.zeros(1, dtype=np.uint32)
+        _check(load().east_score_groups_host(self._h, _ptr(kp_codes, _u32p), _ptr(kp_off, _i64p), len(kp_off) - 1,
+                                             _ptr(group_off, _i64p), G, int(doc_begin), int(doc_count), _ptr(out, _f64p)))
+        self.score_timings = last_timings()
+        return out
+
+    def score_groups_dev(self, kp_devptr, kp_off, group_off, out_devptr, doc_begin=0, doc_count=None, stream=0):
+        """score_groups() with the code points and the [doc_count, G] table on the device (east_score_groups_dev)."""
+        kp_off = np.ascontiguousarray(kp_off, dtype=np.int64)
+        group_off = np.ascontiguousarray(group_off, dtype=np.int64)
+        if doc_count is None:
+            doc_count = self.n_docs - doc_begin
+        _check(load().east_score_groups_dev(self._h, _vp(kp_devptr), _ptr(kp_off, _i64p), len(kp_off) - 1,
+                                            _ptr(group_off, _i64p), len(group_off) - 1, int(doc_begin), int(doc_count),
+                                            _vp(out_devptr), _vp(stream)))
         self.score_timings = last_timings()
 
     def score_probes_dev(self, kp_devptr, kp_off, out_devptr, stream=0):

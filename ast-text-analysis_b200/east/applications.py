@@ -31,7 +31,10 @@ def _score_matrix(keyphrases, texts, similarity_measure, synonimizer, language):
         similarity_measure.set_text_collection(text_collection, language)
     if not kept or not text_titles:
         return kept, text_titles, np.zeros((len(text_titles), len(kept)))
-    if synonimizer is None and hasattr(similarity_measure, "relevance_table"):
+    if synonimizer is not None and isinstance(similarity_measure, relevance.ASTRelevanceMeasure):
+        # every synonym variant of every keyphrase in one grouped call per device batch
+        scores = similarity_measure.relevance_table(prepared, synonimizer)
+    elif synonimizer is None and hasattr(similarity_measure, "relevance_table"):
         scores = similarity_measure.relevance_table(prepared)
     else:
         scores = np.empty((len(text_titles), len(kept)), dtype=np.float64)

@@ -9,13 +9,10 @@ to numpy (int64, like the reference's np.int) on first access.
 Construction and scoring run in libeast_b200.so (hand-written sm_100a CUDA); there is no
 CPU implementation in this package.
 """
-import itertools
-
 import numpy as np
 
 from east import _capi
 from east import consts
-from east import utils as common_utils
 from east.asts import base
 from east.asts import utils
 
@@ -67,12 +64,10 @@ class EnhancedAnnotatedSuffixArray(base.AST):
     # ---- scoring (easa.py:26-36) ----
     def score(self, query, normalized=True, synonimizer=None, return_suffix_scores=False):
         if synonimizer:
-            # easa.py:27-34: best score over all synonym substitutions, always normalized
-            synonyms = synonimizer.get_synonyms()
-            query_words = common_utils.tokenize(query)
-            options = [synonyms[w] + [w] for w in query_words]
-            variants = ["".join(words) for words in itertools.product(*options)]
-            return max(self._score(q) for q in variants)
+            # easa.py:27-34: best score over all synonym substitutions, always normalized -- one grouped engine call
+            codes, off, group_off = _capi.pack_variant_groups([query], synonimizer.get_synonyms())
+            result = self._index.score_groups(codes, off, group_off, doc_begin=self._doc, doc_count=1)[0, 0]
+            return np.float64(result) if result != 0 else 0  # the reference's max keeps _score's int 0
         return self._score(query.replace(" ", ""), normalized, return_suffix_scores)
 
     def _score(self, query, normalized=True, return_suffix_scores=False):

@@ -201,8 +201,19 @@ class ASTRelevanceMeasure(RelevanceMeasure):
     def relevance(self, keyphrase, text, synonimizer=None):
         return self.asts[text].score(keyphrase, normalized=self.normalized, synonimizer=synonimizer)
 
-    def relevance_table(self, prepared_keyphrases):
-        """Scores of every prepared keyphrase against every text: float64 [n_texts, K]."""
+    def relevance_table(self, prepared_keyphrases, synonimizer=None):
+        """Scores of every prepared keyphrase against every text: float64 [n_texts, K].  With a synonimizer, the best
+        score over the synonym substitutions of each keyphrase, always normalized (easa.py:27-34)."""
+        if synonimizer:
+            if self._index is None:
+                return np.array([[ast.score(kp, normalized=self.normalized, synonimizer=synonimizer)
+                                  for kp in prepared_keyphrases] for ast in self.asts], dtype=np.float64)
+            # expanded once; every device batch is one grouped call (the batches after the first reuse the preparation)
+            codes, off, group_off = _capi.pack_variant_groups(prepared_keyphrases, synonimizer.get_synonyms())
+            table = np.empty((len(self.asts), len(prepared_keyphrases)), dtype=np.float64)
+            for index, docs in self._batches:
+                table[docs] = index.score_groups(codes, off, group_off)
+            return table
         if self._index is None:
             return np.array([[ast.score(kp, normalized=self.normalized) for kp in prepared_keyphrases]
                              for ast in self.asts], dtype=np.float64)

@@ -26,6 +26,15 @@ def tokenize(text):
     return _TOKEN_RE.findall(text)
 
 
+def synonym_variants(query, synonyms):
+    """Every substitution of the words of `query` by their synonyms, as the reference scores them with a synonimizer
+    (east/asts/easa.py:27-33).  synonyms: the synonimizer's get_synonyms() mapping -- a word it lacks raises KeyError
+    unless it is a defaultdict.  Variants are not space-stripped (a synonym with a space keeps it); a query without
+    tokens has the single variant ""."""
+    options = [synonyms[w] + [w] for w in tokenize(query)]
+    return ["".join(words) for words in itertools.product(*options)]
+
+
 def tokenize_and_filter(text, min_word_length=3, stopwords=None):
     """east/utils.py:41-46 (stop-word list must be supplied; nltk is not a dependency here)."""
     stopwords = stopwords or set()

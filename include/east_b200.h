@@ -145,6 +145,21 @@ int east_table_host_gather(const void *text, int32_t text_width, const int64_t *
 int east_score_range_dev(const east_index *idx, const uint32_t *kp_dev, const int64_t *kp_off_host,
                          int32_t K, int normalized, int32_t doc_begin, int32_t doc_count,
                          double *out_dev, void *stream);
+/* synonym-expanded scoring (easa.py:27-34): V variants in kp/kp_off (NOT space-stripped), grouped by
+ * group_off[G+1] (host, int64, group_off[0] = 0, strictly increasing, group_off[G] = V); for documents
+ * [doc_begin, doc_begin + doc_count): out[(d - doc_begin) * G + g] = max over the group's variants of the
+ * normalized score.  Always normalized, as the reference's synonym branch.
+ * A group is every substitution of one keyphrase's words by their synonyms: the call walks each distinct query
+ * suffix of all variants once per document and keeps only the best variant of each group, so the document x
+ * variant table is never formed.  Malformed groups fail with EAST_ERR_INVALID, an empty variant with
+ * EAST_ERR_ZERODIV.  The _host entry takes host buffers; the _dev entry takes kp_dev and out_dev on the index's
+ * device (kp_off and group_off stay on the host). */
+int east_score_groups_host(const east_index *idx, const uint32_t *kp, const int64_t *kp_off, int32_t V,
+                           const int64_t *group_off, int32_t G, int32_t doc_begin, int32_t doc_count,
+                           double *out_host);
+int east_score_groups_dev(const east_index *idx, const uint32_t *kp_dev, const int64_t *kp_off, int32_t V,
+                          const int64_t *group_off, int32_t G, int32_t doc_begin, int32_t doc_count,
+                          double *out_dev, void *stream);
 /* same table through an instrumented scorer that also counts the algorithmic bytes it reads:
  * 8 per (SA word, text word) probe (SURVEY 8(d)); on the fast path 5 per (SA word, text byte)
  * probe and 8 per 2-gram bucket lookup.  *probes receives that byte count. */

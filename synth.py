@@ -57,6 +57,20 @@ def keyphrases(k, seed=7, v=V):
     return out
 
 
+def synonyms(prepared_keyphrases, seed=11, v=V):
+    """Seeded synonym dictionary of profiles/bench_synonyms.py: every distinct word of the (upper-cased) keyphrases,
+    in sorted order, gets rng.integers(0, 4) synonyms drawn from the same Zipf, upper-cased.  For keyphrases(1000):
+    9 277 variants, at most 64 per keyphrase."""
+    from east import utils
+    words, cdf, _ = vocabulary(v)
+    rng = np.random.default_rng(seed)
+    out = {}
+    for w in sorted({t for kp in prepared_keyphrases for t in utils.tokenize(kp)}):
+        ids = np.searchsorted(cdf, rng.random(int(rng.integers(0, 4))), side="right")
+        out[w] = [words[i].upper() for i in ids]
+    return out
+
+
 def packed_collection(n_docs, n_bytes, first_seed=1):
     """Documents run through the host preprocessing of the product package and packed:
     returns (list of uint32 arrays, list of m, list of strings collections)."""
