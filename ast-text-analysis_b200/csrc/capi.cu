@@ -1076,7 +1076,8 @@ static KpPrepared *prepare_keyphrases(const east_index *idx, const uint32_t *kp_
 }
 
 // The launches that score documents [doc_begin, doc_begin + doc_count) of `idx` (tile_docs at a time through the
-// scratch tmp[tile_docs][n_uniq]) into out_dev[(d - doc_begin) * K + k]; nothing here waits for the device.
+// scratch tmp[tile_docs][n_uniq]) into out_dev[(d - doc_begin) * K + k] (with groups: [(d - doc_begin) * G + g]);
+// nothing here waits for the device.
 static void score_enqueue(const east_index *idx, const KpPrepared *kp, const uint32_t *kp_dev, int64_t total, int32_t K,
                           int normalized, double *out_dev, int32_t doc_begin, int32_t doc_count, cudaStream_t s,
                           double *tmp, int32_t tile_docs, unsigned long long *probe_count,
@@ -1109,7 +1110,7 @@ static void score_enqueue(const east_index *idx, const KpPrepared *kp, const uin
         if (in.bkt3) part.bkt3 = in.bkt3 + ((size_t)d0 << (3 * in.sym_bits));
         part.algorithmic_bytes = in.algorithmic_bytes * ((double)part.n_docs / (double)doc_count);
         part.n_peers = n_peers;
-        for (int32_t pi = 0; pi < n_peers; ++pi) part.peer_out[pi] = peer_rows[pi] + (size_t)d0 * K;
+        for (int32_t pi = 0; pi < n_peers; ++pi) part.peer_out[pi] = peer_rows[pi] + (size_t)d0 * cols;
         return part;
     };
     const int32_t n_tiles = (doc_count + tile_docs - 1) / tile_docs;
@@ -1149,6 +1150,15 @@ static void score_enqueue(const east_index *idx, const KpPrepared *kp, const uin
     }
 }
 
+// the device copy of a call's group offsets (int32: < 2^31 variants, each has a code point of the keyphrase buffer --
+// check_keyphrases); the host vector may go once this returns (pageable source: staged before the call returns)
+static DevBuf<int32_t> upload_groups(const int64_t *group_off, int32_t G, cudaStream_t s) {
+    const std::vector<int32_t> g32(group_off, group_off + G + 1);
+    DevBuf<int32_t> d((size_t)G + 1, s);
+    EAST_CUDA(cudaMemcpyAsync(d.p, g32.data(), sizeof(int32_t) * ((size_t)G + 1), cudaMemcpyHostToDevice, s));
+    return d;
+}
+
 static void score_common(const east_index *idx, const uint32_t *kp_dev, const int64_t *kp_off, int32_t K,
                          int normalized, double *out_dev, int32_t doc_begin, int32_t doc_count, cudaStream_t s,
                          double *suffix_out_dev /* optional: per-suffix results of the doc range */,
@@ -1173,11 +1183,7 @@ static void score_common(const east_index *idx, const uint32_t *kp_dev, const in
         tmp = tmp_own.p;
     }
     DevBuf<int32_t> d_groups;
-    if (group_off) {   // < 2^31 variants: each has a code point of the keyphrase buffer (check_keyphrases)
-        const std::vector<int32_t> g32(group_off, group_off + G + 1);
-        d_groups = DevBuf<int32_t>((size_t)G + 1, s);
-        EAST_CUDA(cudaMemcpyAsync(d_groups.p, g32.data(), sizeof(int32_t) * ((size_t)G + 1), cudaMemcpyHostToDevice, s));
-    }
+    if (group_off) d_groups = upload_groups(group_off, G, s);
     DevBuf<unsigned long long> d_probes;
     if (probes_out) {
         d_probes = DevBuf<unsigned long long>(1, s);
@@ -1294,6 +1300,12 @@ struct TableRun {
     const int64_t *kp_off = nullptr;
     int32_t K = 0;
     int normalized = 0;
+    // synonym-expanded table: the K queries are variants in G groups (host offsets; d_groups: their device copy) and
+    // every row is G wide.  group_off NULL: one column per query.
+    const int64_t *group_off = nullptr;
+    int32_t G = 0;
+    DevBuf<int32_t> d_groups;
+    int32_t cols() const { return group_off ? G : K; }
     double *d_out = nullptr, *host_out = nullptr;   // host_out NULL: the table stays on the device
     double *const *peer_rows = nullptr;             // sharded table: where this rank's rows start in every other rank's table
     int32_t n_peers = 0;
@@ -1380,7 +1392,8 @@ static void table_run_begin(void *vctx, const RunReady &r, DocScore &score) {
         const int li = table_lane(t, r.stream);
         const int64_t n_uniq = std::max<int64_t>(1, t.kp->n_uniq);
         const int64_t budget = get_option("score_tmp_doubles", (int64_t)1 << 27);
-        const bool in_kernel = t.kp->fast && (int64_t)r.doc_count * n_uniq <= budget && !get_option("no_fused_score", 0);
+        const bool in_kernel = t.kp->fast && (int64_t)r.doc_count * n_uniq <= budget && !get_option("no_fused_score", 0) &&
+                               (!t.group_off || t.G <= DocScore::MAX_GROUPS);   // the groups' maxima fit the shared memory
         const int64_t want = in_kernel ? r.doc_count : std::max<int64_t>(1, std::min<int64_t>(r.doc_count, budget / n_uniq));
         if (t.tmp_docs[li] < want) {
             t.tmp[li] = DevBuf<double>((size_t)want * (size_t)n_uniq, r.stream);
@@ -1390,10 +1403,11 @@ static void table_run_begin(void *vctx, const RunReady &r, DocScore &score) {
             score.recs = t.kp->dev.d_recs.p; score.n_uniq = (int32_t)t.kp->n_uniq; score.q8 = t.kp->dev.d_q8.p; score.kp = t.d_kp;
             score.tmp = t.tmp[li].p; score.normalized = t.normalized ? 1 : 0;
             score.kp_off = t.kp->dev.d_off.p; score.uniq_of = t.kp->dev.d_uniq_of.p; score.K = t.K;
-            score.out = t.d_out + (size_t)r.doc_begin * t.K;
+            score.out = t.d_out + (size_t)r.doc_begin * t.cols();
+            if (t.group_off) { score.group_off = t.d_groups.p; score.G = t.G; }
             score.skip_suffix_keys = get_option("eager_suffix_keys", 0) ? 0 : 1;
             score.n_peers = t.n_peers;
-            for (int32_t pi = 0; pi < t.n_peers; ++pi) score.peer_out[pi] = t.peer_rows[pi] + (size_t)r.doc_begin * t.K;
+            for (int32_t pi = 0; pi < t.n_peers; ++pi) score.peer_out[pi] = t.peer_rows[pi] + (size_t)r.doc_begin * t.cols();
             score.algorithmic_bytes = (double)get_option("score_bytes", 0) * ((double)r.doc_count / (double)t.view.n_docs);
         }
     } catch (...) {
@@ -1408,16 +1422,17 @@ static void table_run_done(void *vctx, const RunReady &r, int in_kernel) {
     if (t.failed || !t.kp) return;
     try {
         const int li = table_lane(t, r.stream);
-        double *rows = t.d_out + (size_t)r.doc_begin * t.K;
+        const int32_t cols = t.cols();
+        double *rows = t.d_out + (size_t)r.doc_begin * cols;
         if (!in_kernel) {
             std::vector<double *> peers((size_t)t.n_peers);
-            for (int32_t pi = 0; pi < t.n_peers; ++pi) peers[(size_t)pi] = t.peer_rows[pi] + (size_t)r.doc_begin * t.K;
+            for (int32_t pi = 0; pi < t.n_peers; ++pi) peers[(size_t)pi] = t.peer_rows[pi] + (size_t)r.doc_begin * cols;
             score_enqueue(&t.view, t.kp, t.d_kp, t.kp_off[t.K], t.K, t.normalized, rows, r.doc_begin, r.doc_count, r.stream,
-                          t.tmp[li].p, (int32_t)t.tmp_docs[li], nullptr, peers.data(), t.n_peers);
+                          t.tmp[li].p, (int32_t)t.tmp_docs[li], nullptr, peers.data(), t.n_peers, t.d_groups.p, t.G);
         }
         t.docs_sent += r.doc_count;   // the rows reach the peers from the kernels that produce them, on either path
         if (t.host_out)
-            EAST_CUDA(cudaMemcpyAsync(t.host_out + (size_t)r.doc_begin * t.K, rows, sizeof(double) * (size_t)r.doc_count * t.K,
+            EAST_CUDA(cudaMemcpyAsync(t.host_out + (size_t)r.doc_begin * cols, rows, sizeof(double) * (size_t)r.doc_count * cols,
                                       cudaMemcpyDeviceToHost, r.stream));
         t.docs_scored += r.doc_count;
     } catch (...) {
@@ -1428,7 +1443,9 @@ static void table_run_done(void *vctx, const RunReady &r, int in_kernel) {
 static void table_host_impl(const void *text, int width, const int64_t *doc_off, const int32_t *doc_m, int32_t n_docs, int device,
                             const uint32_t *kp, const int64_t *kp_off, int32_t K, int normalized, double *out_DxK,
                             east_index **out_idx, double *own_rows_dev = nullptr, double *const *peer_rows = nullptr,
-                            int32_t n_peers = 0) {
+                            int32_t n_peers = 0,
+                            const int64_t *group_off = nullptr /* synonym-expanded table: G + 1 offsets of the variant groups */,
+                            int32_t G = 0) {
     if (!kp || !kp_off || !out_DxK || K <= 0) throw Error(EAST_ERR_INVALID, "bad argument");
     if (n_peers < 0 || n_peers > DocScore::MAX_PEERS || (n_peers > 0 && !peer_rows)) throw Error(EAST_ERR_INVALID, "bad peer list");
     east_index *built = nullptr;
@@ -1439,14 +1456,16 @@ static void table_host_impl(const void *text, int width, const int64_t *doc_off,
     // the keyphrases go first, on a side stream: hashing, ordering and de-duplication of their suffixes (kp_prep.cu)
     // run there while the text is on its way
     cudaStream_t ps = prep_stream(device);
+    const int32_t cols = group_off ? G : K;
     DevBuf<uint32_t> d_kp((size_t)kp_off[K], ps);
     DevBuf<double> d_out_own;
-    if (!own_rows_dev) d_out_own = DevBuf<double>((size_t)n_docs * K, s);
+    if (!own_rows_dev) d_out_own = DevBuf<double>((size_t)n_docs * cols, s);
     double *const d_out = own_rows_dev ? own_rows_dev : d_out_own.p;
     EAST_CUDA(cudaMemcpyAsync(d_kp.p, kp, sizeof(uint32_t) * (size_t)kp_off[K], cudaMemcpyHostToDevice, ps));
     TableRun run;
     run.kp_own = kp_begin(device, d_kp.p, kp, kp_off, K, !get_option("score_no_dedup", 0), false, ps, likely_code_table());
     run.kp_host = kp; run.d_kp = d_kp.p; run.kp_off = kp_off; run.K = K; run.normalized = normalized;
+    if (group_off) { run.group_off = group_off; run.G = G; run.d_groups = upload_groups(group_off, G, s); }
     run.d_out = d_out; run.host_out = out_DxK;
     run.peer_rows = peer_rows; run.n_peers = n_peers;
     RunHook hook;
@@ -1459,12 +1478,12 @@ static void table_host_impl(const void *text, int width, const int64_t *doc_off,
     const bool stands = !run.failed && run.docs_scored == n_docs &&
                         ((built->pipelined && !run.final_pass) || (built->doc_sorted && !built->pipelined && run.final_pass));
     if (!stands) {
-        score_common(built, d_kp.p, kp_off, K, normalized, d_out, 0, n_docs, s, nullptr, nullptr, kp);
-        EAST_CUDA(cudaMemcpyAsync(out_DxK, d_out, sizeof(double) * (size_t)n_docs * K, cudaMemcpyDeviceToHost, s));
+        score_common(built, d_kp.p, kp_off, K, normalized, d_out, 0, n_docs, s, nullptr, nullptr, kp, group_off, G);
+        EAST_CUDA(cudaMemcpyAsync(out_DxK, d_out, sizeof(double) * (size_t)n_docs * cols, cudaMemcpyDeviceToHost, s));
     }
     if (n_peers > 0 && !(stands && run.docs_sent == n_docs))   // rows (also) produced by the batched scorer: plain peer copies
         for (int32_t pi = 0; pi < n_peers; ++pi)
-            EAST_CUDA(cudaMemcpyAsync(peer_rows[pi], d_out, sizeof(double) * (size_t)n_docs * K, cudaMemcpyDefault, s));
+            EAST_CUDA(cudaMemcpyAsync(peer_rows[pi], d_out, sizeof(double) * (size_t)n_docs * cols, cudaMemcpyDefault, s));
     EAST_CUDA(cudaStreamSynchronize(s));
     if (out_idx) *out_idx = guard.release();
 }
@@ -1488,7 +1507,9 @@ int east_table_host_u8(const uint8_t *text8, const int64_t *doc_off, const int32
 static void table_dev_impl(const uint32_t *text_dev, const int64_t *doc_off, const int32_t *doc_m, int32_t n_docs, int device,
                            const uint32_t *kp_dev, const uint32_t *kp_host, const int64_t *kp_off, int32_t K, int normalized,
                            double *out_DxK_dev, double *const *peer_rows, int32_t n_peers, void *stream, east_index **out_idx,
-                           bool owns_text = false /* the index takes the text over (also when the call fails) */) {
+                           bool owns_text = false /* the index takes the text over (also when the call fails) */,
+                           const int64_t *group_off = nullptr /* synonym-expanded table: G + 1 offsets of the variant groups */,
+                           int32_t G = 0) {
     struct TextGuard {   // an owned text that never reached an index
         const uint32_t *p; bool armed;
         ~TextGuard() { if (armed && p) dev_free(const_cast<uint32_t *>(p), 0); }
@@ -1504,6 +1525,7 @@ static void table_dev_impl(const uint32_t *text_dev, const int64_t *doc_off, con
     // keyphrase preparation on a side stream, queued from the build once its alphabet scan is on its way
     run.device = device; run.dedup = !get_option("score_no_dedup", 0); run.kp_stream = prep_stream(device); run.caller_stream = s;
     run.kp_host = kp_host; run.d_kp = kp_dev; run.kp_off = kp_off; run.K = K; run.normalized = normalized;
+    if (group_off) { run.group_off = group_off; run.G = G; run.d_groups = upload_groups(group_off, G, s); }
     run.d_out = out_DxK_dev; run.host_out = nullptr;
     run.peer_rows = peer_rows; run.n_peers = n_peers;
     RunHook hook;
@@ -1514,11 +1536,12 @@ static void table_dev_impl(const uint32_t *text_dev, const int64_t *doc_off, con
     build_common(text_dev, owns_text, doc_off, doc_m, n_docs, device, s, &built, nullptr, &hook);
     std::unique_ptr<east_index, void (*)(east_index *)> guard(built, free_index);
     const bool stands = !run.failed && run.docs_scored == n_docs && built->doc_sorted && run.final_pass;
-    if (!stands) score_common(built, kp_dev, kp_off, K, normalized, out_DxK_dev, 0, n_docs, s, nullptr, nullptr, kp_host);
+    if (!stands)
+        score_common(built, kp_dev, kp_off, K, normalized, out_DxK_dev, 0, n_docs, s, nullptr, nullptr, kp_host, group_off, G);
     if (n_peers > 0 && !(stands && run.docs_sent == n_docs)) {
         // the rows were (also) produced by the batched scorer: plain peer copies of the slice
         for (int32_t pi = 0; pi < n_peers; ++pi)
-            EAST_CUDA(cudaMemcpyAsync(peer_rows[pi], out_DxK_dev, sizeof(double) * (size_t)n_docs * K, cudaMemcpyDefault, s));
+            EAST_CUDA(cudaMemcpyAsync(peer_rows[pi], out_DxK_dev, sizeof(double) * (size_t)n_docs * run.cols(), cudaMemcpyDefault, s));
     }
     EAST_CUDA(cudaStreamSynchronize(s));
     if (out_idx) *out_idx = guard.release();
@@ -1549,6 +1572,36 @@ int east_table_dev_gather(const uint32_t *text_dev, const int64_t *doc_off, cons
     EAST_API_BEGIN
     table_dev_impl(text_dev, doc_off, doc_m, n_docs, device, kp_dev, kp_host, kp_off, K, normalized, out_DxK_dev, peer_rows,
                    n_peers, stream, out_idx);
+    EAST_API_END
+}
+
+// ---- synonym-expanded tables in one call: the per-document kernel keeps the best variant of every group ------------
+// (arguments are checked before anything is built)
+static void check_table_groups(const int64_t *kp_off, int32_t V, const int64_t *group_off, int32_t G) {
+    if (!kp_off || V <= 0) throw Error(EAST_ERR_INVALID, "bad argument");
+    check_groups(group_off, G, V);
+    check_keyphrases(kp_off, V);
+}
+
+int east_table_groups_host(const void *text, int32_t text_width, const int64_t *doc_off, const int32_t *doc_m, int32_t n_docs,
+                           int device, const uint32_t *kp, const int64_t *kp_off, int32_t V, const int64_t *group_off, int32_t G,
+                           double *out_DxG, east_index **out_idx) {
+    EAST_API_BEGIN
+    if (text_width != 1 && text_width != 4) throw Error(EAST_ERR_INVALID, "text_width must be 1 or 4");
+    check_table_groups(kp_off, V, group_off, G);
+    table_host_impl(text, text_width, doc_off, doc_m, n_docs, device, kp, kp_off, V, 1, out_DxG, out_idx, nullptr, nullptr, 0,
+                    group_off, G);
+    EAST_API_END
+}
+
+int east_table_groups_dev(const uint32_t *text_dev, const int64_t *doc_off, const int32_t *doc_m, int32_t n_docs, int device,
+                          const uint32_t *kp_dev, const uint32_t *kp_host, const int64_t *kp_off, int32_t V,
+                          const int64_t *group_off, int32_t G, double *out_DxG_dev, double *const *peer_rows, int32_t n_peers,
+                          void *stream, east_index **out_idx) {
+    EAST_API_BEGIN
+    check_table_groups(kp_off, V, group_off, G);
+    table_dev_impl(text_dev, doc_off, doc_m, n_docs, device, kp_dev, kp_host, kp_off, V, 1, out_DxG_dev, peer_rows, n_peers,
+                   stream, out_idx, false, group_off, G);
     EAST_API_END
 }
 
@@ -1657,12 +1710,12 @@ int east_texts_to_packed_host(const uint8_t *utf8, const int64_t *text_off, int3
     EAST_API_END
 }
 
-int east_table_texts_host(const uint8_t *utf8, const int64_t *text_off, int32_t n_texts, int device, const uint32_t *kp,
-                          const int64_t *kp_off, int32_t K, int normalized, double *out_DxK, int64_t *doc_off_out,
-                          int32_t *doc_m_out, east_index **out_idx) {
-    EAST_API_BEGIN
+static void table_texts_impl(const uint8_t *utf8, const int64_t *text_off, int32_t n_texts, int device, const uint32_t *kp,
+                             const int64_t *kp_off, int32_t K, int normalized, double *out_DxK, int64_t *doc_off_out,
+                             int32_t *doc_m_out, east_index **out_idx, const int64_t *group_off = nullptr, int32_t G = 0) {
     if (!kp || !kp_off || !out_DxK || K <= 0) throw Error(EAST_ERR_INVALID, "bad argument");
     check_keyphrases(kp_off, K);
+    const int32_t cols = group_off ? G : K;
     use_device(device);
     cudaStream_t s = 0;
     PackedTexts pt;
@@ -1670,13 +1723,29 @@ int east_table_texts_host(const uint8_t *utf8, const int64_t *text_off, int32_t 
     if (doc_off_out) std::copy(pt.doc_off.begin(), pt.doc_off.end(), doc_off_out);
     if (doc_m_out) std::copy(pt.doc_m.begin(), pt.doc_m.end(), doc_m_out);
     DevBuf<uint32_t> d_kp((size_t)kp_off[K], s);
-    DevBuf<double> d_out((size_t)n_texts * K, s);
+    DevBuf<double> d_out((size_t)n_texts * cols, s);
     EAST_CUDA(cudaMemcpyAsync(d_kp.p, kp, sizeof(uint32_t) * (size_t)kp_off[K], cudaMemcpyHostToDevice, s));
     const uint32_t *text = pt.text;
     pt.text = nullptr;   // the index owns it from here on
     table_dev_impl(text, pt.doc_off.data(), pt.doc_m.data(), n_texts, device, d_kp.p, kp, kp_off, K, normalized, d_out.p, nullptr, 0,
-                   (void *)s, out_idx, true);
-    EAST_CUDA(cudaMemcpy(out_DxK, d_out.p, sizeof(double) * (size_t)n_texts * K, cudaMemcpyDeviceToHost));
+                   (void *)s, out_idx, true, group_off, G);
+    EAST_CUDA(cudaMemcpy(out_DxK, d_out.p, sizeof(double) * (size_t)n_texts * cols, cudaMemcpyDeviceToHost));
+}
+
+int east_table_texts_host(const uint8_t *utf8, const int64_t *text_off, int32_t n_texts, int device, const uint32_t *kp,
+                          const int64_t *kp_off, int32_t K, int normalized, double *out_DxK, int64_t *doc_off_out,
+                          int32_t *doc_m_out, east_index **out_idx) {
+    EAST_API_BEGIN
+    table_texts_impl(utf8, text_off, n_texts, device, kp, kp_off, K, normalized, out_DxK, doc_off_out, doc_m_out, out_idx);
+    EAST_API_END
+}
+
+int east_table_texts_groups_host(const uint8_t *utf8, const int64_t *text_off, int32_t n_texts, int device, const uint32_t *kp,
+                                 const int64_t *kp_off, int32_t V, const int64_t *group_off, int32_t G, double *out_DxG,
+                                 int64_t *doc_off_out, int32_t *doc_m_out, east_index **out_idx) {
+    EAST_API_BEGIN
+    check_table_groups(kp_off, V, group_off, G);
+    table_texts_impl(utf8, text_off, n_texts, device, kp, kp_off, V, 1, out_DxG, doc_off_out, doc_m_out, out_idx, group_off, G);
     EAST_API_END
 }
 

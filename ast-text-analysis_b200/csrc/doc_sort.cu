@@ -37,7 +37,8 @@
 //      searches coincide)
 //   9  (optional: east_table_host / east_table_dev) score every distinct query suffix against the document
 //      (easa.py:91-139; walks of score_walk.cuh) from a copy of text + suffix array in the freed shared memory,
-//      then add the results up per keyphrase: the CTA writes its row of the score table.
+//      then add the results up per keyphrase: the CTA writes its row of the score table (k_doc_suffix_sort_groups: the
+//      best variant of each group of synonym variants).
 // A bucket of more than 4096 suffixes raises flag bit 0: the host redoes the batch with the global sort.  A
 // document the kernel gives up on gets empty bucket rows (and, for a bad layout, an in-range suffix array), so
 // that a caller that scores speculatively stays inside the arrays.
@@ -62,6 +63,7 @@ constexpr int DS_LIST_CAP = 2048;                   // >= 65535 / 33 buckets can
 constexpr int DS_WIN_BYTES = 64 * 8 + 64 * 4;       // per-warp window scratch: 64 keys + 64 positions
 constexpr int DS_INF = 0x7fffffff;
 static_assert(DS_WARPS * DS_WARP_BYTES <= DS_SCR_BYTES && DS_WARPS * DS_WIN_BYTES <= DS_SCR_BYTES, "scratch");
+static_assert(8 * DocScore::MAX_GROUPS <= DS_SCR_BYTES, "phase 9 keeps the groups' maxima in shared memory");
 
 struct DocSortParams {
     const uint8_t *t8;        // byte-coded text of the batch (n + 128 bytes allocated)
@@ -502,12 +504,41 @@ __device__ __forceinline__ void ds_clear_tables(const DocSortParams &p, int doc,
     }
 }
 
+// Phase 9 of a synonym-expanded table: the variants' sums are taken as for a plain row, one thread per VARIANT (groups
+// are 1-64 variants: a thread per group would leave most lanes idle), and each is folded into its group's maximum with
+// a 64-bit shared-memory atomicMax on the bits of the double.  Scores are >= +0.0 and never NaN, so their bit patterns
+// order as the values do and the maximum has the bits k_score_combine_max finds, whatever the order of the atomics.
+// `smem` (the staged text, no longer read) holds the G running maxima.
+__device__ __forceinline__ void ds_store_group_maxima(const DocSortParams &p, uint8_t *smem, int doc, const double *out, int tid) {
+    unsigned long long *s_best = reinterpret_cast<unsigned long long *>(smem);
+    const int32_t G = p.score.G;
+    for (int g = tid; g < G; g += DS_THREADS) s_best[g] = 0ull;
+    __syncthreads();
+    for (int v = tid; v < p.score.K; v += DS_THREADS) {
+        const int32_t sb = __ldg(p.score.kp_off + v), se = __ldg(p.score.kp_off + v + 1);
+        double result = 0.0;
+        for (int32_t x = sb; x < se; ++x) result = result + __ldcg(out + __ldg(p.score.uniq_of + x));
+        const double score = result / (double)(se - sb);
+        atomicMax(s_best + doc_of(p.score.group_off, G, v), (unsigned long long)__double_as_longlong(score));
+    }
+    __syncthreads();
+    double *table_row = p.score.out + (size_t)(doc - p.doc_begin) * (size_t)G;
+    for (int g = tid; g < G; g += DS_THREADS) {
+        const double v = __longlong_as_double((long long)s_best[g]);
+        table_row[g] = v;
+        const size_t cell = (size_t)(doc - p.doc_begin) * (size_t)G + (size_t)g;
+        for (int pi = 0; pi < p.score.n_peers; ++pi) p.score.peer_out[pi][cell] = v;
+    }
+    if (p.score.n_peers > 0) __threadfence_system();
+}
+
 // ---- phase 9 (optional): score the keyphrases against the document this CTA has just indexed
 // (EnhancedAnnotatedSuffixArray._score, easa.py:91-139, for every distinct query suffix; score_walk.cuh).
 // The CTA's shared memory is free again: the byte text and the suffix array (16-bit local positions) of the
 // document are staged there, so every probe of a walk -- the binary searches over (rank -> symbol at depth d)
 // -- is two shared-memory loads instead of dependent L2 / HBM round trips.  Only the bucket-table lookups that
 // open a walk (one batch of loads per suffix) and the suffix records go to global memory.
+template <bool GROUPS>
 __device__ __forceinline__ void ds_score_document(const DocSortParams &p, uint8_t *smem, int smem_bytes, int doc, int32_t base, int n, int tid) {
     if (p.score.recs == nullptr) return;
     __syncthreads();   // every rank of sa and every bucket start of this document is in place; shared memory is free
@@ -550,6 +581,10 @@ __device__ __forceinline__ void ds_score_document(const DocSortParams &p, uint8_
     // the keyphrase sums: the results of the keyphrase's suffixes IN SUFFIX ORDER (the reference's fp64 order,
     // easa.py:127-134), each fetched through the position of its distinct twin -- k_score_combine's arithmetic
     __syncthreads();
+    if (GROUPS) {
+        ds_store_group_maxima(p, smem, doc, out, tid);
+        return;
+    }
     double *table_row = p.score.out + (size_t)(doc - p.doc_begin) * (size_t)p.score.K;
     for (int k = tid; k < p.score.K; k += DS_THREADS) {
         const int32_t sb = __ldg(p.score.kp_off + k), se = __ldg(p.score.kp_off + k + 1);
@@ -565,8 +600,10 @@ __device__ __forceinline__ void ds_score_document(const DocSortParams &p, uint8_
     if (p.score.n_peers > 0) __threadfence_system();
 }
 
-__global__ void __launch_bounds__(DS_THREADS, 1)
-k_doc_suffix_sort(DocSortParams p) {
+// The per-document kernel; GROUPS: phase 9 writes synonym-expanded rows (G wide).  Two kernels instead of a kernel
+// template, so that the plain one keeps its name (kernel timings, profiles) and its register allocation.
+template <bool GROUPS>
+__device__ __forceinline__ void doc_suffix_sort(const DocSortParams &p) {
     extern __shared__ __align__(16) uint8_t ds_smem[];
     uint8_t *s_raw = ds_smem;                                                    // staged text
     uint32_t *s_scr = reinterpret_cast<uint32_t *>(ds_smem + p.text_cap);        // counters, later sort scratch
@@ -1013,7 +1050,7 @@ k_doc_suffix_sort(DocSortParams p) {
             __syncthreads();
             for (int r = tid; r < n; r += DS_THREADS) p.sk[base + r] = ds_lds4(s_raw, shift + (sa_doc[r] - base) + 2);
         }
-        ds_score_document(p, ds_smem, p.text_cap + DS_SCR_BYTES + 4 * p.bits_words + 2 * (int)sizeof(uint2) * DS_LIST_CAP, doc, base, n, tid);
+        ds_score_document<GROUPS>(p, ds_smem, p.text_cap + DS_SCR_BYTES + 4 * p.bits_words + 2 * (int)sizeof(uint2) * DS_LIST_CAP, doc, base, n, tid);
         return;
     }
 
@@ -1213,11 +1250,17 @@ k_doc_suffix_sort(DocSortParams p) {
     }
     if (p.phase_clk) __syncthreads();
     DS_STAMP(8);
-    ds_score_document(p, ds_smem, p.text_cap + DS_SCR_BYTES + 4 * p.bits_words + 2 * (int)sizeof(uint2) * DS_LIST_CAP, doc, base, n, tid);
+    ds_score_document<GROUPS>(p, ds_smem, p.text_cap + DS_SCR_BYTES + 4 * p.bits_words + 2 * (int)sizeof(uint2) * DS_LIST_CAP, doc, base, n, tid);
     if (p.phase_clk) __syncthreads();
     DS_STAMP(9);
 #undef DS_STAMP
 }
+
+__global__ void __launch_bounds__(DS_THREADS, 1)
+k_doc_suffix_sort(DocSortParams p) { doc_suffix_sort<false>(p); }
+
+__global__ void __launch_bounds__(DS_THREADS, 1)
+k_doc_suffix_sort_groups(DocSortParams p) { doc_suffix_sort<true>(p); }
 
 // Host side: can the batch take the per-document path, and with which parameters
 bool doc_sort_plan(int sigma, int32_t max_doc_n, DocSortPlan &plan) {
@@ -1247,7 +1290,8 @@ void doc_sort_launch(const DocSortPlan &plan, const uint8_t *t8, const uint32_t 
                      int64_t n_total, uint32_t term, int32_t *sa, uint32_t *bkt, uint32_t *bkt3, uint32_t *overflow, cudaStream_t s,
                      unsigned long long *phase_clk, const DocSortTables *tables, uint32_t *sk, const DocScore *score,
                      const uint8_t *code_table, uint32_t *miss, int64_t text_len, const uint8_t *text8) {
-    ensure_dynamic_smem((const void *)k_doc_suffix_sort, 220 * 1024);
+    const bool groups = score && score->recs && bkt && score->group_off;
+    ensure_dynamic_smem(groups ? (const void *)k_doc_suffix_sort_groups : (const void *)k_doc_suffix_sort, 220 * 1024);
     DocSortParams p;
     p.t8 = t8; p.text = text; p.doc_off = doc_off; p.doc_m = doc_m; p.sa = sa; p.bkt = bkt; p.bkt3 = (plan.G == 3) ? bkt3 : nullptr; p.overflow = overflow;
     p.b = plan.b; p.G = plan.G; p.S2 = plan.S2; p.term = term;
@@ -1269,7 +1313,8 @@ void doc_sort_launch(const DocSortPlan &plan, const uint8_t *t8, const uint32_t 
     // with the scorer inside, plus the bytes of its walks (counted by the
     // instrumented scorer, option score_bytes)
     EAST_BYTES(((p.lcp ? 25.0 : 5.0) + (p.code_table ? (p.text8 ? 5.0 : 4.0) : 0.0)) * (double)n_total + (p.score.recs ? p.score.algorithmic_bytes : 0.0));
-    EAST_LAUNCH(k_doc_suffix_sort, n_docs, DS_THREADS, plan.smem, s, p);
+    if (groups) EAST_LAUNCH(k_doc_suffix_sort_groups, n_docs, DS_THREADS, plan.smem, s, p);
+    else EAST_LAUNCH(k_doc_suffix_sort, n_docs, DS_THREADS, plan.smem, s, p);
 }
 
 }  // namespace east

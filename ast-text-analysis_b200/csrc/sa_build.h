@@ -20,6 +20,12 @@ struct DocScore {
     const int32_t *uniq_of = nullptr; // per suffix of the concatenated keyphrases: position of its distinct twin
     int32_t K = 0;
     double *out = nullptr;
+    // synonym-expanded table (k_doc_suffix_sort_groups): the K queries are variants grouped by group_off[G + 1] (device);
+    // the row is G wide, out[(document - doc_begin) * G + g] = the best variant of group g (k_score_combine_max's
+    // arithmetic).  The groups' running maxima live in the CTA's shared memory: at most MAX_GROUPS groups.
+    const int32_t *group_off = nullptr;
+    int32_t G = 0;
+    static constexpr int32_t MAX_GROUPS = 12288;
     // the all-gather of a documents-sharded table, fused: every row is also stored into the gathered tables of the other
     // ranks (their memory mapped into this process: NVLink peer stores), at the same row offset as `out`
     static constexpr int MAX_PEERS = 15;
@@ -193,7 +199,7 @@ struct ScoreInput {
     unsigned long long *probe_count = nullptr;  // device counter: run the probe-counting variant
     double algorithmic_bytes = 0.0;             // 8 B x probes of this workload, if known (roofline numerator)
     // sharded table: k_score_combine also stores every cell into the gathered tables of the other ranks (mapped peer
-    // memory, same offset as out_DxK): the all-gather of the batched scorer path
+    // memory, same offset as out_DxK): the all-gather of the batched scorer path (k_score_combine, k_score_combine_max)
     double *peer_out[DocScore::MAX_PEERS] = {};
     int32_t n_peers = 0;
     // synonym-expanded scoring: the K queries are variants, grouped by group_off[G + 1] (device); the combine step then

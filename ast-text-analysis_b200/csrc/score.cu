@@ -100,7 +100,9 @@ k_score_combine_max(ScoreInput in, const double *__restrict__ tmp, double *__res
             if (v == v0 || score > best) best = score;
         }
         out[idx] = best;
+        for (int pi = 0; pi < in.n_peers; ++pi) in.peer_out[pi][idx] = best;   // as k_score_combine: the fused all-gather
     }
+    if (in.n_peers > 0) __threadfence_system();
 }
 
 __global__ void __launch_bounds__(256)

@@ -35,6 +35,7 @@ EXPORTED_SYMBOLS = [
     "east_score_probes_dev", "east_index_stat", "east_score_range_dev", "east_table_host", "east_table_dev",
     "east_build_host_u8", "east_table_host_u8", "east_table_dev_gather", "east_trim", "east_table_host_gather", "east_index_save", "east_index_load", "east_texts_to_packed_host", "east_table_texts_host",
     "east_score_groups_host", "east_score_groups_dev",
+    "east_table_groups_host", "east_table_groups_dev", "east_table_texts_groups_host",
 ]
 
 _lib = None
@@ -93,6 +94,12 @@ def load():
                                          ctypes.c_int32, _f64p]
     L.east_score_groups_dev.argtypes = [_vp, _vp, _i64p, ctypes.c_int32, _i64p, ctypes.c_int32, ctypes.c_int32,
                                         ctypes.c_int32, _vp, _vp]
+    L.east_table_groups_host.argtypes = [_vp, ctypes.c_int32, _i64p, _i32p, ctypes.c_int32, ctypes.c_int, _u32p, _i64p,
+                                         ctypes.c_int32, _i64p, ctypes.c_int32, _f64p, ctypes.POINTER(_vp)]
+    L.east_table_groups_dev.argtypes = [_vp, _i64p, _i32p, ctypes.c_int32, ctypes.c_int, _vp, _u32p, _i64p, ctypes.c_int32,
+                                        _i64p, ctypes.c_int32, _vp, ctypes.POINTER(_vp), ctypes.c_int32, _vp, ctypes.POINTER(_vp)]
+    L.east_table_texts_groups_host.argtypes = [_u8p, _i64p, ctypes.c_int32, ctypes.c_int, _u32p, _i64p, ctypes.c_int32, _i64p,
+                                               ctypes.c_int32, _f64p, _i64p, _i32p, ctypes.POINTER(_vp)]
     L.east_score_probes_dev.argtypes = [_vp, _vp, _i64p, ctypes.c_int32, _vp, _vp, _i64p]
     L.east_score_one.argtypes = [_vp, ctypes.c_int32, _u32p, ctypes.c_int32, ctypes.c_int, _f64p, _f64p]
     L.east_cooc_dev.argtypes = [_vp, ctypes.c_int64, ctypes.c_int32, ctypes.c_double, _vp, ctypes.c_int, _vp]
@@ -197,6 +204,11 @@ def pack_variant_groups(queries, synonyms):
     return codes, off, group_off
 
 
+def _columns(K, group_off):
+    """Columns of a table: one per keyphrase, or one per group of synonym variants."""
+    return K if group_off is None else len(group_off) - 1
+
+
 def concat_utf8(texts):
     """list of str / bytes -> (uint8 buffer of the UTF-8 texts back to back, int64 offsets [n + 1])"""
     raws = [t if isinstance(t, (bytes, bytearray)) else t.encode("utf-8", errors="surrogatepass") for t in texts]
@@ -267,10 +279,12 @@ class DeviceIndex(object):
         return cls.from_handle(h, doc_off, doc_m, int(device))
 
     @classmethod
-    def table_from_texts(cls, texts, kp_codes, kp_off, out, normalized=True, device=0):
+    def table_from_texts(cls, texts, kp_codes, kp_off, out, normalized=True, device=0, group_off=None):
         """Raw texts in, score table out, in ONE engine call (east_table_texts_host): the texts are upper-cased,
         tokenised, grouped and packed on the device (tokenize.cu), indexed and scored.  texts: list of str / UTF-8
-        bytes (ASCII and Cyrillic; anything else raises UnsupportedText).  Returns the index."""
+        bytes (ASCII and Cyrillic; anything else raises UnsupportedText).  Returns the index.
+        group_off (pack_variant_groups): the keyphrases are synonym variants in G groups and `out` has G columns, the
+        best normalized variant of each group (east_table_texts_groups_host)."""
         L = load()
         # texts may also be (uint8 buffer, int64 offsets): texts already laid out back to back (e.g. in pinned memory)
         buf, off = texts if isinstance(texts, tuple) else concat_utf8(texts)
@@ -278,10 +292,16 @@ class DeviceIndex(object):
         kp_codes = np.ascontiguousarray(kp_codes, dtype=np.uint32)
         kp_off = np.ascontiguousarray(kp_off, dtype=np.int64)
         K = len(kp_off) - 1
-        assert out.dtype == np.float64 and out.flags["C_CONTIGUOUS"] and out.size == n * K
+        assert out.dtype == np.float64 and out.flags["C_CONTIGUOUS"] and out.size == n * _columns(K, group_off)
         doc_off = np.zeros(n + 1, dtype=np.int64)
         doc_m = np.zeros(n, dtype=np.int32)
         h = _vp()
+        if group_off is not None:
+            group_off = np.ascontiguousarray(group_off, dtype=np.int64)
+            _check(L.east_table_texts_groups_host(_ptr(buf, _u8p), _ptr(off, _i64p), n, int(device), _ptr(kp_codes, _u32p),
+                                                  _ptr(kp_off, _i64p), K, _ptr(group_off, _i64p), len(group_off) - 1,
+                                                  _ptr(out, _f64p), _ptr(doc_off, _i64p), _ptr(doc_m, _i32p), ctypes.byref(h)))
+            return cls.from_handle(h, doc_off, doc_m, int(device))
         _check(L.east_table_texts_host(_ptr(buf, _u8p), _ptr(off, _i64p), n, int(device), _ptr(kp_codes, _u32p),
                                        _ptr(kp_off, _i64p), K, 1 if normalized else 0, _ptr(out, _f64p),
                                        _ptr(doc_off, _i64p), _ptr(doc_m, _i32p), ctypes.byref(h)))
@@ -301,11 +321,13 @@ class DeviceIndex(object):
 
     @classmethod
     def build_host_and_score(cls, text, doc_off, doc_m, kp_codes, kp_off, out, normalized=True, device=0, own_rows=None,
-                             peer_rows=None):
+                             peer_rows=None, group_off=None):
         """build_host() + score_table_into() as ONE engine call (east_table_host): on a large batch of small
         documents the runs of documents already sorted are scored, and their rows of `out` copied back, while
         the rest of the text is still on its way to the device.  Returns the index; `out` ([n_docs, K] float64,
-        may be pinned) holds the table."""
+        may be pinned) holds the table.
+        group_off (pack_variant_groups): the keyphrases are synonym variants in G groups and `out` ([n_docs, G]) holds
+        the best normalized variant of each group (east_table_groups_host; not with own_rows / peer_rows)."""
         L = load()
         doc_off = np.ascontiguousarray(doc_off, dtype=np.int64)
         doc_m = np.ascontiguousarray(doc_m, dtype=np.int32)
@@ -313,8 +335,16 @@ class DeviceIndex(object):
         kp_off = np.ascontiguousarray(kp_off, dtype=np.int64)
         K = len(kp_off) - 1
         assert text.dtype in (np.uint32, np.uint8) and text.flags["C_CONTIGUOUS"]
-        assert out.dtype == np.float64 and out.flags["C_CONTIGUOUS"] and out.size == len(doc_m) * K
+        assert out.dtype == np.float64 and out.flags["C_CONTIGUOUS"] and out.size == len(doc_m) * _columns(K, group_off)
         h = _vp()
+        if group_off is not None:
+            if own_rows or peer_rows:
+                raise ValueError("a sharded synonym table is built from device-resident text (build_dev_and_score)")
+            group_off = np.ascontiguousarray(group_off, dtype=np.int64)
+            _check(L.east_table_groups_host(_vp(text.ctypes.data), int(text.itemsize), _ptr(doc_off, _i64p), _ptr(doc_m, _i32p),
+                                            len(doc_m), int(device), _ptr(kp_codes, _u32p), _ptr(kp_off, _i64p), K,
+                                            _ptr(group_off, _i64p), len(group_off) - 1, _ptr(out, _f64p), ctypes.byref(h)))
+            return cls.from_handle(h, doc_off, doc_m, int(device))
         if own_rows or peer_rows:   # sharded table: rows also to the gathered tables on the devices (east_table_host_gather)
             peer_rows = list(peer_rows or [])
             peers = (_vp * max(len(peer_rows), 1))(*[int(a) for a in peer_rows])
@@ -335,11 +365,13 @@ class DeviceIndex(object):
 
     @classmethod
     def build_dev_and_score(cls, text_devptr, doc_off, doc_m, kp_devptr, kp_codes, kp_off, out_devptr, normalized=True,
-                            device=0, stream=0, peer_rows=None):
+                            device=0, stream=0, peer_rows=None, group_off=None):
         """build_dev() + score_table_dev() as ONE engine call (east_table_dev): the per-document kernel scores every
         document right after indexing it.  kp_codes: host copy of the keyphrase code points (or None).
         peer_rows: device addresses in the OTHER ranks' gathered tables where this rank's rows start (mapped peer
-        memory): the kernel stores every row there too (east_table_dev_gather, the fused all-gather)."""
+        memory): the kernel stores every row there too (east_table_dev_gather, the fused all-gather).
+        group_off (pack_variant_groups): the keyphrases are synonym variants in G groups and the table has G columns,
+        the best normalized variant of each group (east_table_groups_dev, with or without peer_rows)."""
         L = load()
         doc_off = np.ascontiguousarray(doc_off, dtype=np.int64)
         doc_m = np.ascontiguousarray(doc_m, dtype=np.int32)
@@ -349,6 +381,15 @@ class DeviceIndex(object):
             kp_codes = np.ascontiguousarray(kp_codes, dtype=np.uint32)
             kp_host = _ptr(kp_codes, _u32p)
         h = _vp()
+        if group_off is not None:
+            group_off = np.ascontiguousarray(group_off, dtype=np.int64)
+            peer_rows = list(peer_rows or [])
+            peers = (_vp * max(len(peer_rows), 1))(*[int(a) for a in peer_rows])
+            _check(L.east_table_groups_dev(_vp(text_devptr), _ptr(doc_off, _i64p), _ptr(doc_m, _i32p), len(doc_m), int(device),
+                                           _vp(kp_devptr), kp_host, _ptr(kp_off, _i64p), len(kp_off) - 1,
+                                           _ptr(group_off, _i64p), len(group_off) - 1, _vp(out_devptr), peers, len(peer_rows),
+                                           _vp(stream), ctypes.byref(h)))
+            return cls.from_handle(h, doc_off, doc_m, int(device))
         if peer_rows:
             peers = (_vp * len(peer_rows))(*[int(a) for a in peer_rows])
             _check(L.east_table_dev_gather(_vp(text_devptr), _ptr(doc_off, _i64p), _ptr(doc_m, _i32p), len(doc_m), int(device),

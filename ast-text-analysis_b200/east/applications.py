@@ -24,15 +24,17 @@ def _score_matrix(keyphrases, texts, similarity_measure, synonimizer, language):
     text_collection = list(texts.values())
     kept = [kp for kp in keyphrases if kp]  # empty keyphrases are skipped (applications.py:44-45)
     prepared = [utils.prepare_text(kp) for kp in kept]
-    if synonimizer is None and isinstance(similarity_measure, relevance.ASTRelevanceMeasure) and prepared:
-        # the measure scores the keyphrases while it indexes the collection (one overlapped engine call)
-        similarity_measure.set_text_collection(text_collection, language, prepared_keyphrases=prepared)
+    if isinstance(similarity_measure, relevance.ASTRelevanceMeasure) and prepared:
+        # the measure scores the keyphrases -- with a synonimizer, their best synonym variants -- while it indexes the
+        # collection (one overlapped engine call)
+        similarity_measure.set_text_collection(text_collection, language, prepared_keyphrases=prepared,
+                                               synonimizer=synonimizer)
     else:
         similarity_measure.set_text_collection(text_collection, language)
     if not kept or not text_titles:
         return kept, text_titles, np.zeros((len(text_titles), len(kept)))
     if synonimizer is not None and isinstance(similarity_measure, relevance.ASTRelevanceMeasure):
-        # every synonym variant of every keyphrase in one grouped call per device batch
+        # the table scored while indexing (a grouped call per device batch for other indexes)
         scores = similarity_measure.relevance_table(prepared, synonimizer)
     elif synonimizer is None and hasattr(similarity_measure, "relevance_table"):
         scores = similarity_measure.relevance_table(prepared)

@@ -124,12 +124,14 @@ def _pack_local(texts):
 
 
 def relevance_table_sharded(texts, prepared_keyphrases, normalized=True, device=None, group=None, fused_gather=None,
-                            return_local=False):
+                            return_local=False, synonimizer=None):
     """[D, K] float64 score table of all texts x keyphrases, computed by all ranks together.
 
     texts: list of raw texts (same list on every rank).  Each rank preprocesses, packs, indexes and scores only
     its own range on its own GPU (east_table_dev: one engine call builds and scores a batch); returns the gathered
-    table as a torch tensor on that GPU (with return_local: also this rank's (begin, end) rows)."""
+    table as a torch tensor on that GPU (with return_local: also this rank's (begin, end) rows).
+    synonimizer: the synonym table of ASTRelevanceMeasure.relevance_table(prepared_keyphrases, synonimizer) -- the best
+    variant of each keyphrase, always normalized (east_table_groups_dev), with the same two ways to gather."""
     import torch
     import torch.distributed as dist
 
@@ -142,8 +144,12 @@ def relevance_table_sharded(texts, prepared_keyphrases, normalized=True, device=
     dev = torch.device("cuda", device)
     ranges = partition_documents([len(t) for t in texts], world)
     begin, end = ranges[rank]
-    codes, off = _capi.pack_keyphrases(prepared_keyphrases)
-    K = len(prepared_keyphrases)
+    group_off = None
+    if synonimizer:
+        codes, off, group_off = _capi.pack_variant_groups(prepared_keyphrases, synonimizer.get_synonyms())
+    else:
+        codes, off = _capi.pack_keyphrases(prepared_keyphrases)
+    K = len(prepared_keyphrases)   # columns: one per keyphrase (with synonyms: one per group of variants)
     D = len(texts)
     cols, packed, batches = _pack_local(texts[begin:end]) if end > begin else ([], [], [])
     # the fused gather writes the rows of ONE batch of consecutive documents; ragged collections (small and large
@@ -164,7 +170,7 @@ def relevance_table_sharded(texts, prepared_keyphrases, normalized=True, device=
         text_dev = torch.from_numpy(text.view(np.int32)).to(dev)
         _capi.DeviceIndex.build_dev_and_score(text_dev.data_ptr(), doc_off, [len(cols[j]) for j in docs], kp_dev.data_ptr(),
                                               codes, off, out_ptr, normalized, device=device, stream=stream.cuda_stream,
-                                              peer_rows=peer_rows).close()
+                                              peer_rows=peer_rows, group_off=group_off).close()
 
     table = None
     if fused:
@@ -218,18 +224,18 @@ def cooccurrence_sharded(local_scores, relevance_threshold, device=None, group=N
 
 
 def keyphrases_graph_sharded(keyphrases, texts, referral_confidence=0.6, relevance_threshold=0.25, support_threshold=1,
-                             normalized=True, device=None, group=None):
+                             normalized=True, device=None, group=None, synonimizer=None):
     """applications.keyphrases_graph computed by all ranks together: the same graph dict on every rank.
 
     texts: {name: text} (same on every rank); documents shard over the ranks, every rank scores its own and
-    counts its own co-occurrences; the K x K counts are all-reduced."""
+    counts its own co-occurrences; the K x K counts are all-reduced.  synonimizer: as in keyphrases_graph."""
     from east import applications
     from east import utils
     kept = [kp for kp in keyphrases if kp]
     prepared = [utils.prepare_text(kp) for kp in kept]
     text_collection = list(texts.values())
     full, (begin, end) = relevance_table_sharded(text_collection, prepared, normalized, device=device, group=group,
-                                                 return_local=True)
+                                                 return_local=True, synonimizer=synonimizer)
     cooc = cooccurrence_sharded(full[begin:end], relevance_threshold, device=device, group=group)
     return applications.graph_from_cooccurrence(keyphrases, kept, cooc.cpu().numpy(), referral_confidence,
                                                 relevance_threshold, support_threshold)

@@ -70,13 +70,17 @@ class ASTRelevanceMeasure(RelevanceMeasure):
         self._batches = []
         self._table = None
         self._table_keyphrases = None
+        self._table_groups = None
 
-    def set_text_collection(self, texts, language=consts.Language.ENGLISH, prepared_keyphrases=None):
+    def set_text_collection(self, texts, language=consts.Language.ENGLISH, prepared_keyphrases=None, synonimizer=None):
         """relevance.py:34-49: one AST per text; here all of them in one batched build.
 
         prepared_keyphrases (optional, what keyphrases_table passes): the keyphrases relevance_table() is
         going to be asked for.  Each batch is then built AND scored by one engine call, which overlaps the
-        scoring of the documents already indexed with the transfer of the rest (east_table_host)."""
+        scoring of the documents already indexed with the transfer of the rest (east_table_host).
+        synonimizer (optional, with prepared_keyphrases): the table scored while indexing is the synonym table of
+        relevance_table(prepared_keyphrases, synonimizer) -- the best variant of each keyphrase, always normalized
+        (east_table_groups_host / east_table_texts_groups_host)."""
         self.texts = texts
         self.language = language
         self.asts = []
@@ -84,6 +88,7 @@ class ASTRelevanceMeasure(RelevanceMeasure):
         self._batches = []
         self._table = None
         self._table_keyphrases = None
+        self._table_groups = None
         total_texts = len(texts)
         if self.ast_algorithm not in tuple(consts.ASTAlgorithm):
             # other registered engines (none ship in this package) go through the registry
@@ -95,14 +100,18 @@ class ASTRelevanceMeasure(RelevanceMeasure):
             return
         if not texts:
             return
-        if prepared_keyphrases and self.device_preprocessing and self._set_text_collection_on_device(texts, prepared_keyphrases):
+        # the synonym variants are expanded and packed once: the same arrays go to every device batch
+        groups = (_capi.pack_variant_groups(prepared_keyphrases, synonimizer.get_synonyms())
+                  if prepared_keyphrases and synonimizer else None)
+        if prepared_keyphrases and self.device_preprocessing and self._set_text_collection_on_device(texts, prepared_keyphrases,
+                                                                                                    groups):
             return
         collections = [utils.text_to_strings_collection(text) for text in texts]
         # one byte per code point where the text allows it (ASCII / Latin-1: a quarter of the bytes over the host link),
         # uint32 code points otherwise; both have one entry per code point + one per string
         packed = [asts_utils.pack_strings_collection_u8(c) for c in collections]
         packed = [p if p is not None else asts_utils.pack_strings_collection(c) for p, c in zip(packed, collections)]
-        fused = _capi.pack_keyphrases(prepared_keyphrases) if prepared_keyphrases else None
+        fused = (groups[:2] if groups else _capi.pack_keyphrases(prepared_keyphrases)) if prepared_keyphrases else None
         # everything is built into locals: a batch that raises leaves the measure empty, not half-initialised
         asts = [None] * len(collections)
         batches = []
@@ -121,20 +130,22 @@ class ASTRelevanceMeasure(RelevanceMeasure):
             else:
                 rows = np.empty((len(docs), len(prepared_keyphrases)), dtype=np.float64)
                 index = _capi.DeviceIndex.build_host_and_score(text, doc_off, doc_m, fused[0], fused[1], rows,
-                                                               normalized=self.normalized, device=self.device)
+                                                               normalized=self.normalized, device=self.device,
+                                                               group_off=groups[2] if groups else None)
                 table[docs] = rows
             batches.append((index, docs))
             for local, j in enumerate(docs):
                 asts[j] = easa.EnhancedAnnotatedSuffixArray(collections[j], _index=index, _doc=local)
         self.asts, self._batches, self._index = asts, batches, batches[0][0]
         if fused:
-            self._table, self._table_keyphrases = table, list(prepared_keyphrases)
+            self._table, self._table_keyphrases, self._table_groups = table, list(prepared_keyphrases), groups
 
-    def _set_text_collection_on_device(self, texts, prepared_keyphrases):
+    def _set_text_collection_on_device(self, texts, prepared_keyphrases, groups=None):
         """keyphrases_table for a collection of small ASCII / Cyrillic texts: ONE engine call takes the raw texts,
         does the preprocessing of utils.text_to_strings_collection on the device (csrc/tokenize.cu), indexes and scores
-        (east_table_texts_host).  Returns False when the collection needs the host preprocessing (other scripts --
-        Python's Unicode tables --, a text too large for the per-document kernel, several device batches)."""
+        (east_table_texts_host; with groups -- pack_variant_groups -- the synonym table, east_table_texts_groups_host).
+        Returns False when the collection needs the host preprocessing (other scripts -- Python's Unicode tables --, a
+        text too large for the per-document kernel, several device batches)."""
         total = 0
         for t in texts:
             if isinstance(t, (bytes, bytearray)):
@@ -150,17 +161,17 @@ class ASTRelevanceMeasure(RelevanceMeasure):
             total += size
         if total >= MAX_BATCH_CODE_POINTS:
             return False
-        fused = _capi.pack_keyphrases(prepared_keyphrases)
+        fused = groups[:2] if groups else _capi.pack_keyphrases(prepared_keyphrases)
         table = np.empty((len(texts), len(prepared_keyphrases)), dtype=np.float64)
         try:
             index = _capi.DeviceIndex.table_from_texts(texts, fused[0], fused[1], table, normalized=self.normalized,
-                                                       device=self.device)
+                                                       device=self.device, group_off=groups[2] if groups else None)
         except _capi.UnsupportedText:
             return False
         docs = list(range(len(texts)))
         self.asts = [easa.EnhancedAnnotatedSuffixArray(None, _index=index, _doc=j) for j in docs]
         self._batches, self._index = [(index, docs)], index
-        self._table, self._table_keyphrases = table, list(prepared_keyphrases)
+        self._table, self._table_keyphrases, self._table_groups = table, list(prepared_keyphrases), groups
         return True
 
     def save_index(self, directory):
@@ -210,6 +221,9 @@ class ASTRelevanceMeasure(RelevanceMeasure):
                                   for kp in prepared_keyphrases] for ast in self.asts], dtype=np.float64)
             # expanded once; every device batch is one grouped call (the batches after the first reuse the preparation)
             codes, off, group_off = _capi.pack_variant_groups(prepared_keyphrases, synonimizer.get_synonyms())
+            if (self._table_groups is not None and list(prepared_keyphrases) == self._table_keyphrases
+                    and all(np.array_equal(a, b) for a, b in zip((codes, off, group_off), self._table_groups))):
+                return self._table   # the same variants were scored while the collection was being indexed
             table = np.empty((len(self.asts), len(prepared_keyphrases)), dtype=np.float64)
             for index, docs in self._batches:
                 table[docs] = index.score_groups(codes, off, group_off)
@@ -217,7 +231,7 @@ class ASTRelevanceMeasure(RelevanceMeasure):
         if self._index is None:
             return np.array([[ast.score(kp, normalized=self.normalized) for kp in prepared_keyphrases]
                              for ast in self.asts], dtype=np.float64)
-        if self._table is not None and list(prepared_keyphrases) == self._table_keyphrases:
+        if self._table is not None and self._table_groups is None and list(prepared_keyphrases) == self._table_keyphrases:
             return self._table   # scored while the collection was being indexed
         codes, off = _capi.pack_keyphrases(prepared_keyphrases)
         if len(self._batches) == 1:

@@ -204,6 +204,32 @@ int east_table_texts_host(const uint8_t *utf8, const int64_t *text_off, int32_t 
                           const uint32_t *kp, const int64_t *kp_off, int32_t K, int normalized, double *out_DxK,
                           int64_t *doc_off_out /* optional */, int32_t *doc_m_out /* optional */, east_index **out_idx);
 
+/* ---- synonym-expanded tables in one call: build and score as the table entries above, with the queries of
+ * east_score_groups_* -- V variants in kp/kp_off (NOT space-stripped), grouped by group_off[G+1] (host, int64,
+ * group_off[0] = 0, strictly increasing, group_off[G] = V) -- and a table G wide: out[d * G + g] = max over the
+ * variants of group g of the normalized score of document d (always normalized, as the reference's synonym branch).
+ * The tables are bit-identical to the entry's build followed by east_score_groups_host on the index.  On a batch of
+ * small documents the per-document kernel keeps the best variant of every group itself (up to 12 288 groups), so the
+ * synonym table inherits the pipelined host build, the one-byte text and the fused all-gather of the plain entries;
+ * otherwise the batched scorer combines the groups after the build.  Groups and variants are checked before anything
+ * is built: malformed groups fail with EAST_ERR_INVALID, an empty variant with EAST_ERR_ZERODIV; a text outside
+ * ASCII / Cyrillic fails the _texts_ entry with EAST_ERR_UNSUPPORTED, as in east_table_texts_host.
+ *   east_table_groups_host: host text (text_width 4: uint32 code points as east_table_host, 1: one byte per code point
+ *     as east_table_host_u8), out_DxG on the host.
+ *   east_table_groups_dev: as east_table_dev_gather (n_peers = 0: no gather; peer_rows then may be NULL).
+ *   east_table_texts_groups_host: raw UTF-8 texts, as east_table_texts_host. */
+int east_table_groups_host(const void *text, int32_t text_width, const int64_t *doc_off, const int32_t *doc_m,
+                           int32_t n_docs, int device, const uint32_t *kp, const int64_t *kp_off, int32_t V,
+                           const int64_t *group_off, int32_t G, double *out_DxG, east_index **out_idx);
+int east_table_groups_dev(const uint32_t *text_dev, const int64_t *doc_off, const int32_t *doc_m, int32_t n_docs,
+                          int device, const uint32_t *kp_dev, const uint32_t *kp_host, const int64_t *kp_off, int32_t V,
+                          const int64_t *group_off, int32_t G, double *out_DxG_dev, double *const *peer_rows,
+                          int32_t n_peers, void *stream, east_index **out_idx);
+int east_table_texts_groups_host(const uint8_t *utf8, const int64_t *text_off, int32_t n_texts, int device,
+                                 const uint32_t *kp, const int64_t *kp_off, int32_t V, const int64_t *group_off,
+                                 int32_t G, double *out_DxG, int64_t *doc_off_out /* optional */,
+                                 int32_t *doc_m_out /* optional */, east_index **out_idx);
+
 /* ---- persistence: the reference rebuilds every structure on every run (relevance.py:38-47); an index -- packed text,
  * suffix array, LCP, child table, annotation and the scorer's side tables of one batch of documents -- can be written
  * to a file and loaded back onto any device.  Scores and arrays of a loaded index are identical to the saved one's. */

@@ -1,11 +1,14 @@
 #!/usr/bin/env python3
 """Synonym-expanded keyphrase table on one GPU: the grouped scoring call (east_score_groups_dev, k_score_combine_max)
-against the plain table on the same index, and the per-variant path it replaces.
+against the plain table on the same index, and the per-variant path it replaces; the one-call synonym table
+(east_table_groups_dev: the per-document kernel keeps the best variant of each group, k_doc_suffix_sort_groups) against
+the plain one-call table and against build + grouped call; keyphrases_table with the synonimizer, one engine call from
+str texts, against the previous route (host preprocessing and build, then the grouped call).
 
 Workload: the headline collection of bench.py (synth.packed_collection_fast(1000, 50 000), synth.keyphrases(1000))
 and synth.synonyms(): every keyphrase word gets 0-3 synonyms from the same Zipf, default_rng(11).
 
-usage: python profiles/bench_synonyms.py [--out DIR] [--reps 20] [--warmup 3] [--sample-pairs 20]
+usage: python profiles/bench_synonyms.py [--out DIR] [--reps 20] [--warmup 3] [--sample-pairs 20] [--e2e-runs 3]
 Writes DIR/bench_synonyms.json and prints it."""
 import argparse
 import json
@@ -48,6 +51,7 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--sample-pairs", type=int, default=20)
     ap.add_argument("--no-e2e", action="store_true")
+    ap.add_argument("--e2e-runs", type=int, default=3)
     args = ap.parse_args()
 
     import torch
@@ -127,6 +131,55 @@ def main():
 
     timed(grouped, "device_ms_score_groups_dev")
     timed(plain, "device_ms_score_table_dev_plain_keyphrases")
+
+    # ---- one engine call: build + score, alternated; each call builds (and frees) its own index
+    out_1 = torch.empty((D, G), dtype=torch.float64, device=dev)
+
+    def one_call_groups():
+        _capi.DeviceIndex.build_dev_and_score(text_dev.data_ptr(), doc_off, doc_m, vk_dev.data_ptr(), vcodes, voff, out_1.data_ptr(),
+                                              stream=stream.cuda_stream, group_off=group_off).close()
+
+    def one_call_plain():
+        _capi.DeviceIndex.build_dev_and_score(text_dev.data_ptr(), doc_off, doc_m, kk_dev.data_ptr(), kcodes, koff, out_k.data_ptr(),
+                                              True, stream=stream.cuda_stream).close()
+
+    def build_then_groups():
+        i2 = _capi.DeviceIndex.build_dev(text_dev.data_ptr(), doc_off, doc_m, stream=stream.cuda_stream)
+        i2.score_groups_dev(vk_dev.data_ptr(), voff, group_off, out_g.data_ptr(), stream=stream.cuda_stream)
+        i2.close()
+
+    def one_call_groups_batched():
+        _capi.set_option("no_fused_score", 1)
+        try:
+            one_call_groups()
+        finally:
+            _capi.set_option("no_fused_score", 0)
+
+    arms = (("east_table_groups_dev", one_call_groups), ("east_table_groups_dev_no_fused_score", one_call_groups_batched),
+            ("east_table_dev_plain", one_call_plain), ("east_build_dev_then_east_score_groups_dev", build_then_groups))
+    for _, fn in arms:
+        for _ in range(args.warmup):
+            fn()
+    torch.cuda.synchronize()
+    per_arm = {name: [] for name, _ in arms}
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    for _ in range(args.reps):
+        for name, fn in arms:
+            e0.record(stream)
+            fn()
+            e1.record(stream)
+            e1.synchronize()
+            per_arm[name].append(e0.elapsed_time(e1))
+    res["one_call_device_ms"] = {name: _stats(ms) for name, ms in per_arm.items()}
+    res["one_call_note"] = ("CUDA events on the call's stream around the whole call (build, scoring, index freed), arms "
+                            "alternated rep by rep; text, keyphrases and table device-resident; no_fused_score = the per-run "
+                            "batched scorer (k_score_suffixes + k_score_combine_max) after the per-document kernel")
+    one = res["one_call_device_ms"]
+    res["one_call_groups_over_plain"] = one["east_table_groups_dev"]["median_ms"] / one["east_table_dev_plain"]["median_ms"]
+    res["one_call_groups_over_no_fused_score"] = (one["east_table_groups_dev"]["median_ms"] /
+                                                  one["east_table_groups_dev_no_fused_score"]["median_ms"])
+    res["one_call_groups_over_build_then_groups"] = (one["east_table_groups_dev"]["median_ms"] /
+                                                     one["east_build_dev_then_east_score_groups_dev"]["median_ms"])
     res["device_note"] = ("CUDA events on the call's stream, preparation cached (same keyphrases as the previous call); the "
                           "per-suffix scratch (documents x distinct suffixes doubles) exceeds the 126 MB L2")
     res["grouped_over_plain"] = (res["device_ms_score_groups_dev"]["median_ms"] /
@@ -134,7 +187,7 @@ def main():
 
     # ---- per-kernel split (separate short pass: an event pair around every launch)
     split = {}
-    for name, fn in (("score_groups_dev", grouped), ("score_table_dev_plain", plain)):
+    for name, fn in (("score_groups_dev", grouped), ("score_table_dev_plain", plain)) + arms:
         fn()
         _capi.set_option("time_kernels", 0)
         _capi.set_option("time_kernels", 1)
@@ -160,8 +213,13 @@ def main():
         "note": "EXTRAPOLATION: host wall time of the sampled pairs x documents x keyphrases, not a measured table"}
 
     # ---- parity, after the timed region: sampled rows against the oracle's max over each group
+    grouped()
+    plain()
+    one_call_groups()
+    torch.cuda.synchronize()
     table = out_g.cpu().numpy()
     plain_table = out_k.cpu().numpy()
+    one_call_table = out_1.cpu().numpy()
     checked, ok = [], True
     for d in sorted({0, D // 2, D - 1}):
         o = oracle.OracleEASA(text=text[doc_off[d]:doc_off[d + 1]], m=int(doc_m[d]))
@@ -171,24 +229,70 @@ def main():
         checked.append(d)
     for (d, k), v in zip(pairs, old):
         ok &= float(v) == float(table[d, k])
-    res["parity"] = {"rows_checked_against_oracle": checked, "old_path_pairs_checked": len(pairs), "bit_exact": ok}
+    ok &= bool(np.array_equal(one_call_table.view(np.uint64), table.view(np.uint64)))   # every row
+    res["parity"] = {"rows_checked_against_oracle": checked, "old_path_pairs_checked": len(pairs),
+                     "one_call_table_rows_checked_against_grouped_call": D, "bit_exact": ok}
     res["grouped_at_least_plain"] = bool((table >= plain_table).all())
 
-    # ---- end to end: applications.keyphrases_table with the synonimizer (host preprocessing, build, grouped call)
+    # ---- end to end: applications.keyphrases_table with the synonimizer from str texts.  New: one engine call per
+    # device batch (device preprocessing, build, in-kernel groups).  Old route: set_text_collection without the
+    # keyphrases (host preprocessing, build), then relevance_table's grouped call.  Alternated run by run.
     if not args.no_e2e:
         class Synonimizer(object):
             def get_synonyms(self):
                 return synonyms
+
+        phases = {"set_text_collection_s": [], "relevance_table_s": []}
+
+        class OldRoute(relevance.ASTRelevanceMeasure):
+            def set_text_collection(self, texts, language=None, prepared_keyphrases=None, synonimizer=None):
+                t = time.perf_counter()
+                super(OldRoute, self).set_text_collection(texts, language)
+                phases["set_text_collection_s"].append(time.perf_counter() - t)
+
+            def relevance_table(self, prepared_keyphrases, synonimizer=None):
+                t = time.perf_counter()
+                out = super(OldRoute, self).relevance_table(prepared_keyphrases, synonimizer)
+                phases["relevance_table_s"].append(time.perf_counter() - t)
+                return out
+
         texts = {"t%d" % j: d for j, d in enumerate(synth.documents(args.docs, args.doc_bytes))}
         kps = synth.keyphrases(args.keyphrases)
-        walls = []
-        for _ in range(2):
-            t = time.perf_counter()
-            tab = applications.keyphrases_table(kps, texts, relevance.ASTRelevanceMeasure(), synonimizer=Synonimizer())
-            walls.append(time.perf_counter() - t)
+        grouped_calls = []
+        real_score_groups = _capi.DeviceIndex.score_groups
+
+        def counting(self, *a, **k):
+            grouped_calls.append(1)
+            return real_score_groups(self, *a, **k)
+        _capi.DeviceIndex.score_groups = counting
+        walls = {"new": [], "old_route": []}
+        tabs = {}
+        new_one_call = True
+        for _ in range(args.e2e_runs):
+            for name, make in (("new", relevance.ASTRelevanceMeasure), ("old_route", OldRoute)):
+                measure = make()
+                del grouped_calls[:]
+                t = time.perf_counter()
+                tabs[name] = applications.keyphrases_table(kps, texts, measure, synonimizer=Synonimizer())
+                walls[name].append(time.perf_counter() - t)
+                if name == "new":   # device preprocessing, one batch, no grouped call after the build
+                    new_one_call &= (measure.asts[0]._strings_collection is None and len(measure._batches) == 1
+                                     and not grouped_calls)
+                del measure
+        _capi.DeviceIndex.score_groups = real_score_groups
         res["e2e_keyphrases_table_with_synonimizer_s"] = {
-            "runs_s": walls, "note": "wall time, synth.documents(%d, %d) as str, host preprocessing included; run 1 is cold"
-                                     % (args.docs, args.doc_bytes)}
+            "new": {"runs_s": walls["new"], "median_s": float(np.median(walls["new"]))},
+            "old_route": {"runs_s": walls["old_route"], "median_s": float(np.median(walls["old_route"])),
+                          "phases": phases},
+            "old_over_new": float(np.median(walls["old_route"]) / np.median(walls["new"])),
+            "new_is_one_engine_call_with_device_preprocessing": bool(new_one_call),
+            "note": "host wall time of applications.keyphrases_table, synth.documents(%d, %d) as str, dict building included; "
+                    "runs alternated, run 1 of each arm is cold; old_route phases: set_text_collection(texts) (host "
+                    "preprocessing + build) and relevance_table(prepared, synonimizer) (grouped call)"
+                    % (args.docs, args.doc_bytes)}
+        tab = tabs["new"]
+        res["parity"]["e2e_new_equals_old_route"] = all(
+            float(tabs["new"][kp][n]).hex() == float(tabs["old_route"][kp][n]).hex() for kp in kps for n in texts)
         name = "t0"
         o = oracle.OracleEASA(utils.text_to_strings_collection(texts[name]))
         exp = _group_max(o.score_many(vcodes, voff, True), group_off)
