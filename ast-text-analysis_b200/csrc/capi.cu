@@ -1159,13 +1159,59 @@ static DevBuf<int32_t> upload_groups(const int64_t *group_off, int32_t G, cudaSt
     return d;
 }
 
+// tcgen05 kernel of the co-occurrence counts (option cooc_variant: 2 = the 128 x 128 kernel, 3 = the cp.async pipeline,
+// otherwise the TMA-fed cluster kernel; 1 selects the AND + POPC kernel of east_cooc_*, which reads the score table)
+static int cooc_tc_kernel() {
+    const int64_t v = get_option("cooc_variant", 0);
+    return v == 2 ? 1 : (v == 3 ? 2 : 0);
+}
+
+// ---- keyphrase graphs: relevance bytes instead of a score table ------------------------------------------------------
+// A graph call fills B[k][d] = (score of document d in column k >= threshold), the zero-padded Kp x Dp byte matrix of the
+// co-occurrence GEMM (cooc_tc.cu), and never a documents x keyphrases table: the per-document kernel stores its column of
+// bytes itself (k_doc_suffix_sort_graph); every other path scores tiles of documents into an fp64 scratch bounded by the
+// score_tmp_doubles budget and thresholds each tile into its columns (graph_enqueue).
+struct GraphOut {
+    double threshold = 0.0;
+    int32_t *C = nullptr;   // device: cols x cols counts
+    DevBuf<uint8_t> B;
+    int64_t Dp = 0;
+    int32_t Kp = 0;
+    void begin(int32_t n_docs, int32_t cols, cudaStream_t s) {
+        cooc_padding(n_docs, cols, &Dp, &Kp);
+        B = DevBuf<uint8_t>((size_t)Kp * (size_t)Dp, s);
+        EAST_CUDA(cudaMemsetAsync(B.p, 0, (size_t)Kp * (size_t)Dp, s));   // padding rows / columns stay zero
+    }
+    void finish(int32_t cols, cudaStream_t s) const { cooc_counts_bytes(B.p, Dp, Kp, cols, C, s, cooc_tc_kernel()); }
+};
+
+// documents per tile of a graph call's fp64 scratch
+static int32_t graph_tile_docs(int32_t doc_count, int32_t cols) {
+    const int64_t budget = get_option("score_tmp_doubles", (int64_t)1 << 27);
+    return (int32_t)std::max<int64_t>(1, std::min<int64_t>(doc_count, budget / std::max<int32_t>(1, cols)));
+}
+
+// score_enqueue for a graph: documents [doc_begin, doc_begin + doc_count) tile by tile into S[S_docs][cols], each tile
+// thresholded into its columns of g.B (stream-ordered: the next tile overwrites S after the previous one is read)
+static void graph_enqueue(const east_index *idx, const KpPrepared *kp, const uint32_t *kp_dev, int64_t total, int32_t K,
+                          int normalized, int32_t doc_begin, int32_t doc_count, cudaStream_t s, double *tmp, int32_t tile_docs,
+                          const int32_t *group_off_dev, int32_t G, const GraphOut &g, double *S, int32_t S_docs) {
+    const int32_t cols = group_off_dev ? G : K;
+    for (int32_t d0 = 0; d0 < doc_count; d0 += S_docs) {
+        const int32_t cnt = std::min(S_docs, doc_count - d0);
+        score_enqueue(idx, kp, kp_dev, total, K, normalized, S, doc_begin + d0, cnt, s, tmp, tile_docs, nullptr, nullptr, 0,
+                      group_off_dev, G);
+        threshold_bytes(S, cnt, cols, g.threshold, g.B.p, g.Dp, (int64_t)doc_begin + d0, s);
+    }
+}
+
 static void score_common(const east_index *idx, const uint32_t *kp_dev, const int64_t *kp_off, int32_t K,
                          int normalized, double *out_dev, int32_t doc_begin, int32_t doc_count, cudaStream_t s,
                          double *suffix_out_dev /* optional: per-suffix results of the doc range */,
                          int64_t *probes_out = nullptr /* optional: run the probe-counting scorer */,
                          const uint32_t *kp_host = nullptr /* optional: the same code points on the host */,
                          const int64_t *group_off = nullptr /* optional: the K queries are variants in G groups (host, G + 1) */,
-                         int32_t G = 0) {
+                         int32_t G = 0, const GraphOut *graph = nullptr /* relevance bytes instead of out_dev */) {
     // per-suffix results wanted (return_suffix_scores): every suffix is its own "distinct" suffix
     const bool dedup = !suffix_out_dev && !get_option("score_no_dedup", 0);
     KpPrepared *kp = prepare_keyphrases(idx, kp_dev, kp_host, kp_off, K, dedup, s);
@@ -1191,8 +1237,15 @@ static void score_common(const east_index *idx, const uint32_t *kp_dev, const in
     }
     StageTimer tm(s);
     tm.mark("score");
-    score_enqueue(idx, kp, kp_dev, total, K, normalized, out_dev, doc_begin, doc_count, s, tmp, tile_docs, d_probes.p, nullptr, 0,
-                  d_groups.p, G);
+    if (graph) {
+        const int32_t S_docs = graph_tile_docs(doc_count, group_off ? G : K);
+        DevBuf<double> S((size_t)S_docs * (group_off ? G : K), s);
+        graph_enqueue(idx, kp, kp_dev, total, K, normalized, doc_begin, doc_count, s, tmp, tile_docs, d_groups.p, G, *graph, S.p,
+                      S_docs);
+    } else {
+        score_enqueue(idx, kp, kp_dev, total, K, normalized, out_dev, doc_begin, doc_count, s, tmp, tile_docs, d_probes.p, nullptr, 0,
+                      d_groups.p, G);
+    }
     tm.finish();
     if (probes_out) {
         unsigned long long h = 0;
@@ -1307,6 +1360,11 @@ struct TableRun {
     DevBuf<int32_t> d_groups;
     int32_t cols() const { return group_off ? G : K; }
     double *d_out = nullptr, *host_out = nullptr;   // host_out NULL: the table stays on the device
+    // keyphrase graph: relevance bytes into graph->B instead of rows (d_out, host_out NULL); the batched scorer's rows go
+    // through the per-stream scratch rows[] of rows_docs documents
+    const GraphOut *graph = nullptr;
+    DevBuf<double> rows[2];
+    int32_t rows_docs[2] = {0, 0};
     double *const *peer_rows = nullptr;             // sharded table: where this rank's rows start in every other rank's table
     int32_t n_peers = 0;
     int32_t docs_sent = 0;                          // documents whose rows have reached the peers (current pass)
@@ -1403,7 +1461,12 @@ static void table_run_begin(void *vctx, const RunReady &r, DocScore &score) {
             score.recs = t.kp->dev.d_recs.p; score.n_uniq = (int32_t)t.kp->n_uniq; score.q8 = t.kp->dev.d_q8.p; score.kp = t.d_kp;
             score.tmp = t.tmp[li].p; score.normalized = t.normalized ? 1 : 0;
             score.kp_off = t.kp->dev.d_off.p; score.uniq_of = t.kp->dev.d_uniq_of.p; score.K = t.K;
-            score.out = t.d_out + (size_t)r.doc_begin * t.cols();
+            if (t.graph) {
+                score.graph = t.graph->B.p; score.graph_pitch = t.graph->Dp; score.graph_col0 = r.doc_begin;
+                score.threshold = t.graph->threshold;
+            } else {
+                score.out = t.d_out + (size_t)r.doc_begin * t.cols();
+            }
             if (t.group_off) { score.group_off = t.d_groups.p; score.G = t.G; }
             score.skip_suffix_keys = get_option("eager_suffix_keys", 0) ? 0 : 1;
             score.n_peers = t.n_peers;
@@ -1423,6 +1486,19 @@ static void table_run_done(void *vctx, const RunReady &r, int in_kernel) {
     try {
         const int li = table_lane(t, r.stream);
         const int32_t cols = t.cols();
+        if (t.graph) {
+            if (!in_kernel) {
+                const int32_t S_docs = graph_tile_docs(r.doc_count, cols);
+                if (t.rows_docs[li] < S_docs) {
+                    t.rows[li] = DevBuf<double>((size_t)S_docs * cols, r.stream);
+                    t.rows_docs[li] = S_docs;
+                }
+                graph_enqueue(&t.view, t.kp, t.d_kp, t.kp_off[t.K], t.K, t.normalized, r.doc_begin, r.doc_count, r.stream,
+                              t.tmp[li].p, (int32_t)t.tmp_docs[li], t.d_groups.p, t.G, *t.graph, t.rows[li].p, t.rows_docs[li]);
+            }
+            t.docs_scored += r.doc_count;
+            return;
+        }
         double *rows = t.d_out + (size_t)r.doc_begin * cols;
         if (!in_kernel) {
             std::vector<double *> peers((size_t)t.n_peers);
@@ -1445,8 +1521,8 @@ static void table_host_impl(const void *text, int width, const int64_t *doc_off,
                             east_index **out_idx, double *own_rows_dev = nullptr, double *const *peer_rows = nullptr,
                             int32_t n_peers = 0,
                             const int64_t *group_off = nullptr /* synonym-expanded table: G + 1 offsets of the variant groups */,
-                            int32_t G = 0) {
-    if (!kp || !kp_off || !out_DxK || K <= 0) throw Error(EAST_ERR_INVALID, "bad argument");
+                            int32_t G = 0, GraphOut *graph = nullptr /* keyphrase graph: counts into graph->C, no table */) {
+    if (!kp || !kp_off || (!out_DxK && !graph) || K <= 0) throw Error(EAST_ERR_INVALID, "bad argument");
     if (n_peers < 0 || n_peers > DocScore::MAX_PEERS || (n_peers > 0 && !peer_rows)) throw Error(EAST_ERR_INVALID, "bad peer list");
     east_index *built = nullptr;
     check_build_args(text, doc_off, doc_m, n_docs, &built);
@@ -1459,14 +1535,15 @@ static void table_host_impl(const void *text, int width, const int64_t *doc_off,
     const int32_t cols = group_off ? G : K;
     DevBuf<uint32_t> d_kp((size_t)kp_off[K], ps);
     DevBuf<double> d_out_own;
-    if (!own_rows_dev) d_out_own = DevBuf<double>((size_t)n_docs * cols, s);
+    if (graph) graph->begin(n_docs, cols, s);
+    else if (!own_rows_dev) d_out_own = DevBuf<double>((size_t)n_docs * cols, s);
     double *const d_out = own_rows_dev ? own_rows_dev : d_out_own.p;
     EAST_CUDA(cudaMemcpyAsync(d_kp.p, kp, sizeof(uint32_t) * (size_t)kp_off[K], cudaMemcpyHostToDevice, ps));
     TableRun run;
     run.kp_own = kp_begin(device, d_kp.p, kp, kp_off, K, !get_option("score_no_dedup", 0), false, ps, likely_code_table());
     run.kp_host = kp; run.d_kp = d_kp.p; run.kp_off = kp_off; run.K = K; run.normalized = normalized;
     if (group_off) { run.group_off = group_off; run.G = G; run.d_groups = upload_groups(group_off, G, s); }
-    run.d_out = d_out; run.host_out = out_DxK;
+    run.d_out = d_out; run.host_out = out_DxK; run.graph = graph;
     run.peer_rows = peer_rows; run.n_peers = n_peers;
     RunHook hook;
     hook.begin = table_run_begin; hook.fn = table_run_done; hook.ctx = &run; hook.building = &run.building;
@@ -1478,12 +1555,13 @@ static void table_host_impl(const void *text, int width, const int64_t *doc_off,
     const bool stands = !run.failed && run.docs_scored == n_docs &&
                         ((built->pipelined && !run.final_pass) || (built->doc_sorted && !built->pipelined && run.final_pass));
     if (!stands) {
-        score_common(built, d_kp.p, kp_off, K, normalized, d_out, 0, n_docs, s, nullptr, nullptr, kp, group_off, G);
-        EAST_CUDA(cudaMemcpyAsync(out_DxK, d_out, sizeof(double) * (size_t)n_docs * cols, cudaMemcpyDeviceToHost, s));
+        score_common(built, d_kp.p, kp_off, K, normalized, d_out, 0, n_docs, s, nullptr, nullptr, kp, group_off, G, graph);
+        if (!graph) EAST_CUDA(cudaMemcpyAsync(out_DxK, d_out, sizeof(double) * (size_t)n_docs * cols, cudaMemcpyDeviceToHost, s));
     }
     if (n_peers > 0 && !(stands && run.docs_sent == n_docs))   // rows (also) produced by the batched scorer: plain peer copies
         for (int32_t pi = 0; pi < n_peers; ++pi)
             EAST_CUDA(cudaMemcpyAsync(peer_rows[pi], d_out, sizeof(double) * (size_t)n_docs * cols, cudaMemcpyDefault, s));
+    if (graph) graph->finish(cols, s);
     EAST_CUDA(cudaStreamSynchronize(s));
     if (out_idx) *out_idx = guard.release();
 }
@@ -1509,24 +1587,26 @@ static void table_dev_impl(const uint32_t *text_dev, const int64_t *doc_off, con
                            double *out_DxK_dev, double *const *peer_rows, int32_t n_peers, void *stream, east_index **out_idx,
                            bool owns_text = false /* the index takes the text over (also when the call fails) */,
                            const int64_t *group_off = nullptr /* synonym-expanded table: G + 1 offsets of the variant groups */,
-                           int32_t G = 0) {
+                           int32_t G = 0, GraphOut *graph = nullptr /* keyphrase graph: counts into graph->C, no table */) {
     struct TextGuard {   // an owned text that never reached an index
         const uint32_t *p; bool armed;
         ~TextGuard() { if (armed && p) dev_free(const_cast<uint32_t *>(p), 0); }
     } text_guard{text_dev, owns_text};
-    if (!kp_dev || !kp_off || !out_DxK_dev || K <= 0) throw Error(EAST_ERR_INVALID, "bad argument");
-    if (n_peers < 0 || n_peers > DocScore::MAX_PEERS || (n_peers > 0 && !peer_rows)) throw Error(EAST_ERR_INVALID, "bad peer list");
+    if (!kp_dev || !kp_off || (!out_DxK_dev && !graph) || K <= 0) throw Error(EAST_ERR_INVALID, "bad argument");
+    if (n_peers < 0 || n_peers > DocScore::MAX_PEERS || (n_peers > 0 && !peer_rows) || (n_peers > 0 && graph))
+        throw Error(EAST_ERR_INVALID, "bad peer list");
     east_index *built = nullptr;
     check_build_args(text_dev, doc_off, doc_m, n_docs, &built);
     check_keyphrases(kp_off, K);
     use_device(device);
     cudaStream_t s = (cudaStream_t)stream;
+    if (graph) graph->begin(n_docs, group_off ? G : K, s);
     TableRun run;
     // keyphrase preparation on a side stream, queued from the build once its alphabet scan is on its way
     run.device = device; run.dedup = !get_option("score_no_dedup", 0); run.kp_stream = prep_stream(device); run.caller_stream = s;
     run.kp_host = kp_host; run.d_kp = kp_dev; run.kp_off = kp_off; run.K = K; run.normalized = normalized;
     if (group_off) { run.group_off = group_off; run.G = G; run.d_groups = upload_groups(group_off, G, s); }
-    run.d_out = out_DxK_dev; run.host_out = nullptr;
+    run.d_out = out_DxK_dev; run.host_out = nullptr; run.graph = graph;
     run.peer_rows = peer_rows; run.n_peers = n_peers;
     RunHook hook;
     hook.begin = table_run_begin; hook.fn = table_run_done; hook.ctx = &run; hook.building = &run.building;
@@ -1537,12 +1617,13 @@ static void table_dev_impl(const uint32_t *text_dev, const int64_t *doc_off, con
     std::unique_ptr<east_index, void (*)(east_index *)> guard(built, free_index);
     const bool stands = !run.failed && run.docs_scored == n_docs && built->doc_sorted && run.final_pass;
     if (!stands)
-        score_common(built, kp_dev, kp_off, K, normalized, out_DxK_dev, 0, n_docs, s, nullptr, nullptr, kp_host, group_off, G);
+        score_common(built, kp_dev, kp_off, K, normalized, out_DxK_dev, 0, n_docs, s, nullptr, nullptr, kp_host, group_off, G, graph);
     if (n_peers > 0 && !(stands && run.docs_sent == n_docs)) {
         // the rows were (also) produced by the batched scorer: plain peer copies of the slice
         for (int32_t pi = 0; pi < n_peers; ++pi)
             EAST_CUDA(cudaMemcpyAsync(peer_rows[pi], out_DxK_dev, sizeof(double) * (size_t)n_docs * run.cols(), cudaMemcpyDefault, s));
     }
+    if (graph) graph->finish(run.cols(), s);
     EAST_CUDA(cudaStreamSynchronize(s));
     if (out_idx) *out_idx = guard.release();
 }
@@ -1632,7 +1713,7 @@ int east_cooc_dev(const double *S_DxK_dev, int64_t D, int32_t K, double threshol
     StageTimer tm(s);
     tm.mark("cooc");
     if (get_option("cooc_variant", 0) == 1) cooc_counts(S_DxK_dev, D, K, threshold, C_KxK_dev, s);
-    else cooc_counts_tc(S_DxK_dev, D, K, threshold, C_KxK_dev, s, get_option("cooc_variant", 0) == 2 ? 1 : (get_option("cooc_variant", 0) == 3 ? 2 : 0));
+    else cooc_counts_tc(S_DxK_dev, D, K, threshold, C_KxK_dev, s, cooc_tc_kernel());
     tm.finish();
     EAST_CUDA(cudaStreamSynchronize(s));
     tm.collect();
@@ -1648,7 +1729,7 @@ int east_cooc_host(const double *S_DxK, int64_t D, int32_t K, double threshold, 
     DevBuf<int32_t> d_C((size_t)K * K, s);
     EAST_CUDA(cudaMemcpyAsync(d_S.p, S_DxK, sizeof(double) * (size_t)D * K, cudaMemcpyHostToDevice, s));
     if (get_option("cooc_variant", 0) == 1) cooc_counts(d_S.p, D, K, threshold, d_C.p, s);
-    else cooc_counts_tc(d_S.p, D, K, threshold, d_C.p, s, get_option("cooc_variant", 0) == 2 ? 1 : (get_option("cooc_variant", 0) == 3 ? 2 : 0));
+    else cooc_counts_tc(d_S.p, D, K, threshold, d_C.p, s, cooc_tc_kernel());
     EAST_CUDA(cudaMemcpy(C_KxK, d_C.p, sizeof(int32_t) * (size_t)K * K, cudaMemcpyDeviceToHost));
     EAST_API_END
 }
@@ -1712,8 +1793,9 @@ int east_texts_to_packed_host(const uint8_t *utf8, const int64_t *text_off, int3
 
 static void table_texts_impl(const uint8_t *utf8, const int64_t *text_off, int32_t n_texts, int device, const uint32_t *kp,
                              const int64_t *kp_off, int32_t K, int normalized, double *out_DxK, int64_t *doc_off_out,
-                             int32_t *doc_m_out, east_index **out_idx, const int64_t *group_off = nullptr, int32_t G = 0) {
-    if (!kp || !kp_off || !out_DxK || K <= 0) throw Error(EAST_ERR_INVALID, "bad argument");
+                             int32_t *doc_m_out, east_index **out_idx, const int64_t *group_off = nullptr, int32_t G = 0,
+                             GraphOut *graph = nullptr) {
+    if (!kp || !kp_off || (!out_DxK && !graph) || K <= 0) throw Error(EAST_ERR_INVALID, "bad argument");
     check_keyphrases(kp_off, K);
     const int32_t cols = group_off ? G : K;
     use_device(device);
@@ -1723,13 +1805,14 @@ static void table_texts_impl(const uint8_t *utf8, const int64_t *text_off, int32
     if (doc_off_out) std::copy(pt.doc_off.begin(), pt.doc_off.end(), doc_off_out);
     if (doc_m_out) std::copy(pt.doc_m.begin(), pt.doc_m.end(), doc_m_out);
     DevBuf<uint32_t> d_kp((size_t)kp_off[K], s);
-    DevBuf<double> d_out((size_t)n_texts * cols, s);
+    DevBuf<double> d_out;
+    if (!graph) d_out = DevBuf<double>((size_t)n_texts * cols, s);
     EAST_CUDA(cudaMemcpyAsync(d_kp.p, kp, sizeof(uint32_t) * (size_t)kp_off[K], cudaMemcpyHostToDevice, s));
     const uint32_t *text = pt.text;
     pt.text = nullptr;   // the index owns it from here on
     table_dev_impl(text, pt.doc_off.data(), pt.doc_m.data(), n_texts, device, d_kp.p, kp, kp_off, K, normalized, d_out.p, nullptr, 0,
-                   (void *)s, out_idx, true, group_off, G);
-    EAST_CUDA(cudaMemcpy(out_DxK, d_out.p, sizeof(double) * (size_t)n_texts * cols, cudaMemcpyDeviceToHost));
+                   (void *)s, out_idx, true, group_off, G, graph);
+    if (!graph) EAST_CUDA(cudaMemcpy(out_DxK, d_out.p, sizeof(double) * (size_t)n_texts * cols, cudaMemcpyDeviceToHost));
 }
 
 int east_table_texts_host(const uint8_t *utf8, const int64_t *text_off, int32_t n_texts, int device, const uint32_t *kp,
@@ -1746,6 +1829,69 @@ int east_table_texts_groups_host(const uint8_t *utf8, const int64_t *text_off, i
     EAST_API_BEGIN
     check_table_groups(kp_off, V, group_off, G);
     table_texts_impl(utf8, text_off, n_texts, device, kp, kp_off, V, 1, out_DxG, doc_off_out, doc_m_out, out_idx, group_off, G);
+    EAST_API_END
+}
+
+// ---- keyphrase graphs in one call: build, score and count co-occurrences, no score table ------------------------------
+// (arguments are checked before anything is built; groups are always normalized, as in the table entries)
+static void check_graph_args(const int64_t *kp_off, int32_t V, const int64_t *group_off, int32_t G, const void *C) {
+    if (!kp_off || V <= 0 || !C) throw Error(EAST_ERR_INVALID, "bad argument");
+    if (group_off) check_groups(group_off, G, V);
+    check_keyphrases(kp_off, V);
+}
+
+// the cols x cols counts of a host entry: C on the device, copied out once the call's stream is done
+struct HostCounts {
+    DevBuf<int32_t> d;
+    int32_t cols;
+    HostCounts(int32_t V, const int64_t *group_off, int32_t G) : d((size_t)(group_off ? G : V) * (group_off ? G : V), 0),
+                                                                  cols(group_off ? G : V) {}
+    void copy_out(int32_t *C_host) {
+        EAST_CUDA(cudaMemcpyAsync(C_host, d.p, sizeof(int32_t) * (size_t)cols * cols, cudaMemcpyDeviceToHost, 0));
+        EAST_CUDA(cudaStreamSynchronize(0));
+    }
+};
+
+int east_graph_host(const void *text, int32_t text_width, const int64_t *doc_off, const int32_t *doc_m, int32_t n_docs,
+                    int device, const uint32_t *kp, const int64_t *kp_off, int32_t V, const int64_t *group_off, int32_t G,
+                    int normalized, double threshold, int32_t *C_host, east_index **out_idx) {
+    EAST_API_BEGIN
+    if (text_width != 1 && text_width != 4) throw Error(EAST_ERR_INVALID, "text_width must be 1 or 4");
+    check_graph_args(kp_off, V, group_off, G, C_host);
+    use_device(device);
+    HostCounts counts(V, group_off, G);
+    GraphOut graph;
+    graph.threshold = threshold; graph.C = counts.d.p;
+    table_host_impl(text, text_width, doc_off, doc_m, n_docs, device, kp, kp_off, V, group_off ? 1 : normalized, nullptr, out_idx,
+                    nullptr, nullptr, 0, group_off, G, &graph);
+    counts.copy_out(C_host);
+    EAST_API_END
+}
+
+int east_graph_dev(const uint32_t *text_dev, const int64_t *doc_off, const int32_t *doc_m, int32_t n_docs, int device,
+                   const uint32_t *kp_dev, const uint32_t *kp_host, const int64_t *kp_off, int32_t V, const int64_t *group_off,
+                   int32_t G, int normalized, double threshold, int32_t *C_dev, void *stream, east_index **out_idx) {
+    EAST_API_BEGIN
+    check_graph_args(kp_off, V, group_off, G, C_dev);
+    GraphOut graph;
+    graph.threshold = threshold; graph.C = C_dev;
+    table_dev_impl(text_dev, doc_off, doc_m, n_docs, device, kp_dev, kp_host, kp_off, V, group_off ? 1 : normalized, nullptr, nullptr, 0,
+                   stream, out_idx, false, group_off, G, &graph);
+    EAST_API_END
+}
+
+int east_graph_texts_host(const uint8_t *utf8, const int64_t *text_off, int32_t n_texts, int device, const uint32_t *kp,
+                          const int64_t *kp_off, int32_t V, const int64_t *group_off, int32_t G, int normalized, double threshold,
+                          int32_t *C_host, int64_t *doc_off_out, int32_t *doc_m_out, east_index **out_idx) {
+    EAST_API_BEGIN
+    check_graph_args(kp_off, V, group_off, G, C_host);
+    use_device(device);
+    HostCounts counts(V, group_off, G);
+    GraphOut graph;
+    graph.threshold = threshold; graph.C = counts.d.p;
+    table_texts_impl(utf8, text_off, n_texts, device, kp, kp_off, V, group_off ? 1 : normalized, nullptr, doc_off_out, doc_m_out,
+                     out_idx, group_off, G, &graph);
+    counts.copy_out(C_host);
     EAST_API_END
 }
 

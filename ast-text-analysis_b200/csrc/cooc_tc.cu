@@ -56,13 +56,16 @@ __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
     } while (!done);
 }
 
-// S[d][k] >= thr  ->  Bm[k][d] (uint8): 128 (documents) x 32 (keyphrases) transposing tiles through shared memory.
+// S[d][k] >= thr  ->  Bm[k][col0 + d] (uint8): 128 (documents) x 32 (keyphrases) transposing tiles through shared memory.
 // Reads: a warp takes 32 consecutive doubles of a row of S (256 bytes), four rows in flight per thread; writes: every
 // keyphrase row of the tile leaves as 128 contiguous bytes (eight 16-byte stores).  HBM-bound: 8 D K bytes in, D K out.
+// Only the columns [col0, col0 + D) are written, so that document tiles scored one after another (possibly on two
+// streams) fill their own columns of one matrix; a piece that is not a whole aligned 16 bytes inside them is stored
+// byte by byte.
 constexpr int TB_D = 128, TB_K = 32;
 __global__ void __launch_bounds__(256)
 k_threshold_bytes(const double *__restrict__ S, int64_t D, int32_t K, double thr, uint8_t *__restrict__ Bm,
-                  int64_t Dp) {
+                  int64_t Dp, int64_t col0) {
     __shared__ __align__(16) uint8_t tile[TB_K][TB_D + 16];    // [k][d]: the store phase reads 16 consecutive d of one k
     const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;  // 32 x 8
     const int64_t d0 = (int64_t)blockIdx.x * TB_D;
@@ -87,9 +90,13 @@ k_threshold_bytes(const double *__restrict__ S, int64_t D, int32_t K, double thr
     const int kr = threadIdx.x >> 3, piece = threadIdx.x & 7;
     const int32_t ko = k0 + kr;
     const int64_t dd = d0 + 16 * piece;
-    if (ko < K && dd < Dp) {   // Dp is a multiple of 128: a piece is inside or outside as a whole
-        const uint4 out = *reinterpret_cast<const uint4 *>(&tile[kr][16 * piece]);
-        *reinterpret_cast<uint4 *>(Bm + (int64_t)ko * Dp + dd) = out;
+    if (ko < K && dd < D) {
+        uint8_t *dst = Bm + (int64_t)ko * Dp + col0 + dd;
+        if (dd + 16 <= D && (col0 & 15) == 0) {
+            *reinterpret_cast<uint4 *>(dst) = *reinterpret_cast<const uint4 *>(&tile[kr][16 * piece]);
+        } else {
+            for (int i = 0; i < 16 && dd + i < D; ++i) dst[i] = tile[kr][16 * piece + i];
+        }
     }
 }
 
@@ -526,29 +533,44 @@ static bool make_b_tensor_map(const uint8_t *Bm, int64_t Dp, int32_t Kp, CUtenso
                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
+void cooc_padding(int64_t D, int32_t K, int64_t *Dp, int32_t *Kp) {
+    *Dp = (D + CT_BK - 1) / CT_BK * CT_BK;
+    *Kp = (K + CP_TN - 1) / CP_TN * CP_TN;   // rows padded to the larger tile edge (256)
+}
+
+void threshold_bytes(const double *S_DxK, int64_t D, int32_t K, double threshold, uint8_t *Bm, int64_t Dp, int64_t col0,
+                     cudaStream_t s) {
+    dim3 tg((unsigned)((D + TB_D - 1) / TB_D), (unsigned)((K + TB_K - 1) / TB_K));
+    EAST_BYTES(8.0 * (double)D * K + (double)K * D);
+    EAST_LAUNCH(k_threshold_bytes, tg, 256, 0, s, S_DxK, D, K, threshold, Bm, Dp, col0);
+}
+
 void cooc_counts_tc(const double *S_DxK, int64_t D, int32_t K, double threshold, int32_t *C, cudaStream_t s, int simple) {
-    const int64_t Dp = (D + CT_BK - 1) / CT_BK * CT_BK;
-    const int32_t Kp = (K + CP_TN - 1) / CP_TN * CP_TN;   // rows padded to the larger tile edge (256)
+    int64_t Dp;
+    int32_t Kp;
+    cooc_padding(D, K, &Dp, &Kp);
     DevBuf<uint8_t> Bm((size_t)Kp * (size_t)Dp, s);
     EAST_CUDA(cudaMemsetAsync(Bm.p, 0, (size_t)Kp * (size_t)Dp, s));  // padding rows / columns are zero
-    dim3 tg((unsigned)((Dp + TB_D - 1) / TB_D), (unsigned)((K + TB_K - 1) / TB_K));
-    EAST_BYTES(8.0 * (double)D * K + (double)K * Dp);
-    EAST_LAUNCH(k_threshold_bytes, tg, 256, 0, s, S_DxK, D, K, threshold, Bm.p, Dp);
+    threshold_bytes(S_DxK, D, K, threshold, Bm.p, Dp, 0, s);
+    cooc_counts_bytes(Bm.p, Dp, Kp, K, C, s, simple);
+}
+
+void cooc_counts_bytes(const uint8_t *Bm, int64_t Dp, int32_t Kp, int32_t K, int32_t *C, cudaStream_t s, int simple) {
     const int smem = 2 * CT_STAGE_BYTES + 1024, smem_pipe = CP_STAGES * CP_STAGE_BYTES + 1024;
     ensure_dynamic_smem((const void *)k_cooc_umma, smem);
     ensure_dynamic_smem((const void *)k_cooc_umma_pipe, smem_pipe);
     CUtensorMap tmap;
-    if (simple == 0 && make_b_tensor_map(Bm.p, Dp, Kp, &tmap)) {
+    if (simple == 0 && make_b_tensor_map(Bm, Dp, Kp, &tmap)) {
         const int smem_tma = CQ_STAGES * CQ_STAGE_BYTES + 1024;
         ensure_dynamic_smem((const void *)k_cooc_umma_tma, smem_tma);
         dim3 grid(Kp / CQ_TN, Kp / CQ_TM);   // Kp is a multiple of 256: an even number of tile rows, clusters of (1, 2)
         EAST_LAUNCH(k_cooc_umma_tma, grid, CQ_THREADS, smem_tma, s, tmap, Dp, K, C);
     } else if (simple == 1) {
         dim3 grid(Kp / CT_TILE, Kp / CT_TILE);
-        EAST_LAUNCH(k_cooc_umma, grid, CT_THREADS, smem, s, Bm.p, Dp, Kp, K, C);
+        EAST_LAUNCH(k_cooc_umma, grid, CT_THREADS, smem, s, Bm, Dp, Kp, K, C);
     } else {
         dim3 grid(Kp / CP_TN, Kp / CP_TM);
-        EAST_LAUNCH(k_cooc_umma_pipe, grid, CP_THREADS, smem_pipe, s, Bm.p, Dp, K, C);
+        EAST_LAUNCH(k_cooc_umma_pipe, grid, CP_THREADS, smem_pipe, s, Bm, Dp, K, C);
     }
 }
 

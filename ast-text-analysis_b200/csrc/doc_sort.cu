@@ -38,7 +38,8 @@
 //   9  (optional: east_table_host / east_table_dev) score every distinct query suffix against the document
 //      (easa.py:91-139; walks of score_walk.cuh) from a copy of text + suffix array in the freed shared memory,
 //      then add the results up per keyphrase: the CTA writes its row of the score table (k_doc_suffix_sort_groups: the
-//      best variant of each group of synonym variants).
+//      best variant of each group of synonym variants); k_doc_suffix_sort_graph / _groups_graph store the document's
+//      column of relevance bytes (score >= threshold) of a keyphrase graph instead of the row.
 // A bucket of more than 4096 suffixes raises flag bit 0: the host redoes the batch with the global sort.  A
 // document the kernel gives up on gets empty bucket rows (and, for a bad layout, an in-range suffix array), so
 // that a caller that scores speculatively stays inside the arrays.
@@ -508,7 +509,8 @@ __device__ __forceinline__ void ds_clear_tables(const DocSortParams &p, int doc,
 // are 1-64 variants: a thread per group would leave most lanes idle), and each is folded into its group's maximum with
 // a 64-bit shared-memory atomicMax on the bits of the double.  Scores are >= +0.0 and never NaN, so their bit patterns
 // order as the values do and the maximum has the bits k_score_combine_max finds, whatever the order of the atomics.
-// `smem` (the staged text, no longer read) holds the G running maxima.
+// `smem` (the staged text, no longer read) holds the G running maxima.  GRAPH: the group's relevance byte instead.
+template <bool GRAPH>
 __device__ __forceinline__ void ds_store_group_maxima(const DocSortParams &p, uint8_t *smem, int doc, const double *out, int tid) {
     unsigned long long *s_best = reinterpret_cast<unsigned long long *>(smem);
     const int32_t G = p.score.G;
@@ -522,6 +524,12 @@ __device__ __forceinline__ void ds_store_group_maxima(const DocSortParams &p, ui
         atomicMax(s_best + doc_of(p.score.group_off, G, v), (unsigned long long)__double_as_longlong(score));
     }
     __syncthreads();
+    if (GRAPH) {
+        uint8_t *col = p.score.graph + p.score.graph_col0 + (doc - p.doc_begin);
+        for (int g = tid; g < G; g += DS_THREADS)
+            col[(size_t)g * (size_t)p.score.graph_pitch] = __longlong_as_double((long long)s_best[g]) >= p.score.threshold ? 1 : 0;
+        return;
+    }
     double *table_row = p.score.out + (size_t)(doc - p.doc_begin) * (size_t)G;
     for (int g = tid; g < G; g += DS_THREADS) {
         const double v = __longlong_as_double((long long)s_best[g]);
@@ -538,7 +546,8 @@ __device__ __forceinline__ void ds_store_group_maxima(const DocSortParams &p, ui
 // document are staged there, so every probe of a walk -- the binary searches over (rank -> symbol at depth d)
 // -- is two shared-memory loads instead of dependent L2 / HBM round trips.  Only the bucket-table lookups that
 // open a walk (one batch of loads per suffix) and the suffix records go to global memory.
-template <bool GROUPS>
+// GRAPH: the CTA stores its document's column of relevance bytes instead of its row of the table (DocScore::graph).
+template <bool GROUPS, bool GRAPH>
 __device__ __forceinline__ void ds_score_document(const DocSortParams &p, uint8_t *smem, int smem_bytes, int doc, int32_t base, int n, int tid) {
     if (p.score.recs == nullptr) return;
     __syncthreads();   // every rank of sa and every bucket start of this document is in place; shared memory is free
@@ -582,7 +591,18 @@ __device__ __forceinline__ void ds_score_document(const DocSortParams &p, uint8_
     // easa.py:127-134), each fetched through the position of its distinct twin -- k_score_combine's arithmetic
     __syncthreads();
     if (GROUPS) {
-        ds_store_group_maxima(p, smem, doc, out, tid);
+        ds_store_group_maxima<GRAPH>(p, smem, doc, out, tid);
+        return;
+    }
+    if (GRAPH) {
+        // the same sums; one byte per keyphrase, Dp apart (the threshold compare of k_threshold_bytes)
+        uint8_t *col = p.score.graph + p.score.graph_col0 + (doc - p.doc_begin);
+        for (int k = tid; k < p.score.K; k += DS_THREADS) {
+            const int32_t sb = __ldg(p.score.kp_off + k), se = __ldg(p.score.kp_off + k + 1);
+            double result = 0.0;
+            for (int32_t x = sb; x < se; ++x) result = result + __ldcg(out + __ldg(p.score.uniq_of + x));
+            col[(size_t)k * (size_t)p.score.graph_pitch] = result / (double)(se - sb) >= p.score.threshold ? 1 : 0;
+        }
         return;
     }
     double *table_row = p.score.out + (size_t)(doc - p.doc_begin) * (size_t)p.score.K;
@@ -600,9 +620,10 @@ __device__ __forceinline__ void ds_score_document(const DocSortParams &p, uint8_
     if (p.score.n_peers > 0) __threadfence_system();
 }
 
-// The per-document kernel; GROUPS: phase 9 writes synonym-expanded rows (G wide).  Two kernels instead of a kernel
-// template, so that the plain one keeps its name (kernel timings, profiles) and its register allocation.
-template <bool GROUPS>
+// The per-document kernel; GROUPS: phase 9 writes synonym-expanded rows (G wide); GRAPH: phase 9 writes relevance bytes
+// instead of rows.  Four kernels instead of a kernel template, so that the plain one keeps its name (kernel timings,
+// profiles) and its register allocation.
+template <bool GROUPS, bool GRAPH>
 __device__ __forceinline__ void doc_suffix_sort(const DocSortParams &p) {
     extern __shared__ __align__(16) uint8_t ds_smem[];
     uint8_t *s_raw = ds_smem;                                                    // staged text
@@ -1050,7 +1071,7 @@ __device__ __forceinline__ void doc_suffix_sort(const DocSortParams &p) {
             __syncthreads();
             for (int r = tid; r < n; r += DS_THREADS) p.sk[base + r] = ds_lds4(s_raw, shift + (sa_doc[r] - base) + 2);
         }
-        ds_score_document<GROUPS>(p, ds_smem, p.text_cap + DS_SCR_BYTES + 4 * p.bits_words + 2 * (int)sizeof(uint2) * DS_LIST_CAP, doc, base, n, tid);
+        ds_score_document<GROUPS, GRAPH>(p, ds_smem, p.text_cap + DS_SCR_BYTES + 4 * p.bits_words + 2 * (int)sizeof(uint2) * DS_LIST_CAP, doc, base, n, tid);
         return;
     }
 
@@ -1250,17 +1271,23 @@ __device__ __forceinline__ void doc_suffix_sort(const DocSortParams &p) {
     }
     if (p.phase_clk) __syncthreads();
     DS_STAMP(8);
-    ds_score_document<GROUPS>(p, ds_smem, p.text_cap + DS_SCR_BYTES + 4 * p.bits_words + 2 * (int)sizeof(uint2) * DS_LIST_CAP, doc, base, n, tid);
+    ds_score_document<GROUPS, GRAPH>(p, ds_smem, p.text_cap + DS_SCR_BYTES + 4 * p.bits_words + 2 * (int)sizeof(uint2) * DS_LIST_CAP, doc, base, n, tid);
     if (p.phase_clk) __syncthreads();
     DS_STAMP(9);
 #undef DS_STAMP
 }
 
 __global__ void __launch_bounds__(DS_THREADS, 1)
-k_doc_suffix_sort(DocSortParams p) { doc_suffix_sort<false>(p); }
+k_doc_suffix_sort(DocSortParams p) { doc_suffix_sort<false, false>(p); }
 
 __global__ void __launch_bounds__(DS_THREADS, 1)
-k_doc_suffix_sort_groups(DocSortParams p) { doc_suffix_sort<true>(p); }
+k_doc_suffix_sort_groups(DocSortParams p) { doc_suffix_sort<true, false>(p); }
+
+__global__ void __launch_bounds__(DS_THREADS, 1)
+k_doc_suffix_sort_graph(DocSortParams p) { doc_suffix_sort<false, true>(p); }
+
+__global__ void __launch_bounds__(DS_THREADS, 1)
+k_doc_suffix_sort_groups_graph(DocSortParams p) { doc_suffix_sort<true, true>(p); }
 
 // Host side: can the batch take the per-document path, and with which parameters
 bool doc_sort_plan(int sigma, int32_t max_doc_n, DocSortPlan &plan) {
@@ -1291,7 +1318,10 @@ void doc_sort_launch(const DocSortPlan &plan, const uint8_t *t8, const uint32_t 
                      unsigned long long *phase_clk, const DocSortTables *tables, uint32_t *sk, const DocScore *score,
                      const uint8_t *code_table, uint32_t *miss, int64_t text_len, const uint8_t *text8) {
     const bool groups = score && score->recs && bkt && score->group_off;
-    ensure_dynamic_smem(groups ? (const void *)k_doc_suffix_sort_groups : (const void *)k_doc_suffix_sort, 220 * 1024);
+    const bool graph = score && score->recs && bkt && score->graph;
+    const void *kernel = graph ? (groups ? (const void *)k_doc_suffix_sort_groups_graph : (const void *)k_doc_suffix_sort_graph)
+                               : (groups ? (const void *)k_doc_suffix_sort_groups : (const void *)k_doc_suffix_sort);
+    ensure_dynamic_smem(kernel, 220 * 1024);
     DocSortParams p;
     p.t8 = t8; p.text = text; p.doc_off = doc_off; p.doc_m = doc_m; p.sa = sa; p.bkt = bkt; p.bkt3 = (plan.G == 3) ? bkt3 : nullptr; p.overflow = overflow;
     p.b = plan.b; p.G = plan.G; p.S2 = plan.S2; p.term = term;
@@ -1313,7 +1343,9 @@ void doc_sort_launch(const DocSortPlan &plan, const uint8_t *t8, const uint32_t 
     // with the scorer inside, plus the bytes of its walks (counted by the
     // instrumented scorer, option score_bytes)
     EAST_BYTES(((p.lcp ? 25.0 : 5.0) + (p.code_table ? (p.text8 ? 5.0 : 4.0) : 0.0)) * (double)n_total + (p.score.recs ? p.score.algorithmic_bytes : 0.0));
-    if (groups) EAST_LAUNCH(k_doc_suffix_sort_groups, n_docs, DS_THREADS, plan.smem, s, p);
+    if (graph && groups) EAST_LAUNCH(k_doc_suffix_sort_groups_graph, n_docs, DS_THREADS, plan.smem, s, p);
+    else if (graph) EAST_LAUNCH(k_doc_suffix_sort_graph, n_docs, DS_THREADS, plan.smem, s, p);
+    else if (groups) EAST_LAUNCH(k_doc_suffix_sort_groups, n_docs, DS_THREADS, plan.smem, s, p);
     else EAST_LAUNCH(k_doc_suffix_sort, n_docs, DS_THREADS, plan.smem, s, p);
 }
 

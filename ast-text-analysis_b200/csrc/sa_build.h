@@ -35,6 +35,12 @@ struct DocScore {
     // the per-rank key words (sk) only serve LATER score calls on the index (the in-kernel walks read the staged text): a
     // launch that scores its documents itself may leave them to the first such call (ensure_suffix_keys in capi.cu)
     int skip_suffix_keys = 0;
+    // keyphrase graph (k_doc_suffix_sort_graph, k_doc_suffix_sort_groups_graph): instead of its row the CTA stores the
+    // relevance bytes graph[k * graph_pitch + graph_col0 + (document - doc_begin)] = (score >= threshold), k < K (G with
+    // groups): the keyphrase-major matrix C = B B^T reads (cooc_tc.cu).  No peers in this mode.
+    uint8_t *graph = nullptr;
+    int64_t graph_pitch = 0, graph_col0 = 0;
+    double threshold = 0.0;
 };
 
 // What a caller-supplied hook sees once the per-document kernel of one run of
@@ -219,7 +225,15 @@ void score_suffixes(const ScoreInput &in, double *suffix_tmp, cudaStream_t s);
 void fill_suffix_keys(const uint8_t *t8, const int32_t *sa, int32_t n, uint32_t *sk, cudaStream_t s);
 
 void cooc_counts(const double *S_DxK, int64_t D, int32_t K, double threshold, int32_t *C, cudaStream_t s);     // AND + POPC
+// tcgen05 co-occurrence counts = threshold_bytes into a zeroed Kp x Dp byte matrix (cooc_padding) + cooc_counts_bytes
 void cooc_counts_tc(const double *S_DxK, int64_t D, int32_t K, double threshold, int32_t *C, cudaStream_t s,
-                    int simple = 0 /* 0: TMA-fed cluster kernel, 1: the non-pipelined 128 x 128 kernel, 2: the cp.async pipeline */);  // tcgen05
+                    int simple = 0 /* 0: TMA-fed cluster kernel, 1: the non-pipelined 128 x 128 kernel, 2: the cp.async pipeline */);
+// the relevance bytes of D documents x K keyphrases: Bm[Kp][Dp], Dp = D rounded up to 128, Kp = K rounded up to 256
+void cooc_padding(int64_t D, int32_t K, int64_t *Dp, int32_t *Kp);
+// Bm[k][col0 + d] = (S[d][k] >= threshold) for d < D, k < K (S: D x K doc-major); nothing else of Bm is written
+void threshold_bytes(const double *S_DxK, int64_t D, int32_t K, double threshold, uint8_t *Bm, int64_t Dp, int64_t col0,
+                     cudaStream_t s);
+// C = Bm Bm^T (K x K int32) from a prepared, zero-padded Kp x Dp matrix
+void cooc_counts_bytes(const uint8_t *Bm, int64_t Dp, int32_t Kp, int32_t K, int32_t *C, cudaStream_t s, int simple = 0);
 
 }  // namespace east

@@ -36,6 +36,7 @@ EXPORTED_SYMBOLS = [
     "east_build_host_u8", "east_table_host_u8", "east_table_dev_gather", "east_trim", "east_table_host_gather", "east_index_save", "east_index_load", "east_texts_to_packed_host", "east_table_texts_host",
     "east_score_groups_host", "east_score_groups_dev",
     "east_table_groups_host", "east_table_groups_dev", "east_table_texts_groups_host",
+    "east_graph_host", "east_graph_dev", "east_graph_texts_host",
 ]
 
 _lib = None
@@ -100,6 +101,12 @@ def load():
                                         _i64p, ctypes.c_int32, _vp, ctypes.POINTER(_vp), ctypes.c_int32, _vp, ctypes.POINTER(_vp)]
     L.east_table_texts_groups_host.argtypes = [_u8p, _i64p, ctypes.c_int32, ctypes.c_int, _u32p, _i64p, ctypes.c_int32, _i64p,
                                                ctypes.c_int32, _f64p, _i64p, _i32p, ctypes.POINTER(_vp)]
+    L.east_graph_host.argtypes = [_vp, ctypes.c_int32, _i64p, _i32p, ctypes.c_int32, ctypes.c_int, _u32p, _i64p, ctypes.c_int32,
+                                  _i64p, ctypes.c_int32, ctypes.c_int, ctypes.c_double, _i32p, ctypes.POINTER(_vp)]
+    L.east_graph_dev.argtypes = [_vp, _i64p, _i32p, ctypes.c_int32, ctypes.c_int, _vp, _u32p, _i64p, ctypes.c_int32, _i64p,
+                                 ctypes.c_int32, ctypes.c_int, ctypes.c_double, _vp, _vp, ctypes.POINTER(_vp)]
+    L.east_graph_texts_host.argtypes = [_u8p, _i64p, ctypes.c_int32, ctypes.c_int, _u32p, _i64p, ctypes.c_int32, _i64p,
+                                        ctypes.c_int32, ctypes.c_int, ctypes.c_double, _i32p, _i64p, _i32p, ctypes.POINTER(_vp)]
     L.east_score_probes_dev.argtypes = [_vp, _vp, _i64p, ctypes.c_int32, _vp, _vp, _i64p]
     L.east_score_one.argtypes = [_vp, ctypes.c_int32, _u32p, ctypes.c_int32, ctypes.c_int, _f64p, _f64p]
     L.east_cooc_dev.argtypes = [_vp, ctypes.c_int64, ctypes.c_int32, ctypes.c_double, _vp, ctypes.c_int, _vp]
@@ -209,6 +216,22 @@ def _columns(K, group_off):
     return K if group_off is None else len(group_off) - 1
 
 
+def _groups_arg(group_off):
+    """(int64 array or None, pointer or None, G) of optional group offsets"""
+    if group_off is None:
+        return None, None, 0
+    group_off = np.ascontiguousarray(group_off, dtype=np.int64)
+    return group_off, _ptr(group_off, _i64p), len(group_off) - 1
+
+
+def _counts_out(C, K, group_off):
+    cols = _columns(K, group_off)
+    if C is None:
+        return np.empty((cols, cols), dtype=np.int32)
+    assert C.dtype == np.int32 and C.flags["C_CONTIGUOUS"] and C.size == cols * cols
+    return C
+
+
 def concat_utf8(texts):
     """list of str / bytes -> (uint8 buffer of the UTF-8 texts back to back, int64 offsets [n + 1])"""
     raws = [t if isinstance(t, (bytes, bytearray)) else t.encode("utf-8", errors="surrogatepass") for t in texts]
@@ -305,6 +328,67 @@ class DeviceIndex(object):
         _check(L.east_table_texts_host(_ptr(buf, _u8p), _ptr(off, _i64p), n, int(device), _ptr(kp_codes, _u32p),
                                        _ptr(kp_off, _i64p), K, 1 if normalized else 0, _ptr(out, _f64p),
                                        _ptr(doc_off, _i64p), _ptr(doc_m, _i32p), ctypes.byref(h)))
+        return cls.from_handle(h, doc_off, doc_m, int(device))
+
+    @classmethod
+    def graph_from_texts(cls, texts, kp_codes, kp_off, threshold, C=None, normalized=True, device=0, group_off=None):
+        """table_from_texts() for a keyphrase graph (east_graph_texts_host): raw texts in, the int32 co-occurrence counts
+        C[i][j] = number of texts in which columns i and j both score >= threshold out, without a score table.
+        Returns (C, index); C: [cols, cols], cols = K, or G with group_off (always normalized)."""
+        L = load()
+        buf, off = texts if isinstance(texts, tuple) else concat_utf8(texts)
+        n = len(off) - 1
+        kp_codes = np.ascontiguousarray(kp_codes, dtype=np.uint32)
+        kp_off = np.ascontiguousarray(kp_off, dtype=np.int64)
+        K = len(kp_off) - 1
+        group_off, gp, G = _groups_arg(group_off)
+        C = _counts_out(C, K, group_off)
+        doc_off = np.zeros(n + 1, dtype=np.int64)
+        doc_m = np.zeros(n, dtype=np.int32)
+        h = _vp()
+        _check(L.east_graph_texts_host(_ptr(buf, _u8p), _ptr(off, _i64p), n, int(device), _ptr(kp_codes, _u32p), _ptr(kp_off, _i64p),
+                                       K, gp, G, 1 if normalized else 0, float(threshold), _ptr(C, _i32p), _ptr(doc_off, _i64p),
+                                       _ptr(doc_m, _i32p), ctypes.byref(h)))
+        return C, cls.from_handle(h, doc_off, doc_m, int(device))
+
+    @classmethod
+    def build_host_and_graph(cls, text, doc_off, doc_m, kp_codes, kp_off, threshold, C=None, normalized=True, device=0,
+                             group_off=None):
+        """build_host_and_score() for a keyphrase graph (east_graph_host): text uint32 code points or one byte per code
+        point (pack_strings_collection_u8).  Returns (int32 counts [cols, cols], index); no score table is formed."""
+        L = load()
+        doc_off = np.ascontiguousarray(doc_off, dtype=np.int64)
+        doc_m = np.ascontiguousarray(doc_m, dtype=np.int32)
+        kp_codes = np.ascontiguousarray(kp_codes, dtype=np.uint32)
+        kp_off = np.ascontiguousarray(kp_off, dtype=np.int64)
+        K = len(kp_off) - 1
+        assert text.dtype in (np.uint32, np.uint8) and text.flags["C_CONTIGUOUS"]
+        group_off, gp, G = _groups_arg(group_off)
+        C = _counts_out(C, K, group_off)
+        h = _vp()
+        _check(L.east_graph_host(_vp(text.ctypes.data), int(text.itemsize), _ptr(doc_off, _i64p), _ptr(doc_m, _i32p), len(doc_m),
+                                 int(device), _ptr(kp_codes, _u32p), _ptr(kp_off, _i64p), K, gp, G, 1 if normalized else 0,
+                                 float(threshold), _ptr(C, _i32p), ctypes.byref(h)))
+        return C, cls.from_handle(h, doc_off, doc_m, int(device))
+
+    @classmethod
+    def build_dev_and_graph(cls, text_devptr, doc_off, doc_m, kp_devptr, kp_codes, kp_off, threshold, C_devptr, normalized=True,
+                            device=0, stream=0, group_off=None):
+        """build_dev_and_score() for a keyphrase graph (east_graph_dev): the int32 [cols, cols] counts go to C_devptr.
+        Returns the index."""
+        L = load()
+        doc_off = np.ascontiguousarray(doc_off, dtype=np.int64)
+        doc_m = np.ascontiguousarray(doc_m, dtype=np.int32)
+        kp_off = np.ascontiguousarray(kp_off, dtype=np.int64)
+        kp_host = None
+        if kp_codes is not None:
+            kp_codes = np.ascontiguousarray(kp_codes, dtype=np.uint32)
+            kp_host = _ptr(kp_codes, _u32p)
+        group_off, gp, G = _groups_arg(group_off)
+        h = _vp()
+        _check(L.east_graph_dev(_vp(text_devptr), _ptr(doc_off, _i64p), _ptr(doc_m, _i32p), len(doc_m), int(device), _vp(kp_devptr),
+                                kp_host, _ptr(kp_off, _i64p), len(kp_off) - 1, gp, G, 1 if normalized else 0, float(threshold),
+                                _vp(C_devptr), _vp(stream), ctypes.byref(h)))
         return cls.from_handle(h, doc_off, doc_m, int(device))
 
     @classmethod

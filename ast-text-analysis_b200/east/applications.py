@@ -71,6 +71,23 @@ def keyphrases_graph(keyphrases, texts, referral_confidence=0.6, relevance_thres
     without renumbering; edges are ordered pairs (permutations order) whose confidence
     |T1 & T2| / max(|T1|, 1) reaches referral_confidence.
     """
+    similarity_measure = similarity_measure or relevance.ASTRelevanceMeasure()
+    if isinstance(similarity_measure, relevance.ASTRelevanceMeasure):
+        # the measure counts the co-occurrences while it indexes the collection (one graph call per device batch): the
+        # relevance bytes come out of the scoring kernel and no score table is formed
+        kept = [kp for kp in keyphrases if kp]
+        prepared = [utils.prepare_text(kp) for kp in kept]
+        text_collection = list(texts.values())
+        if prepared:
+            similarity_measure.set_text_collection(text_collection, language, prepared_keyphrases=prepared,
+                                                   synonimizer=synonimizer, relevance_threshold=relevance_threshold)
+        else:
+            similarity_measure.set_text_collection(text_collection, language)
+        if kept and texts:
+            cooc = similarity_measure.cooccurrence(prepared, relevance_threshold, synonimizer)
+        else:
+            cooc = np.zeros((len(kept), len(kept)), dtype=np.int32)
+        return graph_from_cooccurrence(keyphrases, kept, cooc, referral_confidence, relevance_threshold, support_threshold)
     kept, titles, scores = _score_matrix(keyphrases, texts, similarity_measure, synonimizer, language)
     if scores.size:
         cooc = _capi.cooc_host(scores, relevance_threshold)

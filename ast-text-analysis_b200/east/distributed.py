@@ -14,9 +14,10 @@ join them:
     stores) -- the all-gather happens inside the scoring kernel, row by row; one barrier ends the step;
   * one all_gather_into_tensor of the slices (padded to a common height) -- gloo, ragged batches, no
     symmetric memory.
-Graph.  Co-occurrence counts are additive over documents: every rank computes C_r = B_r B_r^T of its own
-rows on the tensor cores (east_cooc_dev) and ONE all_reduce(int32 sum) of the K x K counts joins them
-(east/applications.py:111-147; SURVEY 5.8).  There is no other exchange on the path.
+Graph.  Co-occurrence counts are additive over documents: every rank indexes its own documents and counts
+C_r = B_r B_r^T of their relevance bytes on the tensor cores (east_graph_dev: the scoring kernel writes the bytes, no
+score table is formed), and ONE all_reduce(int32 sum) of the K x K counts joins them (east/applications.py:111-147;
+SURVEY 5.8).  There is no other exchange on the path.
 """
 import numpy as np
 
@@ -227,15 +228,49 @@ def keyphrases_graph_sharded(keyphrases, texts, referral_confidence=0.6, relevan
                              normalized=True, device=None, group=None, synonimizer=None):
     """applications.keyphrases_graph computed by all ranks together: the same graph dict on every rank.
 
-    texts: {name: text} (same on every rank); documents shard over the ranks, every rank scores its own and
-    counts its own co-occurrences; the K x K counts are all-reduced.  synonimizer: as in keyphrases_graph."""
+    texts: {name: text} (same on every rank); documents shard over the ranks, every rank indexes its own and counts
+    its own co-occurrences with one graph call per device batch (east_graph_dev; several batches are summed on the
+    device); the K x K counts are all-reduced.  No rank forms a score table.  synonimizer: as in keyphrases_graph."""
+    import torch
+    import torch.distributed as dist
+
+    from east import _capi
     from east import applications
     from east import utils
     kept = [kp for kp in keyphrases if kp]
     prepared = [utils.prepare_text(kp) for kp in kept]
     text_collection = list(texts.values())
-    full, (begin, end) = relevance_table_sharded(text_collection, prepared, normalized, device=device, group=group,
-                                                 return_local=True, synonimizer=synonimizer)
-    cooc = cooccurrence_sharded(full[begin:end], relevance_threshold, device=device, group=group)
+    rank = dist.get_rank(group)
+    world = dist.get_world_size(group)
+    if device is None:
+        device = torch.cuda.current_device()
+    dev = torch.device("cuda", device)
+    begin, end = partition_documents([len(t) for t in text_collection], world)[rank]
+    K = len(prepared)
+    cooc = torch.zeros((K, K), dtype=torch.int32, device=dev)
+    cols, packed, batches = _pack_local(text_collection[begin:end]) if end > begin and K else ([], [], [])
+    if batches:
+        group_off = None
+        if synonimizer:
+            codes, off, group_off = _capi.pack_variant_groups(prepared, synonimizer.get_synonyms())
+        else:
+            codes, off = _capi.pack_keyphrases(prepared)
+        stream = torch.cuda.current_stream(dev)
+        kp_dev = torch.from_numpy(codes.view(np.int32).copy()).to(dev)
+        part = torch.empty_like(cooc) if len(batches) > 1 else cooc
+        for b, docs in enumerate(batches):
+            doc_off = np.zeros(len(docs) + 1, dtype=np.int64)
+            np.cumsum([len(packed[j]) for j in docs], out=doc_off[1:])
+            text = np.ascontiguousarray(np.concatenate([packed[j] for j in docs]) if len(docs) > 1 else packed[docs[0]],
+                                        dtype=np.uint32)
+            text_dev = torch.from_numpy(text.view(np.int32)).to(dev)
+            target = cooc if b == 0 else part
+            _capi.DeviceIndex.build_dev_and_graph(text_dev.data_ptr(), doc_off, [len(cols[j]) for j in docs], kp_dev.data_ptr(),
+                                                  codes, off, relevance_threshold, target.data_ptr(), normalized, device=device,
+                                                  stream=stream.cuda_stream, group_off=group_off).close()
+            if b > 0:
+                cooc += part   # int32: exact
+    if world > 1:
+        dist.all_reduce(cooc, op=dist.ReduceOp.SUM, group=group)
     return applications.graph_from_cooccurrence(keyphrases, kept, cooc.cpu().numpy(), referral_confidence,
                                                 relevance_threshold, support_threshold)

@@ -71,8 +71,11 @@ class ASTRelevanceMeasure(RelevanceMeasure):
         self._table = None
         self._table_keyphrases = None
         self._table_groups = None
+        self._cooc = None
+        self._cooc_key = None
 
-    def set_text_collection(self, texts, language=consts.Language.ENGLISH, prepared_keyphrases=None, synonimizer=None):
+    def set_text_collection(self, texts, language=consts.Language.ENGLISH, prepared_keyphrases=None, synonimizer=None,
+                            relevance_threshold=None):
         """relevance.py:34-49: one AST per text; here all of them in one batched build.
 
         prepared_keyphrases (optional, what keyphrases_table passes): the keyphrases relevance_table() is
@@ -80,7 +83,11 @@ class ASTRelevanceMeasure(RelevanceMeasure):
         scoring of the documents already indexed with the transfer of the rest (east_table_host).
         synonimizer (optional, with prepared_keyphrases): the table scored while indexing is the synonym table of
         relevance_table(prepared_keyphrases, synonimizer) -- the best variant of each keyphrase, always normalized
-        (east_table_groups_host / east_table_texts_groups_host)."""
+        (east_table_groups_host / east_table_texts_groups_host).
+        relevance_threshold (optional, with prepared_keyphrases): what keyphrases_graph passes.  Each batch is then built
+        and counted by one graph call instead (east_graph_host / east_graph_texts_host): the co-occurrence counts of
+        cooccurrence(prepared_keyphrases, relevance_threshold, synonimizer) are summed over the batches and no score
+        table is formed."""
         self.texts = texts
         self.language = language
         self.asts = []
@@ -89,6 +96,8 @@ class ASTRelevanceMeasure(RelevanceMeasure):
         self._table = None
         self._table_keyphrases = None
         self._table_groups = None
+        self._cooc = None
+        self._cooc_key = None
         total_texts = len(texts)
         if self.ast_algorithm not in tuple(consts.ASTAlgorithm):
             # other registered engines (none ship in this package) go through the registry
@@ -103,8 +112,10 @@ class ASTRelevanceMeasure(RelevanceMeasure):
         # the synonym variants are expanded and packed once: the same arrays go to every device batch
         groups = (_capi.pack_variant_groups(prepared_keyphrases, synonimizer.get_synonyms())
                   if prepared_keyphrases and synonimizer else None)
+        graph = bool(prepared_keyphrases) and relevance_threshold is not None
+        threshold = relevance_threshold if graph else None
         if prepared_keyphrases and self.device_preprocessing and self._set_text_collection_on_device(texts, prepared_keyphrases,
-                                                                                                    groups):
+                                                                                                    groups, threshold):
             return
         collections = [utils.text_to_strings_collection(text) for text in texts]
         # one byte per code point where the text allows it (ASCII / Latin-1: a quarter of the bytes over the host link),
@@ -115,7 +126,8 @@ class ASTRelevanceMeasure(RelevanceMeasure):
         # everything is built into locals: a batch that raises leaves the measure empty, not half-initialised
         asts = [None] * len(collections)
         batches = []
-        table = np.empty((len(collections), len(prepared_keyphrases)), dtype=np.float64) if fused else None
+        table = np.empty((len(collections), len(prepared_keyphrases)), dtype=np.float64) if fused and not graph else None
+        cooc = None
         for docs in plan_batches([len(p) for p in packed]):
             narrow = all(packed[j].dtype == np.uint8 for j in docs)
             parts = [packed[j] if narrow or packed[j].dtype == np.uint32 else asts_utils.pack_strings_collection(collections[j])
@@ -127,6 +139,11 @@ class ASTRelevanceMeasure(RelevanceMeasure):
             if fused is None:
                 build = _capi.DeviceIndex.build_host_u8 if narrow else _capi.DeviceIndex.build_host
                 index = build(text, doc_off, doc_m, device=self.device)
+            elif graph:
+                counts, index = _capi.DeviceIndex.build_host_and_graph(text, doc_off, doc_m, fused[0], fused[1], threshold,
+                                                                       normalized=self.normalized, device=self.device,
+                                                                       group_off=groups[2] if groups else None)
+                cooc = counts if cooc is None else cooc + counts   # int32: exact (counts <= number of texts)
             else:
                 rows = np.empty((len(docs), len(prepared_keyphrases)), dtype=np.float64)
                 index = _capi.DeviceIndex.build_host_and_score(text, doc_off, doc_m, fused[0], fused[1], rows,
@@ -137,15 +154,21 @@ class ASTRelevanceMeasure(RelevanceMeasure):
             for local, j in enumerate(docs):
                 asts[j] = easa.EnhancedAnnotatedSuffixArray(collections[j], _index=index, _doc=local)
         self.asts, self._batches, self._index = asts, batches, batches[0][0]
-        if fused:
+        if graph:
+            self._cooc, self._cooc_key = cooc, self._counts_key(prepared_keyphrases, groups, threshold)
+        elif fused:
             self._table, self._table_keyphrases, self._table_groups = table, list(prepared_keyphrases), groups
 
-    def _set_text_collection_on_device(self, texts, prepared_keyphrases, groups=None):
+    def _counts_key(self, prepared_keyphrases, groups, threshold):
+        return list(prepared_keyphrases), groups, float(threshold), bool(self.normalized)
+
+    def _set_text_collection_on_device(self, texts, prepared_keyphrases, groups=None, threshold=None):
         """keyphrases_table for a collection of small ASCII / Cyrillic texts: ONE engine call takes the raw texts,
         does the preprocessing of utils.text_to_strings_collection on the device (csrc/tokenize.cu), indexes and scores
         (east_table_texts_host; with groups -- pack_variant_groups -- the synonym table, east_table_texts_groups_host).
         Returns False when the collection needs the host preprocessing (other scripts -- Python's Unicode tables --, a
-        text too large for the per-document kernel, several device batches)."""
+        text too large for the per-document kernel, several device batches).  threshold: the co-occurrence counts of a
+        keyphrase graph instead of the table (east_graph_texts_host)."""
         total = 0
         for t in texts:
             if isinstance(t, (bytes, bytearray)):
@@ -162,16 +185,25 @@ class ASTRelevanceMeasure(RelevanceMeasure):
         if total >= MAX_BATCH_CODE_POINTS:
             return False
         fused = groups[:2] if groups else _capi.pack_keyphrases(prepared_keyphrases)
-        table = np.empty((len(texts), len(prepared_keyphrases)), dtype=np.float64)
+        group_off = groups[2] if groups else None
+        table = None
         try:
-            index = _capi.DeviceIndex.table_from_texts(texts, fused[0], fused[1], table, normalized=self.normalized,
-                                                       device=self.device, group_off=groups[2] if groups else None)
+            if threshold is None:
+                table = np.empty((len(texts), len(prepared_keyphrases)), dtype=np.float64)
+                index = _capi.DeviceIndex.table_from_texts(texts, fused[0], fused[1], table, normalized=self.normalized,
+                                                           device=self.device, group_off=group_off)
+            else:
+                cooc, index = _capi.DeviceIndex.graph_from_texts(texts, fused[0], fused[1], threshold, normalized=self.normalized,
+                                                                 device=self.device, group_off=group_off)
         except _capi.UnsupportedText:
             return False
         docs = list(range(len(texts)))
         self.asts = [easa.EnhancedAnnotatedSuffixArray(None, _index=index, _doc=j) for j in docs]
         self._batches, self._index = [(index, docs)], index
-        self._table, self._table_keyphrases, self._table_groups = table, list(prepared_keyphrases), groups
+        if table is None:
+            self._cooc, self._cooc_key = cooc, self._counts_key(prepared_keyphrases, groups, threshold)
+        else:
+            self._table, self._table_keyphrases, self._table_groups = table, list(prepared_keyphrases), groups
         return True
 
     def save_index(self, directory):
@@ -240,3 +272,21 @@ class ASTRelevanceMeasure(RelevanceMeasure):
         for index, docs in self._batches:
             table[docs] = index.score_table(codes, off, normalized=self.normalized)
         return table
+
+    def cooccurrence(self, prepared_keyphrases, relevance_threshold, synonimizer=None):
+        """int32 [K, K] co-occurrence counts: C[i][j] = number of texts in which prepared keyphrases i and j both score
+        >= relevance_threshold (with a synonimizer: their best synonym variants), C[k][k] the support of k.  The counts
+        of the graph calls made while indexing (set_text_collection with relevance_threshold) when they were made for
+        these keyphrases, variants, threshold and normalization; otherwise those of relevance_table()."""
+        K = len(prepared_keyphrases)
+        if self._cooc is not None:
+            groups = _capi.pack_variant_groups(prepared_keyphrases, synonimizer.get_synonyms()) if synonimizer else None
+            kps, kgroups, kthr, knorm = self._cooc_key
+            same_groups = (groups is None) == (kgroups is None) and (
+                groups is None or all(np.array_equal(a, b) for a, b in zip(groups, kgroups)))
+            if (list(prepared_keyphrases) == kps and same_groups and float(relevance_threshold) == kthr
+                    and bool(self.normalized) == knorm):
+                return self._cooc
+        if not K or not self.asts:
+            return np.zeros((K, K), dtype=np.int32)
+        return _capi.cooc_host(self.relevance_table(prepared_keyphrases, synonimizer), relevance_threshold)

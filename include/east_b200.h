@@ -230,6 +230,33 @@ int east_table_texts_groups_host(const uint8_t *utf8, const int64_t *text_off, i
                                  int32_t G, double *out_DxG, int64_t *doc_off_out /* optional */,
                                  int32_t *doc_m_out /* optional */, east_index **out_idx);
 
+/* ---- keyphrase graphs in one call: build and score as the table entries above, but return the co-occurrence counts
+ * C[i][j] = number of documents in which both column i and column j score >= threshold (applications.py:111-147:
+ * C[k][k] is the support of k), int32, cols x cols row-major, where cols = G with group_off and V without it (group_off
+ * may be NULL: then kp holds V plain keyphrases, space-stripped as for east_table_host, scored with `normalized`; with
+ * group_off the variants of east_table_groups_* are scored, always normalized).  The documents x columns score table is
+ * never formed: the per-document kernel stores one relevance byte per (column, document) -- score >= threshold, the fp64
+ * compare of east_cooc_* -- into the keyphrase-major byte matrix the tensor-core product C = B B^T reads; the paths that
+ * score after the build (batched or tiled scorer, failed speculation, global sort) score bounded tiles of documents and
+ * threshold each tile.  C equals east_cooc_host(table, threshold) of the matching table entry's table element for element.
+ * Arguments, keyphrases and groups are checked before anything is built (EAST_ERR_INVALID, EAST_ERR_ZERODIV for an empty
+ * keyphrase or variant); the _texts_ entry fails with EAST_ERR_UNSUPPORTED as east_table_texts_host does.  Every entry
+ * optionally returns the index (out_idx may be NULL).
+ *   east_graph_host: host text (text_width 4: uint32 code points, 1: one byte per code point), C_host on the host.
+ *   east_graph_dev: device-resident text and keyphrases (kp_host: optional host copy), C_dev on the device, queued on
+ *     `stream` (the call returns once C_dev is written).
+ *   east_graph_texts_host: raw UTF-8 texts, as east_table_texts_host. */
+int east_graph_host(const void *text, int32_t text_width, const int64_t *doc_off, const int32_t *doc_m, int32_t n_docs,
+                    int device, const uint32_t *kp, const int64_t *kp_off, int32_t V, const int64_t *group_off, int32_t G,
+                    int normalized, double threshold, int32_t *C_host, east_index **out_idx);
+int east_graph_dev(const uint32_t *text_dev, const int64_t *doc_off, const int32_t *doc_m, int32_t n_docs, int device,
+                   const uint32_t *kp_dev, const uint32_t *kp_host, const int64_t *kp_off, int32_t V, const int64_t *group_off,
+                   int32_t G, int normalized, double threshold, int32_t *C_dev, void *stream, east_index **out_idx);
+int east_graph_texts_host(const uint8_t *utf8, const int64_t *text_off, int32_t n_texts, int device, const uint32_t *kp,
+                          const int64_t *kp_off, int32_t V, const int64_t *group_off, int32_t G, int normalized,
+                          double threshold, int32_t *C_host, int64_t *doc_off_out /* optional */,
+                          int32_t *doc_m_out /* optional */, east_index **out_idx);
+
 /* ---- persistence: the reference rebuilds every structure on every run (relevance.py:38-47); an index -- packed text,
  * suffix array, LCP, child table, annotation and the scorer's side tables of one batch of documents -- can be written
  * to a file and loaded back onto any device.  Scores and arrays of a loaded index are identical to the saved one's. */
