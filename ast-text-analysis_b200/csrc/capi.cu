@@ -640,9 +640,8 @@ static int build_common(const uint32_t *text_dev, bool owns_text, const int64_t 
     return EAST_OK;
 }
 
-static void check_build_args(const void *text, const int64_t *doc_off, const int32_t *doc_m, int32_t n_docs,
-                             east_index **out) {
-    if (!text || !doc_off || !doc_m || !out) throw Error(EAST_ERR_INVALID, "NULL argument");
+static void check_documents(const void *text, const int64_t *doc_off, const int32_t *doc_m, int32_t n_docs) {
+    if (!text || !doc_off || !doc_m) throw Error(EAST_ERR_INVALID, "NULL argument");
     if (n_docs <= 0) throw Error(EAST_ERR_INVALID, "n_docs must be positive");
     if (doc_off[0] != 0) throw Error(EAST_ERR_INVALID, "doc_off[0] must be 0");
     for (int i = 0; i < n_docs; ++i) {
@@ -660,7 +659,8 @@ static void build_host_impl(const void *text_any, int width /* bytes per code po
     const uint8_t *text8 = static_cast<const uint8_t *>(text_any);
     static const bool debug = getenv("EAST_DEBUG_TIMING") != nullptr;
     if (debug) fprintf(stderr, "[east] host %.3f ms  east_build_host enter\n", host_now_ms());
-    check_build_args(text_any, doc_off, doc_m, n_docs, out);
+    if (!out) throw Error(EAST_ERR_INVALID, "NULL argument");
+    check_documents(text_any, doc_off, doc_m, n_docs);
     use_device(device);
     const int64_t n = doc_off[n_docs];
     const size_t bytes = sizeof(uint32_t) * (size_t)n;
@@ -753,7 +753,8 @@ int east_build_host_u8(const uint8_t *text8, const int64_t *doc_off, const int32
 int east_build_dev(const uint32_t *text_dev, const int64_t *doc_off, const int32_t *doc_m, int32_t n_docs,
                    int device, void *stream, east_index **out) {
     EAST_API_BEGIN
-    check_build_args(text_dev, doc_off, doc_m, n_docs, out);
+    if (!out) throw Error(EAST_ERR_INVALID, "NULL argument");
+    check_documents(text_dev, doc_off, doc_m, n_docs);
     use_device(device);
     build_common(text_dev, false, doc_off, doc_m, n_docs, device, (cudaStream_t)stream, out);
     EAST_API_END
@@ -858,14 +859,6 @@ static void drop_kp_cache() {
     cudaDeviceSynchronize();
     g_kp_cache.reset();
     cudaSetDevice(cur);
-}
-
-static void check_keyphrases(const int64_t *kp_off, int32_t K) {
-    if (kp_off[K] >= (1ll << 31)) throw Error(EAST_ERR_RANGE, "keyphrase buffer too large");
-    for (int32_t k = 0; k < K; ++k) {
-        if (kp_off[k + 1] <= kp_off[k]) throw Error(EAST_ERR_ZERODIV, "empty query: float division by zero");
-        if (kp_off[k + 1] - kp_off[k] > 0xffff) throw Error(EAST_ERR_RANGE, "keyphrase longer than 65535 code points");
-    }
 }
 
 // The host variant of kp_prep.cu (round 1; option "kp_prep_host" = 1, kept as the cross-check of the device pipeline):
@@ -1046,10 +1039,180 @@ static void kp_finish(KpPrepared *c, const uint32_t *kp_dev, bool fast, int sym_
     c->finished = true;
 }
 
+// ---- what a call scores, where its results go, where its documents come from ---------------------------------------
+// The keyphrases of a call -- or, grouped, the synonym variants of east_*_groups_*: K variants in G groups and a row G
+// wide.  kp_off and group_off are host arrays; the code points come from the host (uploaded by the call into kp_dev)
+// or from the device (kp_host: an optional host copy).
+struct Query {
+    const uint32_t *kp_dev = nullptr, *kp_host = nullptr;
+    bool on_host = false;
+    const int64_t *kp_off = nullptr;
+    int32_t K = 0;
+    int normalized = 0;
+    bool grouped = false;
+    const int64_t *group_off = nullptr;
+    int32_t G = 0;
+    DevBuf<int32_t> d_groups;   // the device copy of group_off (upload_groups)
+    Query(const uint32_t *kp, bool on_host_, const uint32_t *kp_host_copy, const int64_t *kp_off_, int32_t K_, int normalized_,
+          bool grouped_ = false, const int64_t *group_off_ = nullptr, int32_t G_ = 0)
+        : kp_dev(on_host_ ? nullptr : kp), kp_host(on_host_ ? kp : kp_host_copy), on_host(on_host_), kp_off(kp_off_), K(K_),
+          normalized(grouped_ ? 1 : (normalized_ ? 1 : 0)),   // groups are always normalized, as the reference's synonym branch
+          grouped(grouped_), group_off(grouped_ ? group_off_ : nullptr), G(grouped_ ? G_ : 0) {}
+    int32_t cols() const { return grouped ? G : K; }
+    int64_t total() const { return kp_off[K]; }
+    // the device copy of host code points, queued on `s`
+    DevBuf<uint32_t> upload(cudaStream_t s) {
+        DevBuf<uint32_t> d((size_t)total(), s);
+        EAST_CUDA(cudaMemcpyAsync(d.p, kp_host, sizeof(uint32_t) * (size_t)total(), cudaMemcpyHostToDevice, s));
+        kp_dev = d.p;
+        return d;
+    }
+    // int32 offsets: < 2^31 variants, each has a code point of the keyphrase buffer (check_keyphrases); uploaded once, on
+    // `s` (the pageable host vector is staged before the copy call returns)
+    void upload_groups(cudaStream_t s) {
+        if (!grouped || d_groups.p) return;
+        const std::vector<int32_t> g32(group_off, group_off + G + 1);
+        d_groups = DevBuf<int32_t>((size_t)G + 1, s);
+        EAST_CUDA(cudaMemcpyAsync(d_groups.p, g32.data(), sizeof(int32_t) * ((size_t)G + 1), cudaMemcpyHostToDevice, s));
+    }
+};
+
+// tcgen05 kernel of the co-occurrence counts (option cooc_variant: 2 = the 128 x 128 kernel, 3 = the cp.async pipeline,
+// otherwise the TMA-fed cluster kernel; 1 selects the AND + POPC kernel of east_cooc_*, which reads the score table)
+static int cooc_tc_kernel() {
+    const int64_t v = get_option("cooc_variant", 0);
+    return v == 2 ? 1 : (v == 3 ? 2 : 0);
+}
+
+// ---- keyphrase graphs: relevance bytes instead of a score table ------------------------------------------------------
+// A graph call fills B[k][d] = (score of document d in column k >= threshold), the zero-padded Kp x Dp byte matrix of the
+// co-occurrence GEMM (cooc_tc.cu), and never a documents x keyphrases table: the per-document kernel stores its column of
+// bytes itself (k_doc_suffix_sort_graph); every other path scores tiles of documents into an fp64 scratch bounded by the
+// score_tmp_doubles budget and thresholds each tile into its columns (graph_enqueue).
+struct GraphOut {
+    double threshold = 0.0;
+    int32_t *C = nullptr;   // device: cols x cols counts
+    DevBuf<uint8_t> B;
+    int64_t Dp = 0;
+    int32_t Kp = 0;
+    void begin(int32_t n_docs, int32_t cols, cudaStream_t s) {
+        cooc_padding(n_docs, cols, &Dp, &Kp);
+        B = DevBuf<uint8_t>((size_t)Kp * (size_t)Dp, s);
+        EAST_CUDA(cudaMemsetAsync(B.p, 0, (size_t)Kp * (size_t)Dp, s));   // padding rows / columns stay zero
+    }
+    void finish(int32_t cols, cudaStream_t s) const { cooc_counts_bytes(B.p, Dp, Kp, cols, C, s, cooc_tc_kernel()); }
+};
+
+// Where a call's results go: the rows of a table on the device (the caller's; host entries: the call's own, copied to
+// the host), optionally stored into the other ranks' tables too, or the counts of a keyphrase graph (to a device
+// pointer, or copied to a host pointer).
+struct Output {
+    double *rows = nullptr;              // device, n_docs x cols
+    bool to_host = false;
+    double *rows_host = nullptr;         // to_host: the host copy of the rows
+    double *const *peer_rows = nullptr;  // sharded table: where this rank's rows start in every other rank's table
+    int32_t n_peers = 0;
+    bool is_graph = false;
+    GraphOut graph;                      // is_graph: counts into graph.C ...
+    int32_t *counts_host = nullptr;      // ... or, given this, into the call's own buffer and then here
+    DevBuf<double> own_rows;
+    DevBuf<int32_t> own_counts;
+
+    static Output table_dev(double *rows, double *const *peer_rows = nullptr, int32_t n_peers = 0) {
+        Output o;
+        o.rows = rows; o.peer_rows = peer_rows; o.n_peers = n_peers;
+        return o;
+    }
+    // rows_dev: where the rows also go on the device (NULL: a buffer of the call)
+    static Output table_host(double *host, double *rows_dev = nullptr, double *const *peer_rows = nullptr, int32_t n_peers = 0) {
+        Output o = table_dev(rows_dev, peer_rows, n_peers);
+        o.to_host = true; o.rows_host = host;
+        return o;
+    }
+    static Output counts(double threshold, int32_t *C_dev, int32_t *C_host) {
+        Output o;
+        o.is_graph = true; o.graph.threshold = threshold; o.graph.C = C_dev; o.counts_host = C_host;
+        return o;
+    }
+    void begin(int32_t n_docs, int32_t cols, cudaStream_t s) {
+        if (is_graph) {
+            if (counts_host) {
+                own_counts = DevBuf<int32_t>((size_t)cols * cols, s);
+                graph.C = own_counts.p;
+            }
+            graph.begin(n_docs, cols, s);
+        } else if (!rows) {
+            own_rows = DevBuf<double>((size_t)n_docs * cols, s);
+            rows = own_rows.p;
+        }
+    }
+};
+
+// Where a build-and-score call's documents come from: packed text on the host (width 4: uint32 code points, 1: one byte
+// per code point), packed text on the device, or raw UTF-8 texts (doc_off: their byte offsets) that the call packs on
+// the device into a text the index then owns, also returning the packed offsets and string counts when asked.
+struct Source {
+    enum Kind { HOST, DEVICE, TEXTS } kind;
+    const void *text;
+    int width;                           // HOST: 4 or 1 (text_width); DEVICE: 4; TEXTS: 1
+    const int64_t *doc_off;
+    const int32_t *doc_m;                // TEXTS: NULL
+    int32_t n_docs;
+    int device;
+    cudaStream_t stream = 0;
+    int64_t *doc_off_out = nullptr;      // TEXTS, optional
+    int32_t *doc_m_out = nullptr;
+};
+
+static void check_keyphrases(const int64_t *kp_off, int32_t K) {
+    if (kp_off[K] >= (1ll << 31)) throw Error(EAST_ERR_RANGE, "keyphrase buffer too large");
+    for (int32_t k = 0; k < K; ++k) {
+        if (kp_off[k + 1] <= kp_off[k]) throw Error(EAST_ERR_ZERODIV, "empty query: float division by zero");
+        if (kp_off[k + 1] - kp_off[k] > 0xffff) throw Error(EAST_ERR_RANGE, "keyphrase longer than 65535 code points");
+    }
+}
+
+// the host-side checks of raw UTF-8 texts (texts_to_packed)
+static void check_texts(const uint8_t *utf8, const int64_t *text_off, int32_t n_texts) {
+    if (!utf8 || !text_off || n_texts <= 0) throw Error(EAST_ERR_INVALID, "bad argument");
+    if (text_off[0] != 0) throw Error(EAST_ERR_INVALID, "text_off[0] must be 0");
+    for (int32_t i = 0; i < n_texts; ++i)
+        if (text_off[i + 1] < text_off[i]) throw Error(EAST_ERR_INVALID, "text offsets must not decrease");
+    if (text_off[n_texts] >= (1ll << 31)) throw Error(EAST_ERR_RANGE, "more than 2^31 bytes of text in one call; split the collection");
+}
+
+// The argument checks of every build-and-score and score entry, made before its first CUDA call, in one order (see
+// include/east_b200.h): the output, peers and text_width; the documents (raw texts: their offsets; a score call on an
+// index: the index and the document range [doc_begin, doc_begin + doc_count)); the groups; the keyphrases.
+static void validate(const Output &out, const Source *src, const Query &q, const east_index *idx = nullptr,
+                     int32_t doc_begin = 0, int32_t doc_count = 0) {
+    if (out.is_graph ? !out.graph.C && !out.counts_host : !(out.to_host ? out.rows_host : out.rows))
+        throw Error(EAST_ERR_INVALID, "bad argument");
+    if (out.n_peers < 0 || out.n_peers > DocScore::MAX_PEERS || (out.n_peers > 0 && !out.peer_rows))
+        throw Error(EAST_ERR_INVALID, "bad peer list");
+    if (src && src->width != 1 && src->width != 4) throw Error(EAST_ERR_INVALID, "text_width must be 1 or 4");
+    if (!src) {
+        if (!idx) throw Error(EAST_ERR_INVALID, "bad argument");
+        if (doc_begin < 0 || doc_count <= 0 || (int64_t)doc_begin + doc_count > idx->n_docs) throw Error(EAST_ERR_INVALID, "bad document range");
+    } else if (src->kind == Source::TEXTS) {
+        check_texts(static_cast<const uint8_t *>(src->text), src->doc_off, src->n_docs);
+    } else {
+        check_documents(src->text, src->doc_off, src->doc_m, src->n_docs);
+    }
+    if (q.grouped) {   // V variants in G groups, every group non-empty, the offsets ending at V
+        if (!q.group_off || q.G < 1) throw Error(EAST_ERR_INVALID, "no groups of variants");
+        if (q.group_off[0] != 0 || q.group_off[q.G] != q.K) throw Error(EAST_ERR_INVALID, "group offsets must run from 0 to the number of variants");
+        for (int32_t g = 0; g < q.G; ++g)
+            if (q.group_off[g + 1] <= q.group_off[g]) throw Error(EAST_ERR_INVALID, "empty group of variants");
+    }
+    if (!q.kp_off || q.K <= 0) throw Error(EAST_ERR_INVALID, "bad argument");
+    check_keyphrases(q.kp_off, q.K);
+    if (!(q.on_host ? q.kp_host : q.kp_dev)) throw Error(EAST_ERR_INVALID, "bad argument");
+}
+
 // score calls on an existing index: what was prepared for the previous call is kept (exact match of the code points)
 static KpPrepared *prepare_keyphrases(const east_index *idx, const uint32_t *kp_dev, const uint32_t *kp_host_in,
                                       const int64_t *kp_off, int32_t K, bool dedup, cudaStream_t s) {
-    check_keyphrases(kp_off, K);
     const int64_t total = kp_off[K];
     const bool fast = idx->bkt && idx->t8 && !get_option("score_generic", 0);
     std::vector<uint32_t> kp_host;
@@ -1076,23 +1239,20 @@ static KpPrepared *prepare_keyphrases(const east_index *idx, const uint32_t *kp_
 }
 
 // The launches that score documents [doc_begin, doc_begin + doc_count) of `idx` (tile_docs at a time through the
-// scratch tmp[tile_docs][n_uniq]) into out_dev[(d - doc_begin) * K + k] (with groups: [(d - doc_begin) * G + g]);
-// nothing here waits for the device.
-static void score_enqueue(const east_index *idx, const KpPrepared *kp, const uint32_t *kp_dev, int64_t total, int32_t K,
-                          int normalized, double *out_dev, int32_t doc_begin, int32_t doc_count, cudaStream_t s,
-                          double *tmp, int32_t tile_docs, unsigned long long *probe_count,
+// scratch tmp[tile_docs][n_uniq]) into out_dev[(d - doc_begin) * cols + column]; with groups, q's groups must have been
+// uploaded.  Nothing here waits for the device.
+static void score_enqueue(const east_index *idx, const KpPrepared *kp, const Query &q, double *out_dev, int32_t doc_begin,
+                          int32_t doc_count, cudaStream_t s, double *tmp, int32_t tile_docs, unsigned long long *probe_count,
                           double *const *peer_rows = nullptr /* sharded table: rows of document doc_begin in the peers' tables */,
-                          int32_t n_peers = 0,
-                          const int32_t *group_off_dev = nullptr /* synonym-expanded scoring: G + 1 offsets of the variant groups */,
-                          int32_t G = 0) {
+                          int32_t n_peers = 0) {
     ensure_suffix_keys(idx, s);
-    const int32_t cols = group_off_dev ? G : K;   // columns of out_dev
+    const int32_t cols = q.cols();   // columns of out_dev
     ScoreInput in;
     in.text = idx->text; in.sa = idx->sa;
     in.doc_off = idx->d_doc_off + doc_begin; in.doc_m = idx->d_doc_m + doc_begin; in.n_docs = doc_count;
-    in.kp = kp_dev; in.kp_off = kp->dev.d_off.p; in.K = K; in.total_suffixes = (int32_t)total;
+    in.kp = q.kp_dev; in.kp_off = kp->dev.d_off.p; in.K = q.K; in.total_suffixes = (int32_t)q.total();
     in.uniq_of = kp->dev.d_uniq_of.p; in.recs = kp->dev.d_recs.p; in.n_uniq = (int32_t)kp->n_uniq;
-    in.normalized = normalized ? 1 : 0;
+    in.normalized = q.normalized;
     if (kp->fast) {
         in.t8 = idx->t8; in.sk = idx->sk; in.q8 = kp->dev.d_q8.p; in.sym_bits = idx->sym_bits;
         in.bkt = idx->bkt + ((size_t)doc_begin << (2 * idx->sym_bits));
@@ -1100,7 +1260,7 @@ static void score_enqueue(const east_index *idx, const KpPrepared *kp, const uin
     }
     in.algorithmic_bytes = (double)get_option("score_bytes", 0);
     in.probe_count = probe_count;
-    in.group_off = group_off_dev; in.G = G;
+    in.group_off = q.d_groups.p; in.G = q.G;
     auto tile = [&](int32_t d0, int32_t cnt) {
         ScoreInput part = in;
         part.n_docs = cnt;
@@ -1150,41 +1310,6 @@ static void score_enqueue(const east_index *idx, const KpPrepared *kp, const uin
     }
 }
 
-// the device copy of a call's group offsets (int32: < 2^31 variants, each has a code point of the keyphrase buffer --
-// check_keyphrases); the host vector may go once this returns (pageable source: staged before the call returns)
-static DevBuf<int32_t> upload_groups(const int64_t *group_off, int32_t G, cudaStream_t s) {
-    const std::vector<int32_t> g32(group_off, group_off + G + 1);
-    DevBuf<int32_t> d((size_t)G + 1, s);
-    EAST_CUDA(cudaMemcpyAsync(d.p, g32.data(), sizeof(int32_t) * ((size_t)G + 1), cudaMemcpyHostToDevice, s));
-    return d;
-}
-
-// tcgen05 kernel of the co-occurrence counts (option cooc_variant: 2 = the 128 x 128 kernel, 3 = the cp.async pipeline,
-// otherwise the TMA-fed cluster kernel; 1 selects the AND + POPC kernel of east_cooc_*, which reads the score table)
-static int cooc_tc_kernel() {
-    const int64_t v = get_option("cooc_variant", 0);
-    return v == 2 ? 1 : (v == 3 ? 2 : 0);
-}
-
-// ---- keyphrase graphs: relevance bytes instead of a score table ------------------------------------------------------
-// A graph call fills B[k][d] = (score of document d in column k >= threshold), the zero-padded Kp x Dp byte matrix of the
-// co-occurrence GEMM (cooc_tc.cu), and never a documents x keyphrases table: the per-document kernel stores its column of
-// bytes itself (k_doc_suffix_sort_graph); every other path scores tiles of documents into an fp64 scratch bounded by the
-// score_tmp_doubles budget and thresholds each tile into its columns (graph_enqueue).
-struct GraphOut {
-    double threshold = 0.0;
-    int32_t *C = nullptr;   // device: cols x cols counts
-    DevBuf<uint8_t> B;
-    int64_t Dp = 0;
-    int32_t Kp = 0;
-    void begin(int32_t n_docs, int32_t cols, cudaStream_t s) {
-        cooc_padding(n_docs, cols, &Dp, &Kp);
-        B = DevBuf<uint8_t>((size_t)Kp * (size_t)Dp, s);
-        EAST_CUDA(cudaMemsetAsync(B.p, 0, (size_t)Kp * (size_t)Dp, s));   // padding rows / columns stay zero
-    }
-    void finish(int32_t cols, cudaStream_t s) const { cooc_counts_bytes(B.p, Dp, Kp, cols, C, s, cooc_tc_kernel()); }
-};
-
 // documents per tile of a graph call's fp64 scratch
 static int32_t graph_tile_docs(int32_t doc_count, int32_t cols) {
     const int64_t budget = get_option("score_tmp_doubles", (int64_t)1 << 27);
@@ -1193,29 +1318,24 @@ static int32_t graph_tile_docs(int32_t doc_count, int32_t cols) {
 
 // score_enqueue for a graph: documents [doc_begin, doc_begin + doc_count) tile by tile into S[S_docs][cols], each tile
 // thresholded into its columns of g.B (stream-ordered: the next tile overwrites S after the previous one is read)
-static void graph_enqueue(const east_index *idx, const KpPrepared *kp, const uint32_t *kp_dev, int64_t total, int32_t K,
-                          int normalized, int32_t doc_begin, int32_t doc_count, cudaStream_t s, double *tmp, int32_t tile_docs,
-                          const int32_t *group_off_dev, int32_t G, const GraphOut &g, double *S, int32_t S_docs) {
-    const int32_t cols = group_off_dev ? G : K;
+static void graph_enqueue(const east_index *idx, const KpPrepared *kp, const Query &q, int32_t doc_begin, int32_t doc_count,
+                          cudaStream_t s, double *tmp, int32_t tile_docs, const GraphOut &g, double *S, int32_t S_docs) {
     for (int32_t d0 = 0; d0 < doc_count; d0 += S_docs) {
         const int32_t cnt = std::min(S_docs, doc_count - d0);
-        score_enqueue(idx, kp, kp_dev, total, K, normalized, S, doc_begin + d0, cnt, s, tmp, tile_docs, nullptr, nullptr, 0,
-                      group_off_dev, G);
-        threshold_bytes(S, cnt, cols, g.threshold, g.B.p, g.Dp, (int64_t)doc_begin + d0, s);
+        score_enqueue(idx, kp, q, S, doc_begin + d0, cnt, s, tmp, tile_docs, nullptr);
+        threshold_bytes(S, cnt, q.cols(), g.threshold, g.B.p, g.Dp, (int64_t)doc_begin + d0, s);
     }
 }
 
-static void score_common(const east_index *idx, const uint32_t *kp_dev, const int64_t *kp_off, int32_t K,
-                         int normalized, double *out_dev, int32_t doc_begin, int32_t doc_count, cudaStream_t s,
-                         double *suffix_out_dev /* optional: per-suffix results of the doc range */,
-                         int64_t *probes_out = nullptr /* optional: run the probe-counting scorer */,
-                         const uint32_t *kp_host = nullptr /* optional: the same code points on the host */,
-                         const int64_t *group_off = nullptr /* optional: the K queries are variants in G groups (host, G + 1) */,
-                         int32_t G = 0, const GraphOut *graph = nullptr /* relevance bytes instead of out_dev */) {
+// documents [doc_begin, doc_begin + doc_count) of `idx` scored into out_dev, or into the relevance bytes of `graph`
+static void score_common(const east_index *idx, Query &q, double *out_dev, const GraphOut *graph, int32_t doc_begin,
+                         int32_t doc_count, cudaStream_t s,
+                         double *suffix_out_dev = nullptr /* optional: per-suffix results of the doc range */,
+                         int64_t *probes_out = nullptr /* optional: run the probe-counting scorer */) {
     // per-suffix results wanted (return_suffix_scores): every suffix is its own "distinct" suffix
     const bool dedup = !suffix_out_dev && !get_option("score_no_dedup", 0);
-    KpPrepared *kp = prepare_keyphrases(idx, kp_dev, kp_host, kp_off, K, dedup, s);
-    const int64_t total = kp_off[K], n_uniq = kp->n_uniq;
+    KpPrepared *kp = prepare_keyphrases(idx, q.kp_dev, q.kp_host, q.kp_off, q.K, dedup, s);
+    const int64_t n_uniq = kp->n_uniq;
 
     // per-suffix results tmp[doc][distinct suffix] are produced and consumed tile by tile over the documents,
     // so the scratch stays <= ~1 GB however large K x D is (config 4: 0.63 M distinct suffixes x 12 500 docs)
@@ -1228,8 +1348,7 @@ static void score_common(const east_index *idx, const uint32_t *kp_dev, const in
         tmp_own = DevBuf<double>((size_t)tile_docs * (size_t)n_uniq, s);
         tmp = tmp_own.p;
     }
-    DevBuf<int32_t> d_groups;
-    if (group_off) d_groups = upload_groups(group_off, G, s);
+    q.upload_groups(s);
     DevBuf<unsigned long long> d_probes;
     if (probes_out) {
         d_probes = DevBuf<unsigned long long>(1, s);
@@ -1238,13 +1357,11 @@ static void score_common(const east_index *idx, const uint32_t *kp_dev, const in
     StageTimer tm(s);
     tm.mark("score");
     if (graph) {
-        const int32_t S_docs = graph_tile_docs(doc_count, group_off ? G : K);
-        DevBuf<double> S((size_t)S_docs * (group_off ? G : K), s);
-        graph_enqueue(idx, kp, kp_dev, total, K, normalized, doc_begin, doc_count, s, tmp, tile_docs, d_groups.p, G, *graph, S.p,
-                      S_docs);
+        const int32_t S_docs = graph_tile_docs(doc_count, q.cols());
+        DevBuf<double> S((size_t)S_docs * q.cols(), s);
+        graph_enqueue(idx, kp, q, doc_begin, doc_count, s, tmp, tile_docs, *graph, S.p, S_docs);
     } else {
-        score_enqueue(idx, kp, kp_dev, total, K, normalized, out_dev, doc_begin, doc_count, s, tmp, tile_docs, d_probes.p, nullptr, 0,
-                      d_groups.p, G);
+        score_enqueue(idx, kp, q, out_dev, doc_begin, doc_count, s, tmp, tile_docs, d_probes.p);
     }
     tm.finish();
     if (probes_out) {
@@ -1257,88 +1374,135 @@ static void score_common(const east_index *idx, const uint32_t *kp_dev, const in
     tm.collect();
 }
 
+// The score calls on an index: checked, then scored; the host entries upload the code points and copy the rows back.
+static void score_index(const east_index *idx, Query q, Output out, int32_t doc_begin, int32_t doc_count, void *stream,
+                        int64_t *probes = nullptr) {
+    validate(out, nullptr, q, idx, doc_begin, doc_count);
+    EAST_CUDA(cudaSetDevice(idx->device));
+    cudaStream_t s = (cudaStream_t)stream;
+    DevBuf<uint32_t> d_kp;
+    if (q.on_host) d_kp = q.upload(s);
+    out.begin(doc_count, q.cols(), s);
+    score_common(idx, q, out.rows, nullptr, doc_begin, doc_count, s, nullptr, probes);
+    if (out.to_host) EAST_CUDA(cudaMemcpy(out.rows_host, out.rows, sizeof(double) * (size_t)doc_count * q.cols(), cudaMemcpyDeviceToHost));
+}
+
 int east_score_table_dev(const east_index *idx, const uint32_t *kp_dev, const int64_t *kp_off, int32_t K,
                          int normalized, double *out_DxK_dev, void *stream) {
     EAST_API_BEGIN
-    if (!idx || !kp_dev || !kp_off || !out_DxK_dev || K <= 0) throw Error(EAST_ERR_INVALID, "bad argument");
-    EAST_CUDA(cudaSetDevice(idx->device));
-    score_common(idx, kp_dev, kp_off, K, normalized, out_DxK_dev, 0, idx->n_docs, (cudaStream_t)stream, nullptr);
+    score_index(idx, Query(kp_dev, false, nullptr, kp_off, K, normalized), Output::table_dev(out_DxK_dev), 0,
+                idx ? idx->n_docs : 0, stream);
     EAST_API_END
 }
 
 int east_score_range_dev(const east_index *idx, const uint32_t *kp_dev, const int64_t *kp_off, int32_t K, int normalized,
                          int32_t doc_begin, int32_t doc_count, double *out_dev, void *stream) {
     EAST_API_BEGIN
-    if (!idx || !kp_dev || !kp_off || !out_dev || K <= 0) throw Error(EAST_ERR_INVALID, "bad argument");
-    if (doc_begin < 0 || doc_count <= 0 || doc_begin + doc_count > idx->n_docs) throw Error(EAST_ERR_INVALID, "bad document range");
-    EAST_CUDA(cudaSetDevice(idx->device));
-    score_common(idx, kp_dev, kp_off, K, normalized, out_dev, doc_begin, doc_count, (cudaStream_t)stream, nullptr);
+    score_index(idx, Query(kp_dev, false, nullptr, kp_off, K, normalized), Output::table_dev(out_dev), doc_begin, doc_count,
+                stream);
     EAST_API_END
 }
 
 int east_score_probes_dev(const east_index *idx, const uint32_t *kp_dev, const int64_t *kp_off, int32_t K,
                           double *out_DxK_dev, void *stream, int64_t *probes) {
     EAST_API_BEGIN
-    if (!idx || !kp_dev || !kp_off || !out_DxK_dev || !probes || K <= 0) throw Error(EAST_ERR_INVALID, "bad argument");
-    EAST_CUDA(cudaSetDevice(idx->device));
-    score_common(idx, kp_dev, kp_off, K, 1, out_DxK_dev, 0, idx->n_docs, (cudaStream_t)stream, nullptr, probes);
+    score_index(idx, Query(kp_dev, false, nullptr, kp_off, K, 1),
+                Output::table_dev(probes ? out_DxK_dev : nullptr /* the probe count is an output too */), 0,
+                idx ? idx->n_docs : 0, stream, probes);
     EAST_API_END
-}
-
-// synonym-expanded scoring: V variants in G groups, every group non-empty, the offsets ending at V
-static void check_groups(const int64_t *group_off, int32_t G, int32_t V) {
-    if (!group_off || G < 1) throw Error(EAST_ERR_INVALID, "no groups of variants");
-    if (group_off[0] != 0 || group_off[G] != V) throw Error(EAST_ERR_INVALID, "group offsets must run from 0 to the number of variants");
-    for (int32_t g = 0; g < G; ++g)
-        if (group_off[g + 1] <= group_off[g]) throw Error(EAST_ERR_INVALID, "empty group of variants");
-}
-
-static void check_groups_call(const east_index *idx, const int64_t *kp_off, int32_t V, const int64_t *group_off, int32_t G,
-                              int32_t doc_begin, int32_t doc_count) {
-    if (!idx || !kp_off || V <= 0) throw Error(EAST_ERR_INVALID, "bad argument");
-    if (doc_begin < 0 || doc_count <= 0 || (int64_t)doc_begin + doc_count > idx->n_docs) throw Error(EAST_ERR_INVALID, "bad document range");
-    check_groups(group_off, G, V);
-    check_keyphrases(kp_off, V);
 }
 
 int east_score_groups_dev(const east_index *idx, const uint32_t *kp_dev, const int64_t *kp_off, int32_t V,
                           const int64_t *group_off, int32_t G, int32_t doc_begin, int32_t doc_count, double *out_dev,
                           void *stream) {
     EAST_API_BEGIN
-    check_groups_call(idx, kp_off, V, group_off, G, doc_begin, doc_count);
-    if (!kp_dev || !out_dev) throw Error(EAST_ERR_INVALID, "bad argument");
-    EAST_CUDA(cudaSetDevice(idx->device));
-    score_common(idx, kp_dev, kp_off, V, 1, out_dev, doc_begin, doc_count, (cudaStream_t)stream, nullptr, nullptr, nullptr,
-                 group_off, G);
+    score_index(idx, Query(kp_dev, false, nullptr, kp_off, V, 1, true, group_off, G), Output::table_dev(out_dev), doc_begin,
+                doc_count, stream);
     EAST_API_END
 }
 
 int east_score_groups_host(const east_index *idx, const uint32_t *kp, const int64_t *kp_off, int32_t V,
                            const int64_t *group_off, int32_t G, int32_t doc_begin, int32_t doc_count, double *out_host) {
     EAST_API_BEGIN
-    check_groups_call(idx, kp_off, V, group_off, G, doc_begin, doc_count);
-    if (!kp || !out_host) throw Error(EAST_ERR_INVALID, "bad argument");
-    EAST_CUDA(cudaSetDevice(idx->device));
-    cudaStream_t s = 0;
-    DevBuf<uint32_t> d_kp((size_t)kp_off[V], s);
-    DevBuf<double> d_out((size_t)doc_count * G, s);
-    EAST_CUDA(cudaMemcpyAsync(d_kp.p, kp, sizeof(uint32_t) * (size_t)kp_off[V], cudaMemcpyHostToDevice, s));
-    score_common(idx, d_kp.p, kp_off, V, 1, d_out.p, doc_begin, doc_count, s, nullptr, nullptr, kp, group_off, G);
-    EAST_CUDA(cudaMemcpy(out_host, d_out.p, sizeof(double) * (size_t)doc_count * G, cudaMemcpyDeviceToHost));
+    score_index(idx, Query(kp, true, nullptr, kp_off, V, 1, true, group_off, G), Output::table_host(out_host), doc_begin,
+                doc_count, 0);
     EAST_API_END
 }
 
 int east_score_table_host(const east_index *idx, const uint32_t *kp, const int64_t *kp_off, int32_t K,
                           int normalized, double *out_DxK) {
     EAST_API_BEGIN
-    if (!idx || !kp || !kp_off || !out_DxK || K <= 0) throw Error(EAST_ERR_INVALID, "bad argument");
+    score_index(idx, Query(kp, true, nullptr, kp_off, K, normalized), Output::table_host(out_DxK), 0, idx ? idx->n_docs : 0, 0);
+    EAST_API_END
+}
+
+int east_score_one(const east_index *idx, int32_t doc, const uint32_t *q, int32_t len, int normalized,
+                   double *score, double *suffix_scores) {
+    EAST_API_BEGIN
+    const int64_t off[2] = {0, q ? len : 0};   // no code points: the empty query
+    Query query(q, true, nullptr, off, 1, normalized);
+    validate(Output::table_host(score), nullptr, query, idx, doc, 1);
     EAST_CUDA(cudaSetDevice(idx->device));
     cudaStream_t s = 0;
-    DevBuf<uint32_t> d_kp((size_t)kp_off[K], s);
-    DevBuf<double> d_out((size_t)idx->n_docs * K, s);
-    EAST_CUDA(cudaMemcpyAsync(d_kp.p, kp, sizeof(uint32_t) * (size_t)kp_off[K], cudaMemcpyHostToDevice, s));
-    score_common(idx, d_kp.p, kp_off, K, normalized, d_out.p, 0, idx->n_docs, s, nullptr, nullptr, kp);
-    EAST_CUDA(cudaMemcpy(out_DxK, d_out.p, sizeof(double) * (size_t)idx->n_docs * K, cudaMemcpyDeviceToHost));
+    DevBuf<uint32_t> d_q = query.upload(s);
+    DevBuf<double> d_out(1, s), d_suf(len, s);
+    score_common(idx, query, d_out.p, nullptr, doc, 1, s, d_suf.p);
+    EAST_CUDA(cudaMemcpy(score, d_out.p, sizeof(double), cudaMemcpyDeviceToHost));
+    if (suffix_scores) EAST_CUDA(cudaMemcpy(suffix_scores, d_suf.p, sizeof(double) * len, cudaMemcpyDeviceToHost));
+    EAST_API_END
+}
+
+// ---- device preprocessing (tokenize.cu) -----------------------------------------------------
+namespace {
+struct PackedTexts {
+    uint32_t *text = nullptr;          // device, owned until released
+    std::vector<int64_t> doc_off;
+    std::vector<int32_t> doc_m;
+    ~PackedTexts() { if (text) dev_free(text, 0); }
+};
+
+// raw UTF-8 texts (host; check_texts has accepted them) -> packed documents on the device; throws EAST_ERR_UNSUPPORTED
+// when a text needs the host path
+void texts_to_packed(const uint8_t *utf8, const int64_t *text_off, int32_t n_texts, cudaStream_t s, PackedTexts &out) {
+    const int64_t bytes = text_off[n_texts];
+    DevBuf<uint8_t> d_raw((size_t)bytes + 16, s);
+    DevBuf<int64_t> d_off((size_t)n_texts + 1, s), d_doc_off((size_t)n_texts + 1, s);
+    DevBuf<int32_t> d_sizes(3 * (size_t)n_texts, s);
+    if (bytes) EAST_CUDA(cudaMemcpyAsync(d_raw.p, utf8, (size_t)bytes, cudaMemcpyHostToDevice, s));
+    EAST_CUDA(cudaMemcpyAsync(d_off.p, text_off, sizeof(int64_t) * ((size_t)n_texts + 1), cudaMemcpyHostToDevice, s));
+    tokenize_texts(d_raw.p, d_off.p, n_texts, d_sizes.p, s);
+    std::vector<int32_t> sizes(3 * (size_t)n_texts);
+    EAST_CUDA(cudaMemcpyAsync(sizes.data(), d_sizes.p, sizeof(int32_t) * sizes.size(), cudaMemcpyDeviceToHost, s));
+    EAST_CUDA(cudaStreamSynchronize(s));
+    out.doc_off.assign((size_t)n_texts + 1, 0);
+    out.doc_m.resize((size_t)n_texts);
+    for (int32_t i = 0; i < n_texts; ++i) {
+        if (sizes[3 * (size_t)i + 2])
+            throw Error(EAST_ERR_UNSUPPORTED, "text " + std::to_string(i) + " has characters outside ASCII / U+0400-045F (or invalid UTF-8): "
+                                              "use the host preprocessing");
+        out.doc_off[(size_t)i + 1] = out.doc_off[(size_t)i] + sizes[3 * (size_t)i];
+        out.doc_m[(size_t)i] = sizes[3 * (size_t)i + 1];
+    }
+    if (out.doc_off.back() >= (1ll << 30)) throw Error(EAST_ERR_RANGE, "more than 2^30 code points in one index; split the batch");
+    EAST_CUDA(cudaMemcpyAsync(d_doc_off.p, out.doc_off.data(), sizeof(int64_t) * out.doc_off.size(), cudaMemcpyHostToDevice, s));
+    out.text = (uint32_t *)dev_alloc(sizeof(uint32_t) * (size_t)out.doc_off.back(), s, true);
+    tokenize_emit(d_raw.p, d_off.p, n_texts, d_doc_off.p, out.text, s);
+    EAST_CUDA(cudaStreamSynchronize(s));   // the staging buffers (and the pageable doc_off upload) end here
+}
+}  // namespace
+
+int east_texts_to_packed_host(const uint8_t *utf8, const int64_t *text_off, int32_t n_texts, int device, uint32_t *packed_out,
+                              int64_t packed_cap, int64_t *doc_off_out, int32_t *doc_m_out) {
+    EAST_API_BEGIN
+    if (!doc_off_out || !doc_m_out) throw Error(EAST_ERR_INVALID, "NULL argument");
+    check_texts(utf8, text_off, n_texts);
+    use_device(device);
+    PackedTexts pt;
+    texts_to_packed(utf8, text_off, n_texts, 0, pt);
+    std::copy(pt.doc_off.begin(), pt.doc_off.end(), doc_off_out);
+    std::copy(pt.doc_m.begin(), pt.doc_m.end(), doc_m_out);
+    if (pt.doc_off.back() > packed_cap || !packed_out) throw Error(EAST_ERR_RANGE, "packed_out is too small (doc_off_out holds the sizes)");
+    EAST_CUDA(cudaMemcpy(packed_out, pt.text, sizeof(uint32_t) * (size_t)pt.doc_off.back(), cudaMemcpyDeviceToHost));
     EAST_API_END
 }
 
@@ -1348,31 +1512,19 @@ int east_score_table_host(const east_index *idx, const uint32_t *kp, const int64
 // later runs of documents, the runs that are already sorted are scored on the stream that sorted them
 // and their rows of the table go back to the host -- copy-in, sort, score and copy-out overlap.
 struct TableRun {
+    Query &q;
+    Output &out;
     const east_index *building = nullptr;
-    const uint32_t *kp_host = nullptr, *d_kp = nullptr;
-    const int64_t *kp_off = nullptr;
-    int32_t K = 0;
-    int normalized = 0;
-    // synonym-expanded table: the K queries are variants in G groups (host offsets; d_groups: their device copy) and
-    // every row is G wide.  group_off NULL: one column per query.
-    const int64_t *group_off = nullptr;
-    int32_t G = 0;
-    DevBuf<int32_t> d_groups;
-    int32_t cols() const { return group_off ? G : K; }
-    double *d_out = nullptr, *host_out = nullptr;   // host_out NULL: the table stays on the device
-    // keyphrase graph: relevance bytes into graph->B instead of rows (d_out, host_out NULL); the batched scorer's rows go
-    // through the per-stream scratch rows[] of rows_docs documents
-    const GraphOut *graph = nullptr;
+    double *host_out = nullptr;           // the host build: each run's rows are copied here as they are scored
+    // the batched scorer's rows of a graph call go through the per-stream scratch rows[] of rows_docs documents
     DevBuf<double> rows[2];
     int32_t rows_docs[2] = {0, 0};
-    double *const *peer_rows = nullptr;             // sharded table: where this rank's rows start in every other rank's table
-    int32_t n_peers = 0;
-    int32_t docs_sent = 0;                          // documents whose rows have reached the peers (current pass)
+    int32_t docs_sent = 0;                // documents whose rows have reached the peers (current pass)
     std::unique_ptr<KpPrepared> kp_own;   // prepared for this call only (a table call is made once per collection)
-    // east_table_dev: stage 1 of the preparation is queued from the build's scan_queued hook (its ~15 launches are host
+    // device builds: stage 1 of the preparation is queued from the build's scan_queued hook (its ~15 launches are host
     // time that hides under the round trip of the alphabet scan); everything it needs:
     int device = 0;
-    bool dedup = true;
+    bool dedup = !get_option("score_no_dedup", 0);
     cudaStream_t kp_stream = nullptr, caller_stream = nullptr;
     cudaEvent_t kp_ready = nullptr;       // dense codes of the current pass queued
     KpPrepared *kp = nullptr;
@@ -1384,6 +1536,7 @@ struct TableRun {
     int32_t docs_scored = 0;         // of the current pass over the batch (a pass starts with document 0)
     int final_pass = 0;              // the last pass was not speculative
     bool failed = false;
+    TableRun(Query &q_, Output &out_, int device_) : q(q_), out(out_), device(device_) {}
     ~TableRun() { if (kp_ready) cudaEventDestroy(kp_ready); }
 };
 
@@ -1403,7 +1556,7 @@ static void table_kp_begin(void *vctx) {
         EAST_CUDA(cudaEventRecord(inputs_ready, t.caller_stream));
         EAST_CUDA(cudaStreamWaitEvent(t.kp_stream, inputs_ready, 0));
         EAST_CUDA(cudaEventDestroy(inputs_ready));
-        t.kp_own = kp_begin(t.device, t.d_kp, t.kp_host, t.kp_off, t.K, t.dedup, false, t.kp_stream, likely_code_table());
+        t.kp_own = kp_begin(t.device, t.q.kp_dev, t.q.kp_host, t.q.kp_off, t.q.K, t.dedup, false, t.kp_stream, likely_code_table());
     } catch (...) {
         t.failed = true;
     }
@@ -1420,6 +1573,7 @@ static int table_lane(TableRun &t, cudaStream_t s) {
 // before the per-document kernel of a run is launched: have it score the run itself when the scratch fits
 static void table_run_begin(void *vctx, const RunReady &r, DocScore &score) {
     TableRun &t = *static_cast<TableRun *>(vctx);
+    const Query &q = t.q;
     try {
         if (r.doc_begin == 0) {   // a new pass over the batch (the first, or the ordinary build after a failed speculation)
             t.failed = false;
@@ -1439,7 +1593,7 @@ static void table_run_begin(void *vctx, const RunReady &r, DocScore &score) {
             table_kp_begin(&t);   // (the builds that do not scan first -- pipelined host build -- have queued it long ago)
             if (!t.kp_own) return;
             host_debug_mark("kp_finish begin");
-            kp_finish(t.kp_own.get(), t.d_kp, fast, v.sym_bits, v.code_table, r.stream);
+            kp_finish(t.kp_own.get(), q.kp_dev, fast, v.sym_bits, v.code_table, r.stream);
             t.kp = t.kp_own.get();
             if (!t.kp_ready) EAST_CUDA(cudaEventCreateWithFlags(&t.kp_ready, cudaEventDisableTiming));
             EAST_CUDA(cudaEventRecord(t.kp_ready, r.stream));
@@ -1451,26 +1605,26 @@ static void table_run_begin(void *vctx, const RunReady &r, DocScore &score) {
         const int64_t n_uniq = std::max<int64_t>(1, t.kp->n_uniq);
         const int64_t budget = get_option("score_tmp_doubles", (int64_t)1 << 27);
         const bool in_kernel = t.kp->fast && (int64_t)r.doc_count * n_uniq <= budget && !get_option("no_fused_score", 0) &&
-                               (!t.group_off || t.G <= DocScore::MAX_GROUPS);   // the groups' maxima fit the shared memory
+                               (!q.grouped || q.G <= DocScore::MAX_GROUPS);   // the groups' maxima fit the shared memory
         const int64_t want = in_kernel ? r.doc_count : std::max<int64_t>(1, std::min<int64_t>(r.doc_count, budget / n_uniq));
         if (t.tmp_docs[li] < want) {
             t.tmp[li] = DevBuf<double>((size_t)want * (size_t)n_uniq, r.stream);
             t.tmp_docs[li] = want;
         }
         if (in_kernel) {
-            score.recs = t.kp->dev.d_recs.p; score.n_uniq = (int32_t)t.kp->n_uniq; score.q8 = t.kp->dev.d_q8.p; score.kp = t.d_kp;
-            score.tmp = t.tmp[li].p; score.normalized = t.normalized ? 1 : 0;
-            score.kp_off = t.kp->dev.d_off.p; score.uniq_of = t.kp->dev.d_uniq_of.p; score.K = t.K;
-            if (t.graph) {
-                score.graph = t.graph->B.p; score.graph_pitch = t.graph->Dp; score.graph_col0 = r.doc_begin;
-                score.threshold = t.graph->threshold;
+            score.recs = t.kp->dev.d_recs.p; score.n_uniq = (int32_t)t.kp->n_uniq; score.q8 = t.kp->dev.d_q8.p; score.kp = q.kp_dev;
+            score.tmp = t.tmp[li].p; score.normalized = q.normalized;
+            score.kp_off = t.kp->dev.d_off.p; score.uniq_of = t.kp->dev.d_uniq_of.p; score.K = q.K;
+            if (t.out.is_graph) {
+                score.graph = t.out.graph.B.p; score.graph_pitch = t.out.graph.Dp; score.graph_col0 = r.doc_begin;
+                score.threshold = t.out.graph.threshold;
             } else {
-                score.out = t.d_out + (size_t)r.doc_begin * t.cols();
+                score.out = t.out.rows + (size_t)r.doc_begin * q.cols();
             }
-            if (t.group_off) { score.group_off = t.d_groups.p; score.G = t.G; }
+            if (q.grouped) { score.group_off = q.d_groups.p; score.G = q.G; }
             score.skip_suffix_keys = get_option("eager_suffix_keys", 0) ? 0 : 1;
-            score.n_peers = t.n_peers;
-            for (int32_t pi = 0; pi < t.n_peers; ++pi) score.peer_out[pi] = t.peer_rows[pi] + (size_t)r.doc_begin * t.cols();
+            score.n_peers = t.out.n_peers;
+            for (int32_t pi = 0; pi < t.out.n_peers; ++pi) score.peer_out[pi] = t.out.peer_rows[pi] + (size_t)r.doc_begin * q.cols();
             score.algorithmic_bytes = (double)get_option("score_bytes", 0) * ((double)r.doc_count / (double)t.view.n_docs);
         }
     } catch (...) {
@@ -1485,26 +1639,26 @@ static void table_run_done(void *vctx, const RunReady &r, int in_kernel) {
     if (t.failed || !t.kp) return;
     try {
         const int li = table_lane(t, r.stream);
-        const int32_t cols = t.cols();
-        if (t.graph) {
+        const int32_t cols = t.q.cols();
+        if (t.out.is_graph) {
             if (!in_kernel) {
                 const int32_t S_docs = graph_tile_docs(r.doc_count, cols);
                 if (t.rows_docs[li] < S_docs) {
                     t.rows[li] = DevBuf<double>((size_t)S_docs * cols, r.stream);
                     t.rows_docs[li] = S_docs;
                 }
-                graph_enqueue(&t.view, t.kp, t.d_kp, t.kp_off[t.K], t.K, t.normalized, r.doc_begin, r.doc_count, r.stream,
-                              t.tmp[li].p, (int32_t)t.tmp_docs[li], t.d_groups.p, t.G, *t.graph, t.rows[li].p, t.rows_docs[li]);
+                graph_enqueue(&t.view, t.kp, t.q, r.doc_begin, r.doc_count, r.stream, t.tmp[li].p, (int32_t)t.tmp_docs[li],
+                              t.out.graph, t.rows[li].p, t.rows_docs[li]);
             }
             t.docs_scored += r.doc_count;
             return;
         }
-        double *rows = t.d_out + (size_t)r.doc_begin * cols;
+        double *rows = t.out.rows + (size_t)r.doc_begin * cols;
         if (!in_kernel) {
-            std::vector<double *> peers((size_t)t.n_peers);
-            for (int32_t pi = 0; pi < t.n_peers; ++pi) peers[(size_t)pi] = t.peer_rows[pi] + (size_t)r.doc_begin * cols;
-            score_enqueue(&t.view, t.kp, t.d_kp, t.kp_off[t.K], t.K, t.normalized, rows, r.doc_begin, r.doc_count, r.stream,
-                          t.tmp[li].p, (int32_t)t.tmp_docs[li], nullptr, peers.data(), t.n_peers, t.d_groups.p, t.G);
+            std::vector<double *> peers((size_t)t.out.n_peers);
+            for (int32_t pi = 0; pi < t.out.n_peers; ++pi) peers[(size_t)pi] = t.out.peer_rows[pi] + (size_t)r.doc_begin * cols;
+            score_enqueue(&t.view, t.kp, t.q, rows, r.doc_begin, r.doc_count, r.stream, t.tmp[li].p, (int32_t)t.tmp_docs[li],
+                          nullptr, peers.data(), t.out.n_peers);
         }
         t.docs_sent += r.doc_count;   // the rows reach the peers from the kernels that produce them, on either path
         if (t.host_out)
@@ -1516,52 +1670,65 @@ static void table_run_done(void *vctx, const RunReady &r, int in_kernel) {
     }
 }
 
-static void table_host_impl(const void *text, int width, const int64_t *doc_off, const int32_t *doc_m, int32_t n_docs, int device,
-                            const uint32_t *kp, const int64_t *kp_off, int32_t K, int normalized, double *out_DxK,
-                            east_index **out_idx, double *own_rows_dev = nullptr, double *const *peer_rows = nullptr,
-                            int32_t n_peers = 0,
-                            const int64_t *group_off = nullptr /* synonym-expanded table: G + 1 offsets of the variant groups */,
-                            int32_t G = 0, GraphOut *graph = nullptr /* keyphrase graph: counts into graph->C, no table */) {
-    if (!kp || !kp_off || (!out_DxK && !graph) || K <= 0) throw Error(EAST_ERR_INVALID, "bad argument");
-    if (n_peers < 0 || n_peers > DocScore::MAX_PEERS || (n_peers > 0 && !peer_rows)) throw Error(EAST_ERR_INVALID, "bad peer list");
-    east_index *built = nullptr;
-    check_build_args(text, doc_off, doc_m, n_docs, &built);
-    check_keyphrases(kp_off, K);
-    use_device(device);
-    cudaStream_t s = 0;
-    // the keyphrases go first, on a side stream: hashing, ordering and de-duplication of their suffixes (kp_prep.cu)
-    // run there while the text is on its way
-    cudaStream_t ps = prep_stream(device);
-    const int32_t cols = group_off ? G : K;
-    DevBuf<uint32_t> d_kp((size_t)kp_off[K], ps);
-    DevBuf<double> d_out_own;
-    if (graph) graph->begin(n_docs, cols, s);
-    else if (!own_rows_dev) d_out_own = DevBuf<double>((size_t)n_docs * cols, s);
-    double *const d_out = own_rows_dev ? own_rows_dev : d_out_own.p;
-    EAST_CUDA(cudaMemcpyAsync(d_kp.p, kp, sizeof(uint32_t) * (size_t)kp_off[K], cudaMemcpyHostToDevice, ps));
-    TableRun run;
-    run.kp_own = kp_begin(device, d_kp.p, kp, kp_off, K, !get_option("score_no_dedup", 0), false, ps, likely_code_table());
-    run.kp_host = kp; run.d_kp = d_kp.p; run.kp_off = kp_off; run.K = K; run.normalized = normalized;
-    if (group_off) { run.group_off = group_off; run.G = G; run.d_groups = upload_groups(group_off, G, s); }
-    run.d_out = d_out; run.host_out = out_DxK; run.graph = graph;
-    run.peer_rows = peer_rows; run.n_peers = n_peers;
+// Every build-and-score entry: checks, builds the index of `src` with `q` scored into `out` on the way, and re-scores the
+// index when the rows scored during the build do not stand.
+static void run_table(Source src, Query q, Output out, east_index **out_idx) {
+    validate(out, &src, q);
+    use_device(src.device);
+    cudaStream_t s = src.stream;
+    TableRun run(q, out, src.device);
     RunHook hook;
     hook.begin = table_run_begin; hook.fn = table_run_done; hook.ctx = &run; hook.building = &run.building;
-    build_host_impl(text, width, doc_off, doc_m, n_docs, device, &built, &hook);
+    DevBuf<uint32_t> d_kp;   // the host code points, uploaded
+    PackedTexts pt;          // raw texts: the packed text, owned here until the index takes it over
+    east_index *built = nullptr;
+    if (src.kind == Source::HOST) {
+        // the keyphrases go first, on a side stream: hashing, ordering and de-duplication of their suffixes (kp_prep.cu)
+        // run there while the text is on its way
+        cudaStream_t ps = prep_stream(src.device);
+        d_kp = q.upload(ps);
+        out.begin(src.n_docs, q.cols(), s);
+        run.kp_own = kp_begin(src.device, q.kp_dev, q.kp_host, q.kp_off, q.K, run.dedup, false, ps, likely_code_table());
+        q.upload_groups(s);
+        run.host_out = out.rows_host;
+        build_host_impl(src.text, src.width, src.doc_off, src.doc_m, src.n_docs, src.device, &built, &hook);
+    } else {
+        if (src.kind == Source::TEXTS) {
+            texts_to_packed(static_cast<const uint8_t *>(src.text), src.doc_off, src.n_docs, s, pt);
+            if (src.doc_off_out) std::copy(pt.doc_off.begin(), pt.doc_off.end(), src.doc_off_out);
+            if (src.doc_m_out) std::copy(pt.doc_m.begin(), pt.doc_m.end(), src.doc_m_out);
+            d_kp = q.upload(s);
+            src.text = pt.text; src.doc_off = pt.doc_off.data(); src.doc_m = pt.doc_m.data();
+        }
+        out.begin(src.n_docs, q.cols(), s);
+        q.upload_groups(s);
+        // keyphrase preparation on a side stream, queued from the build once its alphabet scan is on its way
+        run.kp_stream = prep_stream(src.device); run.caller_stream = s;
+        hook.scan_queued = table_kp_begin;
+        if (get_option("kp_upfront", 0)) table_kp_begin(&run);   // A/B: queue the preparation before the build starts
+        const bool owns_text = src.kind == Source::TEXTS;
+        pt.text = nullptr;   // build_common's index owns it from its first statement on
+        build_common(static_cast<const uint32_t *>(src.text), owns_text, src.doc_off, src.doc_m, src.n_docs, src.device, s,
+                     &built, nullptr, &hook);
+    }
     std::unique_ptr<east_index, void (*)(east_index *)> guard(built, free_index);
     // Rows scored on the way stand if the pass that produced them is the one the index came from: the speculative
-    // pipelined pass (pipelined = 1: the build ended on a host sync after both streams, the rows are in out_DxK)
-    // or the ordinary per-document pass (its copy is still in flight on stream s).
+    // pipelined pass of a host build (pipelined = 1: the build ended on a host sync after both streams, the rows are in
+    // place) or the ordinary per-document pass (its copies are still in flight on stream s).
+    const int32_t n_docs = src.n_docs, cols = q.cols();
     const bool stands = !run.failed && run.docs_scored == n_docs &&
                         ((built->pipelined && !run.final_pass) || (built->doc_sorted && !built->pipelined && run.final_pass));
-    if (!stands) {
-        score_common(built, d_kp.p, kp_off, K, normalized, d_out, 0, n_docs, s, nullptr, nullptr, kp, group_off, G, graph);
-        if (!graph) EAST_CUDA(cudaMemcpyAsync(out_DxK, d_out, sizeof(double) * (size_t)n_docs * cols, cudaMemcpyDeviceToHost, s));
+    if (!stands) score_common(built, q, out.rows, out.is_graph ? &out.graph : nullptr, 0, n_docs, s);
+    if (out.to_host && !(stands && run.host_out))   // the rows did not go to the host run by run
+        EAST_CUDA(cudaMemcpyAsync(out.rows_host, out.rows, sizeof(double) * (size_t)n_docs * cols, cudaMemcpyDeviceToHost, s));
+    if (out.n_peers > 0 && !(stands && run.docs_sent == n_docs))   // rows (also) produced by the batched scorer: plain peer copies
+        for (int32_t pi = 0; pi < out.n_peers; ++pi)
+            EAST_CUDA(cudaMemcpyAsync(out.peer_rows[pi], out.rows, sizeof(double) * (size_t)n_docs * cols, cudaMemcpyDefault, s));
+    if (out.is_graph) {
+        out.graph.finish(cols, s);
+        if (out.counts_host)
+            EAST_CUDA(cudaMemcpyAsync(out.counts_host, out.graph.C, sizeof(int32_t) * (size_t)cols * cols, cudaMemcpyDeviceToHost, s));
     }
-    if (n_peers > 0 && !(stands && run.docs_sent == n_docs))   // rows (also) produced by the batched scorer: plain peer copies
-        for (int32_t pi = 0; pi < n_peers; ++pi)
-            EAST_CUDA(cudaMemcpyAsync(peer_rows[pi], d_out, sizeof(double) * (size_t)n_docs * cols, cudaMemcpyDefault, s));
-    if (graph) graph->finish(cols, s);
     EAST_CUDA(cudaStreamSynchronize(s));
     if (out_idx) *out_idx = guard.release();
 }
@@ -1570,7 +1737,8 @@ int east_table_host(const uint32_t *text, const int64_t *doc_off, const int32_t 
                     const uint32_t *kp, const int64_t *kp_off, int32_t K, int normalized, double *out_DxK,
                     east_index **out_idx) {
     EAST_API_BEGIN
-    table_host_impl(text, 4, doc_off, doc_m, n_docs, device, kp, kp_off, K, normalized, out_DxK, out_idx);
+    run_table({Source::HOST, text, 4, doc_off, doc_m, n_docs, device},
+              Query(kp, true, nullptr, kp_off, K, normalized), Output::table_host(out_DxK), out_idx);
     EAST_API_END
 }
 
@@ -1578,63 +1746,18 @@ int east_table_host_u8(const uint8_t *text8, const int64_t *doc_off, const int32
                        const uint32_t *kp, const int64_t *kp_off, int32_t K, int normalized, double *out_DxK,
                        east_index **out_idx) {
     EAST_API_BEGIN
-    table_host_impl(text8, 1, doc_off, doc_m, n_docs, device, kp, kp_off, K, normalized, out_DxK, out_idx);
+    run_table({Source::HOST, text8, 1, doc_off, doc_m, n_docs, device},
+              Query(kp, true, nullptr, kp_off, K, normalized), Output::table_host(out_DxK), out_idx);
     EAST_API_END
-}
-
-static void table_dev_impl(const uint32_t *text_dev, const int64_t *doc_off, const int32_t *doc_m, int32_t n_docs, int device,
-                           const uint32_t *kp_dev, const uint32_t *kp_host, const int64_t *kp_off, int32_t K, int normalized,
-                           double *out_DxK_dev, double *const *peer_rows, int32_t n_peers, void *stream, east_index **out_idx,
-                           bool owns_text = false /* the index takes the text over (also when the call fails) */,
-                           const int64_t *group_off = nullptr /* synonym-expanded table: G + 1 offsets of the variant groups */,
-                           int32_t G = 0, GraphOut *graph = nullptr /* keyphrase graph: counts into graph->C, no table */) {
-    struct TextGuard {   // an owned text that never reached an index
-        const uint32_t *p; bool armed;
-        ~TextGuard() { if (armed && p) dev_free(const_cast<uint32_t *>(p), 0); }
-    } text_guard{text_dev, owns_text};
-    if (!kp_dev || !kp_off || (!out_DxK_dev && !graph) || K <= 0) throw Error(EAST_ERR_INVALID, "bad argument");
-    if (n_peers < 0 || n_peers > DocScore::MAX_PEERS || (n_peers > 0 && !peer_rows) || (n_peers > 0 && graph))
-        throw Error(EAST_ERR_INVALID, "bad peer list");
-    east_index *built = nullptr;
-    check_build_args(text_dev, doc_off, doc_m, n_docs, &built);
-    check_keyphrases(kp_off, K);
-    use_device(device);
-    cudaStream_t s = (cudaStream_t)stream;
-    if (graph) graph->begin(n_docs, group_off ? G : K, s);
-    TableRun run;
-    // keyphrase preparation on a side stream, queued from the build once its alphabet scan is on its way
-    run.device = device; run.dedup = !get_option("score_no_dedup", 0); run.kp_stream = prep_stream(device); run.caller_stream = s;
-    run.kp_host = kp_host; run.d_kp = kp_dev; run.kp_off = kp_off; run.K = K; run.normalized = normalized;
-    if (group_off) { run.group_off = group_off; run.G = G; run.d_groups = upload_groups(group_off, G, s); }
-    run.d_out = out_DxK_dev; run.host_out = nullptr; run.graph = graph;
-    run.peer_rows = peer_rows; run.n_peers = n_peers;
-    RunHook hook;
-    hook.begin = table_run_begin; hook.fn = table_run_done; hook.ctx = &run; hook.building = &run.building;
-    hook.scan_queued = table_kp_begin;
-    if (get_option("kp_upfront", 0)) table_kp_begin(&run);   // A/B: queue the preparation before the build starts
-    text_guard.armed = false;   // build_common's index owns it from its first statement on
-    build_common(text_dev, owns_text, doc_off, doc_m, n_docs, device, s, &built, nullptr, &hook);
-    std::unique_ptr<east_index, void (*)(east_index *)> guard(built, free_index);
-    const bool stands = !run.failed && run.docs_scored == n_docs && built->doc_sorted && run.final_pass;
-    if (!stands)
-        score_common(built, kp_dev, kp_off, K, normalized, out_DxK_dev, 0, n_docs, s, nullptr, nullptr, kp_host, group_off, G, graph);
-    if (n_peers > 0 && !(stands && run.docs_sent == n_docs)) {
-        // the rows were (also) produced by the batched scorer: plain peer copies of the slice
-        for (int32_t pi = 0; pi < n_peers; ++pi)
-            EAST_CUDA(cudaMemcpyAsync(peer_rows[pi], out_DxK_dev, sizeof(double) * (size_t)n_docs * run.cols(), cudaMemcpyDefault, s));
-    }
-    if (graph) graph->finish(run.cols(), s);
-    EAST_CUDA(cudaStreamSynchronize(s));
-    if (out_idx) *out_idx = guard.release();
 }
 
 int east_table_host_gather(const void *text, int32_t text_width, const int64_t *doc_off, const int32_t *doc_m, int32_t n_docs,
                            int device, const uint32_t *kp, const int64_t *kp_off, int32_t K, int normalized, double *out_DxK,
                            double *own_rows_dev, double *const *peer_rows, int32_t n_peers, east_index **out_idx) {
     EAST_API_BEGIN
-    if (text_width != 1 && text_width != 4) throw Error(EAST_ERR_INVALID, "text_width must be 1 or 4");
-    table_host_impl(text, text_width, doc_off, doc_m, n_docs, device, kp, kp_off, K, normalized, out_DxK, out_idx, own_rows_dev,
-                    peer_rows, n_peers);
+    run_table({Source::HOST, text, text_width, doc_off, doc_m, n_docs, device},
+              Query(kp, true, nullptr, kp_off, K, normalized),
+              Output::table_host(out_DxK, own_rows_dev, peer_rows, n_peers), out_idx);
     EAST_API_END
 }
 
@@ -1642,8 +1765,8 @@ int east_table_dev(const uint32_t *text_dev, const int64_t *doc_off, const int32
                    const uint32_t *kp_dev, const uint32_t *kp_host, const int64_t *kp_off, int32_t K, int normalized,
                    double *out_DxK_dev, void *stream, east_index **out_idx) {
     EAST_API_BEGIN
-    table_dev_impl(text_dev, doc_off, doc_m, n_docs, device, kp_dev, kp_host, kp_off, K, normalized, out_DxK_dev, nullptr, 0,
-                   stream, out_idx);
+    run_table({Source::DEVICE, text_dev, 4, doc_off, doc_m, n_docs, device, (cudaStream_t)stream},
+              Query(kp_dev, false, kp_host, kp_off, K, normalized), Output::table_dev(out_DxK_dev), out_idx);
     EAST_API_END
 }
 
@@ -1651,27 +1774,27 @@ int east_table_dev_gather(const uint32_t *text_dev, const int64_t *doc_off, cons
                           const uint32_t *kp_dev, const uint32_t *kp_host, const int64_t *kp_off, int32_t K, int normalized,
                           double *out_DxK_dev, double *const *peer_rows, int32_t n_peers, void *stream, east_index **out_idx) {
     EAST_API_BEGIN
-    table_dev_impl(text_dev, doc_off, doc_m, n_docs, device, kp_dev, kp_host, kp_off, K, normalized, out_DxK_dev, peer_rows,
-                   n_peers, stream, out_idx);
+    run_table({Source::DEVICE, text_dev, 4, doc_off, doc_m, n_docs, device, (cudaStream_t)stream},
+              Query(kp_dev, false, kp_host, kp_off, K, normalized), Output::table_dev(out_DxK_dev, peer_rows, n_peers), out_idx);
+    EAST_API_END
+}
+
+int east_table_texts_host(const uint8_t *utf8, const int64_t *text_off, int32_t n_texts, int device, const uint32_t *kp,
+                          const int64_t *kp_off, int32_t K, int normalized, double *out_DxK, int64_t *doc_off_out,
+                          int32_t *doc_m_out, east_index **out_idx) {
+    EAST_API_BEGIN
+    run_table({Source::TEXTS, utf8, 1, text_off, nullptr, n_texts, device, 0, doc_off_out, doc_m_out},
+              Query(kp, true, nullptr, kp_off, K, normalized), Output::table_host(out_DxK), out_idx);
     EAST_API_END
 }
 
 // ---- synonym-expanded tables in one call: the per-document kernel keeps the best variant of every group ------------
-// (arguments are checked before anything is built)
-static void check_table_groups(const int64_t *kp_off, int32_t V, const int64_t *group_off, int32_t G) {
-    if (!kp_off || V <= 0) throw Error(EAST_ERR_INVALID, "bad argument");
-    check_groups(group_off, G, V);
-    check_keyphrases(kp_off, V);
-}
-
 int east_table_groups_host(const void *text, int32_t text_width, const int64_t *doc_off, const int32_t *doc_m, int32_t n_docs,
                            int device, const uint32_t *kp, const int64_t *kp_off, int32_t V, const int64_t *group_off, int32_t G,
                            double *out_DxG, east_index **out_idx) {
     EAST_API_BEGIN
-    if (text_width != 1 && text_width != 4) throw Error(EAST_ERR_INVALID, "text_width must be 1 or 4");
-    check_table_groups(kp_off, V, group_off, G);
-    table_host_impl(text, text_width, doc_off, doc_m, n_docs, device, kp, kp_off, V, 1, out_DxG, out_idx, nullptr, nullptr, 0,
-                    group_off, G);
+    run_table({Source::HOST, text, text_width, doc_off, doc_m, n_docs, device},
+              Query(kp, true, nullptr, kp_off, V, 1, true, group_off, G), Output::table_host(out_DxG), out_idx);
     EAST_API_END
 }
 
@@ -1680,26 +1803,50 @@ int east_table_groups_dev(const uint32_t *text_dev, const int64_t *doc_off, cons
                           const int64_t *group_off, int32_t G, double *out_DxG_dev, double *const *peer_rows, int32_t n_peers,
                           void *stream, east_index **out_idx) {
     EAST_API_BEGIN
-    check_table_groups(kp_off, V, group_off, G);
-    table_dev_impl(text_dev, doc_off, doc_m, n_docs, device, kp_dev, kp_host, kp_off, V, 1, out_DxG_dev, peer_rows, n_peers,
-                   stream, out_idx, false, group_off, G);
+    run_table({Source::DEVICE, text_dev, 4, doc_off, doc_m, n_docs, device, (cudaStream_t)stream},
+              Query(kp_dev, false, kp_host, kp_off, V, 1, true, group_off, G),
+              Output::table_dev(out_DxG_dev, peer_rows, n_peers), out_idx);
     EAST_API_END
 }
 
-int east_score_one(const east_index *idx, int32_t doc, const uint32_t *q, int32_t len, int normalized,
-                   double *score, double *suffix_scores) {
+int east_table_texts_groups_host(const uint8_t *utf8, const int64_t *text_off, int32_t n_texts, int device, const uint32_t *kp,
+                                 const int64_t *kp_off, int32_t V, const int64_t *group_off, int32_t G, double *out_DxG,
+                                 int64_t *doc_off_out, int32_t *doc_m_out, east_index **out_idx) {
     EAST_API_BEGIN
-    if (!idx || !score || doc < 0 || doc >= idx->n_docs) throw Error(EAST_ERR_INVALID, "bad argument");
-    if (len <= 0 || !q) throw Error(EAST_ERR_ZERODIV, "empty query: float division by zero");
-    EAST_CUDA(cudaSetDevice(idx->device));
-    cudaStream_t s = 0;
-    int64_t off[2] = {0, len};
-    DevBuf<uint32_t> d_q(len, s);
-    DevBuf<double> d_out(1, s), d_suf(len, s);
-    EAST_CUDA(cudaMemcpyAsync(d_q.p, q, sizeof(uint32_t) * len, cudaMemcpyHostToDevice, s));
-    score_common(idx, d_q.p, off, 1, normalized, d_out.p, doc, 1, s, d_suf.p, nullptr, q);
-    EAST_CUDA(cudaMemcpy(score, d_out.p, sizeof(double), cudaMemcpyDeviceToHost));
-    if (suffix_scores) EAST_CUDA(cudaMemcpy(suffix_scores, d_suf.p, sizeof(double) * len, cudaMemcpyDeviceToHost));
+    run_table({Source::TEXTS, utf8, 1, text_off, nullptr, n_texts, device, 0, doc_off_out, doc_m_out},
+              Query(kp, true, nullptr, kp_off, V, 1, true, group_off, G), Output::table_host(out_DxG), out_idx);
+    EAST_API_END
+}
+
+// ---- keyphrase graphs in one call: build, score and count co-occurrences, no score table ------------------------------
+// (group_off NULL: plain keyphrases)
+int east_graph_host(const void *text, int32_t text_width, const int64_t *doc_off, const int32_t *doc_m, int32_t n_docs,
+                    int device, const uint32_t *kp, const int64_t *kp_off, int32_t V, const int64_t *group_off, int32_t G,
+                    int normalized, double threshold, int32_t *C_host, east_index **out_idx) {
+    EAST_API_BEGIN
+    run_table({Source::HOST, text, text_width, doc_off, doc_m, n_docs, device},
+              Query(kp, true, nullptr, kp_off, V, normalized, group_off != nullptr, group_off, G),
+              Output::counts(threshold, nullptr, C_host), out_idx);
+    EAST_API_END
+}
+
+int east_graph_dev(const uint32_t *text_dev, const int64_t *doc_off, const int32_t *doc_m, int32_t n_docs, int device,
+                   const uint32_t *kp_dev, const uint32_t *kp_host, const int64_t *kp_off, int32_t V, const int64_t *group_off,
+                   int32_t G, int normalized, double threshold, int32_t *C_dev, void *stream, east_index **out_idx) {
+    EAST_API_BEGIN
+    run_table({Source::DEVICE, text_dev, 4, doc_off, doc_m, n_docs, device, (cudaStream_t)stream},
+              Query(kp_dev, false, kp_host, kp_off, V, normalized, group_off != nullptr, group_off, G),
+              Output::counts(threshold, C_dev, nullptr), out_idx);
+    EAST_API_END
+}
+
+int east_graph_texts_host(const uint8_t *utf8, const int64_t *text_off, int32_t n_texts, int device, const uint32_t *kp,
+                          const int64_t *kp_off, int32_t V, const int64_t *group_off, int32_t G, int normalized, double threshold,
+                          int32_t *C_host, int64_t *doc_off_out, int32_t *doc_m_out, east_index **out_idx) {
+    EAST_API_BEGIN
+    run_table({Source::TEXTS, utf8, 1, text_off, nullptr, n_texts, device, 0, doc_off_out, doc_m_out},
+              Query(kp, true, nullptr, kp_off, V, normalized, group_off != nullptr, group_off, G),
+              Output::counts(threshold, nullptr, C_host), out_idx);
     EAST_API_END
 }
 
@@ -1731,167 +1878,6 @@ int east_cooc_host(const double *S_DxK, int64_t D, int32_t K, double threshold, 
     if (get_option("cooc_variant", 0) == 1) cooc_counts(d_S.p, D, K, threshold, d_C.p, s);
     else cooc_counts_tc(d_S.p, D, K, threshold, d_C.p, s, cooc_tc_kernel());
     EAST_CUDA(cudaMemcpy(C_KxK, d_C.p, sizeof(int32_t) * (size_t)K * K, cudaMemcpyDeviceToHost));
-    EAST_API_END
-}
-
-// ---- device preprocessing (tokenize.cu) -----------------------------------------------------
-namespace {
-struct PackedTexts {
-    uint32_t *text = nullptr;          // device, owned until released
-    std::vector<int64_t> doc_off;
-    std::vector<int32_t> doc_m;
-    ~PackedTexts() { if (text) dev_free(text, 0); }
-};
-
-// raw UTF-8 texts (host) -> packed documents on the device; throws EAST_ERR_UNSUPPORTED when a text needs the host path
-void texts_to_packed(const uint8_t *utf8, const int64_t *text_off, int32_t n_texts, cudaStream_t s, PackedTexts &out) {
-    if (!utf8 || !text_off || n_texts <= 0) throw Error(EAST_ERR_INVALID, "bad argument");
-    if (text_off[0] != 0) throw Error(EAST_ERR_INVALID, "text_off[0] must be 0");
-    for (int32_t i = 0; i < n_texts; ++i)
-        if (text_off[i + 1] < text_off[i]) throw Error(EAST_ERR_INVALID, "text offsets must not decrease");
-    const int64_t bytes = text_off[n_texts];
-    if (bytes >= (1ll << 31)) throw Error(EAST_ERR_RANGE, "more than 2^31 bytes of text in one call; split the collection");
-    DevBuf<uint8_t> d_raw((size_t)bytes + 16, s);
-    DevBuf<int64_t> d_off((size_t)n_texts + 1, s), d_doc_off((size_t)n_texts + 1, s);
-    DevBuf<int32_t> d_sizes(3 * (size_t)n_texts, s);
-    if (bytes) EAST_CUDA(cudaMemcpyAsync(d_raw.p, utf8, (size_t)bytes, cudaMemcpyHostToDevice, s));
-    EAST_CUDA(cudaMemcpyAsync(d_off.p, text_off, sizeof(int64_t) * ((size_t)n_texts + 1), cudaMemcpyHostToDevice, s));
-    tokenize_texts(d_raw.p, d_off.p, n_texts, d_sizes.p, s);
-    std::vector<int32_t> sizes(3 * (size_t)n_texts);
-    EAST_CUDA(cudaMemcpyAsync(sizes.data(), d_sizes.p, sizeof(int32_t) * sizes.size(), cudaMemcpyDeviceToHost, s));
-    EAST_CUDA(cudaStreamSynchronize(s));
-    out.doc_off.assign((size_t)n_texts + 1, 0);
-    out.doc_m.resize((size_t)n_texts);
-    for (int32_t i = 0; i < n_texts; ++i) {
-        if (sizes[3 * (size_t)i + 2])
-            throw Error(EAST_ERR_UNSUPPORTED, "text " + std::to_string(i) + " has characters outside ASCII / U+0400-045F (or invalid UTF-8): "
-                                              "use the host preprocessing");
-        out.doc_off[(size_t)i + 1] = out.doc_off[(size_t)i] + sizes[3 * (size_t)i];
-        out.doc_m[(size_t)i] = sizes[3 * (size_t)i + 1];
-    }
-    if (out.doc_off.back() >= (1ll << 30)) throw Error(EAST_ERR_RANGE, "more than 2^30 code points in one index; split the batch");
-    EAST_CUDA(cudaMemcpyAsync(d_doc_off.p, out.doc_off.data(), sizeof(int64_t) * out.doc_off.size(), cudaMemcpyHostToDevice, s));
-    out.text = (uint32_t *)dev_alloc(sizeof(uint32_t) * (size_t)out.doc_off.back(), s, true);
-    tokenize_emit(d_raw.p, d_off.p, n_texts, d_doc_off.p, out.text, s);
-    EAST_CUDA(cudaStreamSynchronize(s));   // the staging buffers (and the pageable doc_off upload) end here
-}
-}  // namespace
-
-int east_texts_to_packed_host(const uint8_t *utf8, const int64_t *text_off, int32_t n_texts, int device, uint32_t *packed_out,
-                              int64_t packed_cap, int64_t *doc_off_out, int32_t *doc_m_out) {
-    EAST_API_BEGIN
-    if (!doc_off_out || !doc_m_out) throw Error(EAST_ERR_INVALID, "NULL argument");
-    use_device(device);
-    PackedTexts pt;
-    texts_to_packed(utf8, text_off, n_texts, 0, pt);
-    std::copy(pt.doc_off.begin(), pt.doc_off.end(), doc_off_out);
-    std::copy(pt.doc_m.begin(), pt.doc_m.end(), doc_m_out);
-    if (pt.doc_off.back() > packed_cap || !packed_out) throw Error(EAST_ERR_RANGE, "packed_out is too small (doc_off_out holds the sizes)");
-    EAST_CUDA(cudaMemcpy(packed_out, pt.text, sizeof(uint32_t) * (size_t)pt.doc_off.back(), cudaMemcpyDeviceToHost));
-    EAST_API_END
-}
-
-static void table_texts_impl(const uint8_t *utf8, const int64_t *text_off, int32_t n_texts, int device, const uint32_t *kp,
-                             const int64_t *kp_off, int32_t K, int normalized, double *out_DxK, int64_t *doc_off_out,
-                             int32_t *doc_m_out, east_index **out_idx, const int64_t *group_off = nullptr, int32_t G = 0,
-                             GraphOut *graph = nullptr) {
-    if (!kp || !kp_off || (!out_DxK && !graph) || K <= 0) throw Error(EAST_ERR_INVALID, "bad argument");
-    check_keyphrases(kp_off, K);
-    const int32_t cols = group_off ? G : K;
-    use_device(device);
-    cudaStream_t s = 0;
-    PackedTexts pt;
-    texts_to_packed(utf8, text_off, n_texts, s, pt);
-    if (doc_off_out) std::copy(pt.doc_off.begin(), pt.doc_off.end(), doc_off_out);
-    if (doc_m_out) std::copy(pt.doc_m.begin(), pt.doc_m.end(), doc_m_out);
-    DevBuf<uint32_t> d_kp((size_t)kp_off[K], s);
-    DevBuf<double> d_out;
-    if (!graph) d_out = DevBuf<double>((size_t)n_texts * cols, s);
-    EAST_CUDA(cudaMemcpyAsync(d_kp.p, kp, sizeof(uint32_t) * (size_t)kp_off[K], cudaMemcpyHostToDevice, s));
-    const uint32_t *text = pt.text;
-    pt.text = nullptr;   // the index owns it from here on
-    table_dev_impl(text, pt.doc_off.data(), pt.doc_m.data(), n_texts, device, d_kp.p, kp, kp_off, K, normalized, d_out.p, nullptr, 0,
-                   (void *)s, out_idx, true, group_off, G, graph);
-    if (!graph) EAST_CUDA(cudaMemcpy(out_DxK, d_out.p, sizeof(double) * (size_t)n_texts * cols, cudaMemcpyDeviceToHost));
-}
-
-int east_table_texts_host(const uint8_t *utf8, const int64_t *text_off, int32_t n_texts, int device, const uint32_t *kp,
-                          const int64_t *kp_off, int32_t K, int normalized, double *out_DxK, int64_t *doc_off_out,
-                          int32_t *doc_m_out, east_index **out_idx) {
-    EAST_API_BEGIN
-    table_texts_impl(utf8, text_off, n_texts, device, kp, kp_off, K, normalized, out_DxK, doc_off_out, doc_m_out, out_idx);
-    EAST_API_END
-}
-
-int east_table_texts_groups_host(const uint8_t *utf8, const int64_t *text_off, int32_t n_texts, int device, const uint32_t *kp,
-                                 const int64_t *kp_off, int32_t V, const int64_t *group_off, int32_t G, double *out_DxG,
-                                 int64_t *doc_off_out, int32_t *doc_m_out, east_index **out_idx) {
-    EAST_API_BEGIN
-    check_table_groups(kp_off, V, group_off, G);
-    table_texts_impl(utf8, text_off, n_texts, device, kp, kp_off, V, 1, out_DxG, doc_off_out, doc_m_out, out_idx, group_off, G);
-    EAST_API_END
-}
-
-// ---- keyphrase graphs in one call: build, score and count co-occurrences, no score table ------------------------------
-// (arguments are checked before anything is built; groups are always normalized, as in the table entries)
-static void check_graph_args(const int64_t *kp_off, int32_t V, const int64_t *group_off, int32_t G, const void *C) {
-    if (!kp_off || V <= 0 || !C) throw Error(EAST_ERR_INVALID, "bad argument");
-    if (group_off) check_groups(group_off, G, V);
-    check_keyphrases(kp_off, V);
-}
-
-// the cols x cols counts of a host entry: C on the device, copied out once the call's stream is done
-struct HostCounts {
-    DevBuf<int32_t> d;
-    int32_t cols;
-    HostCounts(int32_t V, const int64_t *group_off, int32_t G) : d((size_t)(group_off ? G : V) * (group_off ? G : V), 0),
-                                                                  cols(group_off ? G : V) {}
-    void copy_out(int32_t *C_host) {
-        EAST_CUDA(cudaMemcpyAsync(C_host, d.p, sizeof(int32_t) * (size_t)cols * cols, cudaMemcpyDeviceToHost, 0));
-        EAST_CUDA(cudaStreamSynchronize(0));
-    }
-};
-
-int east_graph_host(const void *text, int32_t text_width, const int64_t *doc_off, const int32_t *doc_m, int32_t n_docs,
-                    int device, const uint32_t *kp, const int64_t *kp_off, int32_t V, const int64_t *group_off, int32_t G,
-                    int normalized, double threshold, int32_t *C_host, east_index **out_idx) {
-    EAST_API_BEGIN
-    if (text_width != 1 && text_width != 4) throw Error(EAST_ERR_INVALID, "text_width must be 1 or 4");
-    check_graph_args(kp_off, V, group_off, G, C_host);
-    use_device(device);
-    HostCounts counts(V, group_off, G);
-    GraphOut graph;
-    graph.threshold = threshold; graph.C = counts.d.p;
-    table_host_impl(text, text_width, doc_off, doc_m, n_docs, device, kp, kp_off, V, group_off ? 1 : normalized, nullptr, out_idx,
-                    nullptr, nullptr, 0, group_off, G, &graph);
-    counts.copy_out(C_host);
-    EAST_API_END
-}
-
-int east_graph_dev(const uint32_t *text_dev, const int64_t *doc_off, const int32_t *doc_m, int32_t n_docs, int device,
-                   const uint32_t *kp_dev, const uint32_t *kp_host, const int64_t *kp_off, int32_t V, const int64_t *group_off,
-                   int32_t G, int normalized, double threshold, int32_t *C_dev, void *stream, east_index **out_idx) {
-    EAST_API_BEGIN
-    check_graph_args(kp_off, V, group_off, G, C_dev);
-    GraphOut graph;
-    graph.threshold = threshold; graph.C = C_dev;
-    table_dev_impl(text_dev, doc_off, doc_m, n_docs, device, kp_dev, kp_host, kp_off, V, group_off ? 1 : normalized, nullptr, nullptr, 0,
-                   stream, out_idx, false, group_off, G, &graph);
-    EAST_API_END
-}
-
-int east_graph_texts_host(const uint8_t *utf8, const int64_t *text_off, int32_t n_texts, int device, const uint32_t *kp,
-                          const int64_t *kp_off, int32_t V, const int64_t *group_off, int32_t G, int normalized, double threshold,
-                          int32_t *C_host, int64_t *doc_off_out, int32_t *doc_m_out, east_index **out_idx) {
-    EAST_API_BEGIN
-    check_graph_args(kp_off, V, group_off, G, C_host);
-    use_device(device);
-    HostCounts counts(V, group_off, G);
-    GraphOut graph;
-    graph.threshold = threshold; graph.C = counts.d.p;
-    table_texts_impl(utf8, text_off, n_texts, device, kp, kp_off, V, group_off ? 1 : normalized, nullptr, doc_off_out, doc_m_out,
-                     out_idx, group_off, G, &graph);
-    counts.copy_out(C_host);
     EAST_API_END
 }
 

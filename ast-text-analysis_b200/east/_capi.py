@@ -216,6 +216,38 @@ def _columns(K, group_off):
     return K if group_off is None else len(group_off) - 1
 
 
+def _keyphrases_args(kp_codes, kp_off):
+    """(uint32 code points, int64 offsets, K) of packed keyphrases or variants; kp_codes may be None (the optional host
+    copy of device-resident code points)"""
+    kp_off = np.ascontiguousarray(kp_off, dtype=np.int64)
+    codes = None if kp_codes is None else np.ascontiguousarray(kp_codes, dtype=np.uint32)
+    return codes, kp_off, len(kp_off) - 1
+
+
+def _kp_host_arg(kp_codes):
+    """pointer to the optional host copy of device-resident code points (None: no copy)"""
+    return None if kp_codes is None else _ptr(kp_codes, _u32p)
+
+
+def _documents_args(doc_off, doc_m):
+    """(int64 offsets [n + 1], int32 string counts [n]) of packed documents"""
+    return np.ascontiguousarray(doc_off, dtype=np.int64), np.ascontiguousarray(doc_m, dtype=np.int32)
+
+
+def _texts_args(texts):
+    """raw texts (list of str / UTF-8 bytes, or (uint8 buffer, int64 offsets) already laid out back to back, e.g. in
+    pinned memory) -> (buffer, offsets, n, doc_off and doc_m for the packed documents the call returns)"""
+    buf, off = texts if isinstance(texts, tuple) else concat_utf8(texts)
+    n = len(off) - 1
+    return buf, off, n, np.zeros(n + 1, dtype=np.int64), np.zeros(n, dtype=np.int32)
+
+
+def _peers_arg(peer_rows):
+    """(ctypes array of the peer row addresses, their number)"""
+    peer_rows = list(peer_rows or [])
+    return (_vp * max(len(peer_rows), 1))(*[int(a) for a in peer_rows]), len(peer_rows)
+
+
 def _groups_arg(group_off):
     """(int64 array or None, pointer or None, G) of optional group offsets"""
     if group_off is None:
@@ -302,6 +334,14 @@ class DeviceIndex(object):
         return cls.from_handle(h, doc_off, doc_m, int(device))
 
     @classmethod
+    def _adopt(cls, entry, doc_off, doc_m, device, *args):
+        """Call a build entry with its arguments and the out_idx pointer; the index it returns (doc_off / doc_m may be
+        filled by the call)."""
+        h = _vp()
+        _check(entry(*args, ctypes.byref(h)))
+        return cls.from_handle(h, doc_off, doc_m, int(device))
+
+    @classmethod
     def table_from_texts(cls, texts, kp_codes, kp_off, out, normalized=True, device=0, group_off=None):
         """Raw texts in, score table out, in ONE engine call (east_table_texts_host): the texts are upper-cased,
         tokenised, grouped and packed on the device (tokenize.cu), indexed and scored.  texts: list of str / UTF-8
@@ -309,87 +349,54 @@ class DeviceIndex(object):
         group_off (pack_variant_groups): the keyphrases are synonym variants in G groups and `out` has G columns, the
         best normalized variant of each group (east_table_texts_groups_host)."""
         L = load()
-        # texts may also be (uint8 buffer, int64 offsets): texts already laid out back to back (e.g. in pinned memory)
-        buf, off = texts if isinstance(texts, tuple) else concat_utf8(texts)
-        n = len(off) - 1
-        kp_codes = np.ascontiguousarray(kp_codes, dtype=np.uint32)
-        kp_off = np.ascontiguousarray(kp_off, dtype=np.int64)
-        K = len(kp_off) - 1
+        buf, off, n, doc_off, doc_m = _texts_args(texts)
+        kp_codes, kp_off, K = _keyphrases_args(kp_codes, kp_off)
+        group_off, gp, G = _groups_arg(group_off)
         assert out.dtype == np.float64 and out.flags["C_CONTIGUOUS"] and out.size == n * _columns(K, group_off)
-        doc_off = np.zeros(n + 1, dtype=np.int64)
-        doc_m = np.zeros(n, dtype=np.int32)
-        h = _vp()
+        texts_args = (_ptr(buf, _u8p), _ptr(off, _i64p), n, int(device), _ptr(kp_codes, _u32p), _ptr(kp_off, _i64p), K)
+        outs = (_ptr(out, _f64p), _ptr(doc_off, _i64p), _ptr(doc_m, _i32p))
         if group_off is not None:
-            group_off = np.ascontiguousarray(group_off, dtype=np.int64)
-            _check(L.east_table_texts_groups_host(_ptr(buf, _u8p), _ptr(off, _i64p), n, int(device), _ptr(kp_codes, _u32p),
-                                                  _ptr(kp_off, _i64p), K, _ptr(group_off, _i64p), len(group_off) - 1,
-                                                  _ptr(out, _f64p), _ptr(doc_off, _i64p), _ptr(doc_m, _i32p), ctypes.byref(h)))
-            return cls.from_handle(h, doc_off, doc_m, int(device))
-        _check(L.east_table_texts_host(_ptr(buf, _u8p), _ptr(off, _i64p), n, int(device), _ptr(kp_codes, _u32p),
-                                       _ptr(kp_off, _i64p), K, 1 if normalized else 0, _ptr(out, _f64p),
-                                       _ptr(doc_off, _i64p), _ptr(doc_m, _i32p), ctypes.byref(h)))
-        return cls.from_handle(h, doc_off, doc_m, int(device))
+            return cls._adopt(L.east_table_texts_groups_host, doc_off, doc_m, device, *texts_args, gp, G, *outs)
+        return cls._adopt(L.east_table_texts_host, doc_off, doc_m, device, *texts_args, 1 if normalized else 0, *outs)
 
     @classmethod
     def graph_from_texts(cls, texts, kp_codes, kp_off, threshold, C=None, normalized=True, device=0, group_off=None):
         """table_from_texts() for a keyphrase graph (east_graph_texts_host): raw texts in, the int32 co-occurrence counts
         C[i][j] = number of texts in which columns i and j both score >= threshold out, without a score table.
         Returns (C, index); C: [cols, cols], cols = K, or G with group_off (always normalized)."""
-        L = load()
-        buf, off = texts if isinstance(texts, tuple) else concat_utf8(texts)
-        n = len(off) - 1
-        kp_codes = np.ascontiguousarray(kp_codes, dtype=np.uint32)
-        kp_off = np.ascontiguousarray(kp_off, dtype=np.int64)
-        K = len(kp_off) - 1
+        buf, off, n, doc_off, doc_m = _texts_args(texts)
+        kp_codes, kp_off, K = _keyphrases_args(kp_codes, kp_off)
         group_off, gp, G = _groups_arg(group_off)
         C = _counts_out(C, K, group_off)
-        doc_off = np.zeros(n + 1, dtype=np.int64)
-        doc_m = np.zeros(n, dtype=np.int32)
-        h = _vp()
-        _check(L.east_graph_texts_host(_ptr(buf, _u8p), _ptr(off, _i64p), n, int(device), _ptr(kp_codes, _u32p), _ptr(kp_off, _i64p),
-                                       K, gp, G, 1 if normalized else 0, float(threshold), _ptr(C, _i32p), _ptr(doc_off, _i64p),
-                                       _ptr(doc_m, _i32p), ctypes.byref(h)))
-        return C, cls.from_handle(h, doc_off, doc_m, int(device))
+        return C, cls._adopt(load().east_graph_texts_host, doc_off, doc_m, device, _ptr(buf, _u8p), _ptr(off, _i64p), n,
+                             int(device), _ptr(kp_codes, _u32p), _ptr(kp_off, _i64p), K, gp, G, 1 if normalized else 0,
+                             float(threshold), _ptr(C, _i32p), _ptr(doc_off, _i64p), _ptr(doc_m, _i32p))
 
     @classmethod
     def build_host_and_graph(cls, text, doc_off, doc_m, kp_codes, kp_off, threshold, C=None, normalized=True, device=0,
                              group_off=None):
         """build_host_and_score() for a keyphrase graph (east_graph_host): text uint32 code points or one byte per code
         point (pack_strings_collection_u8).  Returns (int32 counts [cols, cols], index); no score table is formed."""
-        L = load()
-        doc_off = np.ascontiguousarray(doc_off, dtype=np.int64)
-        doc_m = np.ascontiguousarray(doc_m, dtype=np.int32)
-        kp_codes = np.ascontiguousarray(kp_codes, dtype=np.uint32)
-        kp_off = np.ascontiguousarray(kp_off, dtype=np.int64)
-        K = len(kp_off) - 1
+        doc_off, doc_m = _documents_args(doc_off, doc_m)
+        kp_codes, kp_off, K = _keyphrases_args(kp_codes, kp_off)
         assert text.dtype in (np.uint32, np.uint8) and text.flags["C_CONTIGUOUS"]
         group_off, gp, G = _groups_arg(group_off)
         C = _counts_out(C, K, group_off)
-        h = _vp()
-        _check(L.east_graph_host(_vp(text.ctypes.data), int(text.itemsize), _ptr(doc_off, _i64p), _ptr(doc_m, _i32p), len(doc_m),
-                                 int(device), _ptr(kp_codes, _u32p), _ptr(kp_off, _i64p), K, gp, G, 1 if normalized else 0,
-                                 float(threshold), _ptr(C, _i32p), ctypes.byref(h)))
-        return C, cls.from_handle(h, doc_off, doc_m, int(device))
+        return C, cls._adopt(load().east_graph_host, doc_off, doc_m, device, _vp(text.ctypes.data), int(text.itemsize),
+                             _ptr(doc_off, _i64p), _ptr(doc_m, _i32p), len(doc_m), int(device), _ptr(kp_codes, _u32p),
+                             _ptr(kp_off, _i64p), K, gp, G, 1 if normalized else 0, float(threshold), _ptr(C, _i32p))
 
     @classmethod
     def build_dev_and_graph(cls, text_devptr, doc_off, doc_m, kp_devptr, kp_codes, kp_off, threshold, C_devptr, normalized=True,
                             device=0, stream=0, group_off=None):
         """build_dev_and_score() for a keyphrase graph (east_graph_dev): the int32 [cols, cols] counts go to C_devptr.
         Returns the index."""
-        L = load()
-        doc_off = np.ascontiguousarray(doc_off, dtype=np.int64)
-        doc_m = np.ascontiguousarray(doc_m, dtype=np.int32)
-        kp_off = np.ascontiguousarray(kp_off, dtype=np.int64)
-        kp_host = None
-        if kp_codes is not None:
-            kp_codes = np.ascontiguousarray(kp_codes, dtype=np.uint32)
-            kp_host = _ptr(kp_codes, _u32p)
+        doc_off, doc_m = _documents_args(doc_off, doc_m)
+        kp_codes, kp_off, K = _keyphrases_args(kp_codes, kp_off)
         group_off, gp, G = _groups_arg(group_off)
-        h = _vp()
-        _check(L.east_graph_dev(_vp(text_devptr), _ptr(doc_off, _i64p), _ptr(doc_m, _i32p), len(doc_m), int(device), _vp(kp_devptr),
-                                kp_host, _ptr(kp_off, _i64p), len(kp_off) - 1, gp, G, 1 if normalized else 0, float(threshold),
-                                _vp(C_devptr), _vp(stream), ctypes.byref(h)))
-        return cls.from_handle(h, doc_off, doc_m, int(device))
+        return cls._adopt(load().east_graph_dev, doc_off, doc_m, device, _vp(text_devptr), _ptr(doc_off, _i64p),
+                          _ptr(doc_m, _i32p), len(doc_m), int(device), _vp(kp_devptr), _kp_host_arg(kp_codes),
+                          _ptr(kp_off, _i64p), K, gp, G, 1 if normalized else 0, float(threshold), _vp(C_devptr), _vp(stream))
 
     @classmethod
     def build_host_u8(cls, text8, doc_off, doc_m, device=0):
@@ -413,39 +420,26 @@ class DeviceIndex(object):
         group_off (pack_variant_groups): the keyphrases are synonym variants in G groups and `out` ([n_docs, G]) holds
         the best normalized variant of each group (east_table_groups_host; not with own_rows / peer_rows)."""
         L = load()
-        doc_off = np.ascontiguousarray(doc_off, dtype=np.int64)
-        doc_m = np.ascontiguousarray(doc_m, dtype=np.int32)
-        kp_codes = np.ascontiguousarray(kp_codes, dtype=np.uint32)
-        kp_off = np.ascontiguousarray(kp_off, dtype=np.int64)
-        K = len(kp_off) - 1
+        doc_off, doc_m = _documents_args(doc_off, doc_m)
+        kp_codes, kp_off, K = _keyphrases_args(kp_codes, kp_off)
         assert text.dtype in (np.uint32, np.uint8) and text.flags["C_CONTIGUOUS"]
         assert out.dtype == np.float64 and out.flags["C_CONTIGUOUS"] and out.size == len(doc_m) * _columns(K, group_off)
-        h = _vp()
+        group_off, gp, G = _groups_arg(group_off)
+        norm = 1 if normalized else 0
+        docs = (_ptr(doc_off, _i64p), _ptr(doc_m, _i32p), len(doc_m), int(device))
+        kps = (_ptr(kp_codes, _u32p), _ptr(kp_off, _i64p), K)
         if group_off is not None:
             if own_rows or peer_rows:
                 raise ValueError("a sharded synonym table is built from device-resident text (build_dev_and_score)")
-            group_off = np.ascontiguousarray(group_off, dtype=np.int64)
-            _check(L.east_table_groups_host(_vp(text.ctypes.data), int(text.itemsize), _ptr(doc_off, _i64p), _ptr(doc_m, _i32p),
-                                            len(doc_m), int(device), _ptr(kp_codes, _u32p), _ptr(kp_off, _i64p), K,
-                                            _ptr(group_off, _i64p), len(group_off) - 1, _ptr(out, _f64p), ctypes.byref(h)))
-            return cls.from_handle(h, doc_off, doc_m, int(device))
+            return cls._adopt(L.east_table_groups_host, doc_off, doc_m, device, _vp(text.ctypes.data), int(text.itemsize),
+                              *docs, *kps, gp, G, _ptr(out, _f64p))
         if own_rows or peer_rows:   # sharded table: rows also to the gathered tables on the devices (east_table_host_gather)
-            peer_rows = list(peer_rows or [])
-            peers = (_vp * max(len(peer_rows), 1))(*[int(a) for a in peer_rows])
-            _check(L.east_table_host_gather(_vp(text.ctypes.data), int(text.itemsize), _ptr(doc_off, _i64p), _ptr(doc_m, _i32p),
-                                            len(doc_m), int(device), _ptr(kp_codes, _u32p), _ptr(kp_off, _i64p), K,
-                                            1 if normalized else 0, _ptr(out, _f64p), _vp(own_rows or 0), peers, len(peer_rows),
-                                            ctypes.byref(h)))
-            return cls.from_handle(h, doc_off, doc_m, int(device))
+            peers, n_peers = _peers_arg(peer_rows)
+            return cls._adopt(L.east_table_host_gather, doc_off, doc_m, device, _vp(text.ctypes.data), int(text.itemsize),
+                              *docs, *kps, norm, _ptr(out, _f64p), _vp(own_rows or 0), peers, n_peers)
         if text.dtype == np.uint8:   # one byte per code point, 0xFF ends a string (pack_strings_collection_u8)
-            _check(L.east_table_host_u8(_ptr(text, _u8p), _ptr(doc_off, _i64p), _ptr(doc_m, _i32p), len(doc_m), int(device),
-                                        _ptr(kp_codes, _u32p), _ptr(kp_off, _i64p), K, 1 if normalized else 0,
-                                        _ptr(out, _f64p), ctypes.byref(h)))
-            return cls.from_handle(h, doc_off, doc_m, int(device))
-        _check(L.east_table_host(_ptr(text, _u32p), _ptr(doc_off, _i64p), _ptr(doc_m, _i32p), len(doc_m), int(device),
-                                 _ptr(kp_codes, _u32p), _ptr(kp_off, _i64p), K, 1 if normalized else 0,
-                                 _ptr(out, _f64p), ctypes.byref(h)))
-        return cls.from_handle(h, doc_off, doc_m, int(device))
+            return cls._adopt(L.east_table_host_u8, doc_off, doc_m, device, _ptr(text, _u8p), *docs, *kps, norm, _ptr(out, _f64p))
+        return cls._adopt(L.east_table_host, doc_off, doc_m, device, _ptr(text, _u32p), *docs, *kps, norm, _ptr(out, _f64p))
 
     @classmethod
     def build_dev_and_score(cls, text_devptr, doc_off, doc_m, kp_devptr, kp_codes, kp_off, out_devptr, normalized=True,
@@ -457,34 +451,18 @@ class DeviceIndex(object):
         group_off (pack_variant_groups): the keyphrases are synonym variants in G groups and the table has G columns,
         the best normalized variant of each group (east_table_groups_dev, with or without peer_rows)."""
         L = load()
-        doc_off = np.ascontiguousarray(doc_off, dtype=np.int64)
-        doc_m = np.ascontiguousarray(doc_m, dtype=np.int32)
-        kp_off = np.ascontiguousarray(kp_off, dtype=np.int64)
-        kp_host = None
-        if kp_codes is not None:
-            kp_codes = np.ascontiguousarray(kp_codes, dtype=np.uint32)
-            kp_host = _ptr(kp_codes, _u32p)
-        h = _vp()
+        doc_off, doc_m = _documents_args(doc_off, doc_m)
+        kp_codes, kp_off, K = _keyphrases_args(kp_codes, kp_off)
+        group_off, gp, G = _groups_arg(group_off)
+        args = (_vp(text_devptr), _ptr(doc_off, _i64p), _ptr(doc_m, _i32p), len(doc_m), int(device), _vp(kp_devptr),
+                _kp_host_arg(kp_codes), _ptr(kp_off, _i64p), K)
         if group_off is not None:
-            group_off = np.ascontiguousarray(group_off, dtype=np.int64)
-            peer_rows = list(peer_rows or [])
-            peers = (_vp * max(len(peer_rows), 1))(*[int(a) for a in peer_rows])
-            _check(L.east_table_groups_dev(_vp(text_devptr), _ptr(doc_off, _i64p), _ptr(doc_m, _i32p), len(doc_m), int(device),
-                                           _vp(kp_devptr), kp_host, _ptr(kp_off, _i64p), len(kp_off) - 1,
-                                           _ptr(group_off, _i64p), len(group_off) - 1, _vp(out_devptr), peers, len(peer_rows),
-                                           _vp(stream), ctypes.byref(h)))
-            return cls.from_handle(h, doc_off, doc_m, int(device))
+            return cls._adopt(L.east_table_groups_dev, doc_off, doc_m, device, *args, gp, G, _vp(out_devptr),
+                              *_peers_arg(peer_rows), _vp(stream))
         if peer_rows:
-            peers = (_vp * len(peer_rows))(*[int(a) for a in peer_rows])
-            _check(L.east_table_dev_gather(_vp(text_devptr), _ptr(doc_off, _i64p), _ptr(doc_m, _i32p), len(doc_m), int(device),
-                                           _vp(kp_devptr), kp_host, _ptr(kp_off, _i64p), len(kp_off) - 1,
-                                           1 if normalized else 0, _vp(out_devptr), peers, len(peer_rows), _vp(stream),
-                                           ctypes.byref(h)))
-            return cls.from_handle(h, doc_off, doc_m, int(device))
-        _check(L.east_table_dev(_vp(text_devptr), _ptr(doc_off, _i64p), _ptr(doc_m, _i32p), len(doc_m), int(device),
-                                _vp(kp_devptr), kp_host, _ptr(kp_off, _i64p), len(kp_off) - 1, 1 if normalized else 0,
-                                _vp(out_devptr), _vp(stream), ctypes.byref(h)))
-        return cls.from_handle(h, doc_off, doc_m, int(device))
+            return cls._adopt(L.east_table_dev_gather, doc_off, doc_m, device, *args, 1 if normalized else 0, _vp(out_devptr),
+                              *_peers_arg(peer_rows), _vp(stream))
+        return cls._adopt(L.east_table_dev, doc_off, doc_m, device, *args, 1 if normalized else 0, _vp(out_devptr), _vp(stream))
 
     def score_table_into(self, kp_codes, kp_off, out, normalized=True):
         """score_table() into a caller-provided float64 [n_docs, K] host array (may be pinned)."""

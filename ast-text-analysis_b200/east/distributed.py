@@ -124,6 +124,15 @@ def _pack_local(texts):
     return cols, packed, plan_batches([len(p) for p in packed])
 
 
+def _upload_batch(packed, cols, docs, dev):
+    """One device batch of _pack_local's documents: (its packed text concatenated on `dev`, doc_off, doc_m)."""
+    import torch
+    doc_off = np.zeros(len(docs) + 1, dtype=np.int64)
+    np.cumsum([len(packed[j]) for j in docs], out=doc_off[1:])
+    text = np.ascontiguousarray(np.concatenate([packed[j] for j in docs]) if len(docs) > 1 else packed[docs[0]], dtype=np.uint32)
+    return torch.from_numpy(text.view(np.int32)).to(dev), doc_off, [len(cols[j]) for j in docs]
+
+
 def relevance_table_sharded(texts, prepared_keyphrases, normalized=True, device=None, group=None, fused_gather=None,
                             return_local=False, synonimizer=None):
     """[D, K] float64 score table of all texts x keyphrases, computed by all ranks together.
@@ -164,14 +173,10 @@ def relevance_table_sharded(texts, prepared_keyphrases, normalized=True, device=
     kp_dev = torch.from_numpy(codes.view(np.int32).copy()).to(dev)
 
     def score_batch(docs, out_ptr, peer_rows):
-        doc_off = np.zeros(len(docs) + 1, dtype=np.int64)
-        np.cumsum([len(packed[j]) for j in docs], out=doc_off[1:])
-        text = np.ascontiguousarray(np.concatenate([packed[j] for j in docs]) if len(docs) > 1 else packed[docs[0]],
-                                    dtype=np.uint32)
-        text_dev = torch.from_numpy(text.view(np.int32)).to(dev)
-        _capi.DeviceIndex.build_dev_and_score(text_dev.data_ptr(), doc_off, [len(cols[j]) for j in docs], kp_dev.data_ptr(),
-                                              codes, off, out_ptr, normalized, device=device, stream=stream.cuda_stream,
-                                              peer_rows=peer_rows, group_off=group_off).close()
+        text_dev, doc_off, doc_m = _upload_batch(packed, cols, docs, dev)
+        _capi.DeviceIndex.build_dev_and_score(text_dev.data_ptr(), doc_off, doc_m, kp_dev.data_ptr(), codes, off, out_ptr,
+                                              normalized, device=device, stream=stream.cuda_stream, peer_rows=peer_rows,
+                                              group_off=group_off).close()
 
     table = None
     if fused:
@@ -259,14 +264,10 @@ def keyphrases_graph_sharded(keyphrases, texts, referral_confidence=0.6, relevan
         kp_dev = torch.from_numpy(codes.view(np.int32).copy()).to(dev)
         part = torch.empty_like(cooc) if len(batches) > 1 else cooc
         for b, docs in enumerate(batches):
-            doc_off = np.zeros(len(docs) + 1, dtype=np.int64)
-            np.cumsum([len(packed[j]) for j in docs], out=doc_off[1:])
-            text = np.ascontiguousarray(np.concatenate([packed[j] for j in docs]) if len(docs) > 1 else packed[docs[0]],
-                                        dtype=np.uint32)
-            text_dev = torch.from_numpy(text.view(np.int32)).to(dev)
+            text_dev, doc_off, doc_m = _upload_batch(packed, cols, docs, dev)
             target = cooc if b == 0 else part
-            _capi.DeviceIndex.build_dev_and_graph(text_dev.data_ptr(), doc_off, [len(cols[j]) for j in docs], kp_dev.data_ptr(),
-                                                  codes, off, relevance_threshold, target.data_ptr(), normalized, device=device,
+            _capi.DeviceIndex.build_dev_and_graph(text_dev.data_ptr(), doc_off, doc_m, kp_dev.data_ptr(), codes, off,
+                                                  relevance_threshold, target.data_ptr(), normalized, device=device,
                                                   stream=stream.cuda_stream, group_off=group_off).close()
             if b > 0:
                 cooc += part   # int32: exact

@@ -17,7 +17,11 @@
  *     several documents are concatenated and delimited by doc_off[n_docs+1];
  *   - *_host entry points take host buffers and do their own H<->D copies;
  *     *_dev entry points take device pointers that live on the index's device;
- *   - there is no CPU fallback: without a usable CUDA device every entry point fails.
+ *   - there is no CPU fallback: without a usable CUDA device every entry point fails;
+ *   - the build-and-score entries (east_table_*, east_graph_*) and the score entries (east_score_*) check their
+ *     arguments before they touch the device, in one order, and report the first failure: the output (and the peer
+ *     list, text_width); the documents (raw texts: their offsets; a score entry: the index and the document range);
+ *     the groups; the keyphrases (EAST_ERR_ZERODIV for an empty one).
  */
 #ifndef EAST_B200_H
 #define EAST_B200_H

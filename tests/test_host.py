@@ -111,6 +111,69 @@ def test_argument_validation_needs_no_gpu():
         _capi.DeviceIndex.build_host_and_score(text, good_off, m, np.array([65], dtype=np.uint32), np.array([0, 1, 1]), out)
 
 
+def test_every_build_and_score_entry_checks_its_arguments_in_one_order_without_a_gpu():
+    # every check runs before the first CUDA call (no DeviceError without a GPU, no fake pointer is ever dereferenced),
+    # in one order: output, documents (raw texts: their offsets), groups, keyphrases
+    from east import _capi
+    Dx = _capi.DeviceIndex
+    fake = 1 << 20   # device addresses the calls must never reach
+    text32, text8 = np.array([65, 0x0A00], dtype=np.uint32), np.array([65, 0xFF], dtype=np.uint8)
+    m = np.array([1], dtype=np.int32)
+    docs = {"bad": np.array([0, 0], dtype=np.int64), "good": np.array([0, 2], dtype=np.int64)}
+    texts = {"bad": (np.frombuffer(b"ABC DEF", dtype=np.uint8), np.array([0, 7, 3], dtype=np.int64)),
+             "good": (np.frombuffer(b"ABC DEF", dtype=np.uint8), np.array([0, 3, 7], dtype=np.int64))}
+    codes, empty_kp = np.array([65], dtype=np.uint32), np.array([0, 1, 1], dtype=np.int64)   # the second keyphrase is empty
+    groups, bad_groups = np.array([0, 2], dtype=np.int64), np.array([0, 3], dtype=np.int64)
+
+    def table(n, g):
+        return np.zeros((n, 2 if g is None else len(g) - 1))
+
+    def host(t):
+        return lambda d, g: Dx.build_host_and_score(t, docs[d], m, codes, empty_kp, table(1, g), group_off=g)
+
+    entries = {   # C entry: call(documents, group_off)
+        "east_table_host": host(text32),
+        "east_table_host_u8": host(text8),
+        "east_table_host_gather": lambda d, g: Dx.build_host_and_score(text32, docs[d], m, codes, empty_kp, table(1, g),
+                                                                       own_rows=fake),
+        "east_table_dev": lambda d, g: Dx.build_dev_and_score(fake, docs[d], m, fake, None, empty_kp, fake),   # no host copy
+        "east_table_dev_gather": lambda d, g: Dx.build_dev_and_score(fake, docs[d], m, fake, codes, empty_kp, fake,
+                                                                     peer_rows=[fake]),
+        "east_table_texts_host": lambda d, g: Dx.table_from_texts(texts[d], codes, empty_kp, table(2, g)),
+        "east_table_groups_host": host(text32),
+        "east_table_groups_dev": lambda d, g: Dx.build_dev_and_score(fake, docs[d], m, fake, codes, empty_kp, fake, group_off=g),
+        "east_table_texts_groups_host": lambda d, g: Dx.table_from_texts(texts[d], codes, empty_kp, table(2, g),
+                                                                         group_off=g),
+        "east_graph_host": lambda d, g: Dx.build_host_and_graph(text32, docs[d], m, codes, empty_kp, 0.5, group_off=g),
+        "east_graph_dev": lambda d, g: Dx.build_dev_and_graph(fake, docs[d], m, fake, None, empty_kp, 0.5, fake, group_off=g),
+        "east_graph_texts_host": lambda d, g: Dx.graph_from_texts(texts[d], codes, empty_kp, 0.5, group_off=g),
+    }
+    for name, call in entries.items():
+        # the groups entries always take groups; the graph entries with and without them
+        for g in ([groups] if "_groups_" in name else [None, groups] if "_graph_" in name else [None]):
+            with pytest.raises(ValueError):   # malformed documents before the empty keyphrase
+                call("bad", g)
+            with pytest.raises(ZeroDivisionError):
+                call("good", g)
+        if "_groups_" in name or "_graph_" in name:
+            with pytest.raises(ValueError):   # malformed groups before the empty keyphrase
+                call("good", bad_groups)
+    # the score calls on an index: a NULL index before the (empty) keyphrases
+    L = _capi.load()
+    kp, off = codes.ctypes.data_as(ctypes.POINTER(ctypes.c_uint32)), empty_kp.ctypes.data_as(ctypes.POINTER(ctypes.c_int64))
+    gp = groups.ctypes.data_as(ctypes.POINTER(ctypes.c_int64))
+    out = np.zeros(4).ctypes.data_as(ctypes.POINTER(ctypes.c_double))
+    probes, score = ctypes.c_int64(), ctypes.c_double()
+    for rc in (L.east_score_table_host(None, kp, off, 2, 1, out),
+               L.east_score_table_dev(None, fake, off, 2, 1, fake, None),
+               L.east_score_range_dev(None, fake, off, 2, 1, 0, 1, fake, None),
+               L.east_score_probes_dev(None, fake, off, 2, fake, None, ctypes.byref(probes)),
+               L.east_score_groups_host(None, kp, off, 2, gp, 1, 0, 1, out),
+               L.east_score_groups_dev(None, fake, off, 2, gp, 1, 0, 1, fake, None),
+               L.east_score_one(None, 0, kp, 0, 1, ctypes.byref(score), None)):
+        assert rc == -1, L.east_last_error()
+
+
 def test_synthetic_generator_is_deterministic():
     import synth
     d1, d2 = synth.document(10000, 1), synth.document(10000, 1)
