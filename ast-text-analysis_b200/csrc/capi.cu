@@ -268,6 +268,8 @@ static void use_device(int device) {
 using namespace east;
 
 struct east_index {
+    // device and n_docs lead the struct: the argument checks of the entries on an index read only n_docs, and
+    // tests/test_gpu_index_graph.py exercises them without a GPU on a stand-in that holds just these two fields
     int device = 0;
     int32_t n_docs = 0;
     int32_t n = 0;
@@ -1088,19 +1090,27 @@ static int cooc_tc_kernel() {
 // A graph call fills B[k][d] = (score of document d in column k >= threshold), the zero-padded Kp x Dp byte matrix of the
 // co-occurrence GEMM (cooc_tc.cu), and never a documents x keyphrases table: the per-document kernel stores its column of
 // bytes itself (k_doc_suffix_sort_graph); every other path scores tiles of documents into an fp64 scratch bounded by the
-// score_tmp_doubles budget and thresholds each tile into its columns (graph_enqueue).
+// score_tmp_doubles budget and thresholds each tile into its columns (graph_enqueue).  A graph call on an existing index
+// takes up to MAX_THRESHOLDS thresholds: B then holds one plane per threshold, all written from one read of each tile,
+// and C one cols x cols plane of counts per threshold.
 struct GraphOut {
-    double threshold = 0.0;
-    int32_t *C = nullptr;   // device: cols x cols counts
+    const double *thresholds = nullptr;   // T of them (the build-and-score entries: one)
+    int32_t T = 1;
+    int32_t *C = nullptr;   // device: T x cols x cols counts
+    int64_t doc0 = 0;       // the document column 0 of B stands for: 0 for a whole batch, doc_begin for a range of an index
     DevBuf<uint8_t> B;
     int64_t Dp = 0;
     int32_t Kp = 0;
+    size_t plane() const { return (size_t)Kp * (size_t)Dp; }
     void begin(int32_t n_docs, int32_t cols, cudaStream_t s) {
         cooc_padding(n_docs, cols, &Dp, &Kp);
-        B = DevBuf<uint8_t>((size_t)Kp * (size_t)Dp, s);
-        EAST_CUDA(cudaMemsetAsync(B.p, 0, (size_t)Kp * (size_t)Dp, s));   // padding rows / columns stay zero
+        B = DevBuf<uint8_t>((size_t)T * plane(), s);
+        EAST_CUDA(cudaMemsetAsync(B.p, 0, (size_t)T * plane(), s));   // padding rows / columns stay zero
     }
-    void finish(int32_t cols, cudaStream_t s) const { cooc_counts_bytes(B.p, Dp, Kp, cols, C, s, cooc_tc_kernel()); }
+    void finish(int32_t cols, cudaStream_t s) const {
+        for (int32_t t = 0; t < T; ++t)
+            cooc_counts_bytes(B.p + (size_t)t * plane(), Dp, Kp, cols, C + (size_t)t * cols * cols, s, cooc_tc_kernel());
+    }
 };
 
 // Where a call's results go: the rows of a table on the device (the caller's; host entries: the call's own, copied to
@@ -1129,15 +1139,16 @@ struct Output {
         o.to_host = true; o.rows_host = host;
         return o;
     }
-    static Output counts(double threshold, int32_t *C_dev, int32_t *C_host) {
+    // thresholds: T host doubles, read while the call runs
+    static Output counts(const double *thresholds, int32_t T, int32_t *C_dev, int32_t *C_host) {
         Output o;
-        o.is_graph = true; o.graph.threshold = threshold; o.graph.C = C_dev; o.counts_host = C_host;
+        o.is_graph = true; o.graph.thresholds = thresholds; o.graph.T = T; o.graph.C = C_dev; o.counts_host = C_host;
         return o;
     }
     void begin(int32_t n_docs, int32_t cols, cudaStream_t s) {
         if (is_graph) {
             if (counts_host) {
-                own_counts = DevBuf<int32_t>((size_t)cols * cols, s);
+                own_counts = DevBuf<int32_t>((size_t)graph.T * cols * cols, s);
                 graph.C = own_counts.p;
             }
             graph.begin(n_docs, cols, s);
@@ -1188,6 +1199,8 @@ static void validate(const Output &out, const Source *src, const Query &q, const
                      int32_t doc_begin = 0, int32_t doc_count = 0) {
     if (out.is_graph ? !out.graph.C && !out.counts_host : !(out.to_host ? out.rows_host : out.rows))
         throw Error(EAST_ERR_INVALID, "bad argument");
+    if (out.is_graph && (out.graph.T < 1 || out.graph.T > MAX_THRESHOLDS || !out.graph.thresholds))
+        throw Error(EAST_ERR_INVALID, "a graph takes 1 to 8 relevance thresholds");
     if (out.n_peers < 0 || out.n_peers > DocScore::MAX_PEERS || (out.n_peers > 0 && !out.peer_rows))
         throw Error(EAST_ERR_INVALID, "bad peer list");
     if (src && src->width != 1 && src->width != 4) throw Error(EAST_ERR_INVALID, "text_width must be 1 or 4");
@@ -1317,13 +1330,14 @@ static int32_t graph_tile_docs(int32_t doc_count, int32_t cols) {
 }
 
 // score_enqueue for a graph: documents [doc_begin, doc_begin + doc_count) tile by tile into S[S_docs][cols], each tile
-// thresholded into its columns of g.B (stream-ordered: the next tile overwrites S after the previous one is read)
+// thresholded into its columns of every plane of g.B (stream-ordered: the next tile overwrites S after the previous one
+// is read)
 static void graph_enqueue(const east_index *idx, const KpPrepared *kp, const Query &q, int32_t doc_begin, int32_t doc_count,
                           cudaStream_t s, double *tmp, int32_t tile_docs, const GraphOut &g, double *S, int32_t S_docs) {
     for (int32_t d0 = 0; d0 < doc_count; d0 += S_docs) {
         const int32_t cnt = std::min(S_docs, doc_count - d0);
         score_enqueue(idx, kp, q, S, doc_begin + d0, cnt, s, tmp, tile_docs, nullptr);
-        threshold_bytes(S, cnt, q.cols(), g.threshold, g.B.p, g.Dp, (int64_t)doc_begin + d0, s);
+        threshold_bytes(S, cnt, q.cols(), g.thresholds, g.T, g.B.p, g.Dp, (int64_t)g.plane(), (int64_t)doc_begin + d0 - g.doc0, s);
     }
 }
 
@@ -1375,6 +1389,7 @@ static void score_common(const east_index *idx, Query &q, double *out_dev, const
 }
 
 // The score calls on an index: checked, then scored; the host entries upload the code points and copy the rows back.
+// A graph output gets the relevance bytes of the range (column 0 = document doc_begin) and then its counts.
 static void score_index(const east_index *idx, Query q, Output out, int32_t doc_begin, int32_t doc_count, void *stream,
                         int64_t *probes = nullptr) {
     validate(out, nullptr, q, idx, doc_begin, doc_count);
@@ -1382,9 +1397,17 @@ static void score_index(const east_index *idx, Query q, Output out, int32_t doc_
     cudaStream_t s = (cudaStream_t)stream;
     DevBuf<uint32_t> d_kp;
     if (q.on_host) d_kp = q.upload(s);
+    out.graph.doc0 = doc_begin;
     out.begin(doc_count, q.cols(), s);
-    score_common(idx, q, out.rows, nullptr, doc_begin, doc_count, s, nullptr, probes);
+    score_common(idx, q, out.rows, out.is_graph ? &out.graph : nullptr, doc_begin, doc_count, s, nullptr, probes);
     if (out.to_host) EAST_CUDA(cudaMemcpy(out.rows_host, out.rows, sizeof(double) * (size_t)doc_count * q.cols(), cudaMemcpyDeviceToHost));
+    if (out.is_graph) {
+        const size_t counts = (size_t)out.graph.T * q.cols() * q.cols();
+        out.graph.finish(q.cols(), s);
+        if (out.counts_host) EAST_CUDA(cudaMemcpyAsync(out.counts_host, out.graph.C, sizeof(int32_t) * counts, cudaMemcpyDeviceToHost, s));
+        EAST_CUDA(cudaStreamSynchronize(s));
+        ktime_collect();   // option time_kernels: the GEMM launches belong to this call's kernel statistics
+    }
 }
 
 int east_score_table_dev(const east_index *idx, const uint32_t *kp_dev, const int64_t *kp_off, int32_t K,
@@ -1433,6 +1456,26 @@ int east_score_table_host(const east_index *idx, const uint32_t *kp, const int64
                           int normalized, double *out_DxK) {
     EAST_API_BEGIN
     score_index(idx, Query(kp, true, nullptr, kp_off, K, normalized), Output::table_host(out_DxK), 0, idx ? idx->n_docs : 0, 0);
+    EAST_API_END
+}
+
+// keyphrase graphs on an existing index: the counts of documents [doc_begin, doc_begin + doc_count) at every threshold,
+// no score table (group_off NULL: plain keyphrases)
+int east_graph_index_host(const east_index *idx, const uint32_t *kp, const int64_t *kp_off, int32_t V, const int64_t *group_off,
+                          int32_t G, int normalized, const double *thresholds, int32_t n_thresholds, int32_t doc_begin,
+                          int32_t doc_count, int32_t *C_host) {
+    EAST_API_BEGIN
+    score_index(idx, Query(kp, true, nullptr, kp_off, V, normalized, group_off != nullptr, group_off, G),
+                Output::counts(thresholds, n_thresholds, nullptr, C_host), doc_begin, doc_count, 0);
+    EAST_API_END
+}
+
+int east_graph_index_dev(const east_index *idx, const uint32_t *kp_dev, const uint32_t *kp_host, const int64_t *kp_off, int32_t V,
+                         const int64_t *group_off, int32_t G, int normalized, const double *thresholds, int32_t n_thresholds,
+                         int32_t doc_begin, int32_t doc_count, int32_t *C_dev, void *stream) {
+    EAST_API_BEGIN
+    score_index(idx, Query(kp_dev, false, kp_host, kp_off, V, normalized, group_off != nullptr, group_off, G),
+                Output::counts(thresholds, n_thresholds, C_dev, nullptr), doc_begin, doc_count, stream);
     EAST_API_END
 }
 
@@ -1617,7 +1660,7 @@ static void table_run_begin(void *vctx, const RunReady &r, DocScore &score) {
             score.kp_off = t.kp->dev.d_off.p; score.uniq_of = t.kp->dev.d_uniq_of.p; score.K = q.K;
             if (t.out.is_graph) {
                 score.graph = t.out.graph.B.p; score.graph_pitch = t.out.graph.Dp; score.graph_col0 = r.doc_begin;
-                score.threshold = t.out.graph.threshold;
+                score.threshold = t.out.graph.thresholds[0];   // the build-and-score graph entries take one threshold
             } else {
                 score.out = t.out.rows + (size_t)r.doc_begin * q.cols();
             }
@@ -1826,7 +1869,7 @@ int east_graph_host(const void *text, int32_t text_width, const int64_t *doc_off
     EAST_API_BEGIN
     run_table({Source::HOST, text, text_width, doc_off, doc_m, n_docs, device},
               Query(kp, true, nullptr, kp_off, V, normalized, group_off != nullptr, group_off, G),
-              Output::counts(threshold, nullptr, C_host), out_idx);
+              Output::counts(&threshold, 1, nullptr, C_host), out_idx);
     EAST_API_END
 }
 
@@ -1836,7 +1879,7 @@ int east_graph_dev(const uint32_t *text_dev, const int64_t *doc_off, const int32
     EAST_API_BEGIN
     run_table({Source::DEVICE, text_dev, 4, doc_off, doc_m, n_docs, device, (cudaStream_t)stream},
               Query(kp_dev, false, kp_host, kp_off, V, normalized, group_off != nullptr, group_off, G),
-              Output::counts(threshold, C_dev, nullptr), out_idx);
+              Output::counts(&threshold, 1, C_dev, nullptr), out_idx);
     EAST_API_END
 }
 
@@ -1846,7 +1889,7 @@ int east_graph_texts_host(const uint8_t *utf8, const int64_t *text_off, int32_t 
     EAST_API_BEGIN
     run_table({Source::TEXTS, utf8, 1, text_off, nullptr, n_texts, device, 0, doc_off_out, doc_m_out},
               Query(kp, true, nullptr, kp_off, V, normalized, group_off != nullptr, group_off, G),
-              Output::counts(threshold, nullptr, C_host), out_idx);
+              Output::counts(&threshold, 1, nullptr, C_host), out_idx);
     EAST_API_END
 }
 

@@ -46,6 +46,18 @@ void host_debug_mark(const char *what);   // EAST_DEBUG_TIMING: host timestamp o
         if (_e != cudaSuccess)                                                               \
             throw ::east::Error(-2, std::string(#kernel) + " launch: " + cudaGetErrorString(_e)); \
     } while (0)
+// the same for an instance of a kernel template, counted and timed under `name` (every instance under one name)
+#define EAST_LAUNCH_AS(name, kernel, grid, block, smem, stream, ...)                         \
+    do {                                                                                     \
+        if (::east::g_time_kernels) ::east::ktime_begin((name), (stream));                   \
+        kernel<<<(grid), (block), (smem), (stream)>>>(__VA_ARGS__);                          \
+        if (::east::g_time_kernels) ::east::ktime_end((stream));                             \
+        ++::east::g_launches;                                                                \
+        ::east::g_next_bytes = 0.0;                                                          \
+        cudaError_t _e = cudaGetLastError();                                                 \
+        if (_e != cudaSuccess)                                                               \
+            throw ::east::Error(-2, std::string(name) + " launch: " + cudaGetErrorString(_e)); \
+    } while (0)
 #define EAST_BYTES(b) (::east::g_next_bytes = (double)(b))
 
 // Stream-ordered allocations from two library-private memory pools per device (the device's default pool and its

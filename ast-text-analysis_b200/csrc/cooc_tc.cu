@@ -56,17 +56,21 @@ __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
     } while (!done);
 }
 
-// S[d][k] >= thr  ->  Bm[k][col0 + d] (uint8): 128 (documents) x 32 (keyphrases) transposing tiles through shared memory.
-// Reads: a warp takes 32 consecutive doubles of a row of S (256 bytes), four rows in flight per thread; writes: every
-// keyphrase row of the tile leaves as 128 contiguous bytes (eight 16-byte stores).  HBM-bound: 8 D K bytes in, D K out.
+// S[d][k] >= thr.v[t]  ->  Bm[t * plane + k * Dp + col0 + d] (uint8), for the T <= MAX_THRESHOLDS thresholds of one
+// call: 128 (documents) x 32 (keyphrases) transposing tiles through shared memory, one tile per threshold.
+// Reads: a warp takes 32 consecutive doubles of a row of S (256 bytes), four rows in flight per thread, each double is
+// loaded once and compared with every threshold; writes: every keyphrase row of a plane's tile leaves as 128 contiguous
+// bytes (eight 16-byte stores).  HBM-bound: 8 D K bytes in, T D K out.
 // Only the columns [col0, col0 + D) are written, so that document tiles scored one after another (possibly on two
 // streams) fill their own columns of one matrix; a piece that is not a whole aligned 16 bytes inside them is stored
-// byte by byte.
+// byte by byte.  One instance per T (T x 4.5 KB of static shared memory, 36 KB at T = 8): T = 1 is the single-threshold
+// kernel with the footprint, registers and occupancy of a single tile.
 constexpr int TB_D = 128, TB_K = 32;
+template <int T>
 __global__ void __launch_bounds__(256)
-k_threshold_bytes(const double *__restrict__ S, int64_t D, int32_t K, double thr, uint8_t *__restrict__ Bm,
-                  int64_t Dp, int64_t col0) {
-    __shared__ __align__(16) uint8_t tile[TB_K][TB_D + 16];    // [k][d]: the store phase reads 16 consecutive d of one k
+k_threshold_bytes(const double *__restrict__ S, int64_t D, int32_t K, ThresholdSet thr, uint8_t *__restrict__ Bm,
+                  int64_t Dp, int64_t plane, int64_t col0) {
+    __shared__ __align__(16) uint8_t tile[T][TB_K][TB_D + 16];   // [t][k][d]: the store phase reads 16 consecutive d of one k
     const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;  // 32 x 8
     const int64_t d0 = (int64_t)blockIdx.x * TB_D;
     const int32_t k0 = blockIdx.y * TB_K;
@@ -82,7 +86,8 @@ k_threshold_bytes(const double *__restrict__ S, int64_t D, int32_t K, double thr
 #pragma unroll
         for (int u = 0; u < 4; ++u) {
             const int64_t d = d0 + r0 + ty + 8 * u;
-            tile[tx][r0 + ty + 8 * u] = (d < D && k < K && v[u] >= thr) ? 1 : 0;
+#pragma unroll
+            for (int t = 0; t < T; ++t) tile[t][tx][r0 + ty + 8 * u] = (d < D && k < K && v[u] >= thr.v[t]) ? 1 : 0;
         }
     }
     __syncthreads();
@@ -91,11 +96,14 @@ k_threshold_bytes(const double *__restrict__ S, int64_t D, int32_t K, double thr
     const int32_t ko = k0 + kr;
     const int64_t dd = d0 + 16 * piece;
     if (ko < K && dd < D) {
-        uint8_t *dst = Bm + (int64_t)ko * Dp + col0 + dd;
-        if (dd + 16 <= D && (col0 & 15) == 0) {
-            *reinterpret_cast<uint4 *>(dst) = *reinterpret_cast<const uint4 *>(&tile[kr][16 * piece]);
-        } else {
-            for (int i = 0; i < 16 && dd + i < D; ++i) dst[i] = tile[kr][16 * piece + i];
+#pragma unroll
+        for (int t = 0; t < T; ++t) {
+            uint8_t *dst = Bm + t * plane + (int64_t)ko * Dp + col0 + dd;
+            if (dd + 16 <= D && (col0 & 15) == 0) {
+                *reinterpret_cast<uint4 *>(dst) = *reinterpret_cast<const uint4 *>(&tile[t][kr][16 * piece]);
+            } else {
+                for (int i = 0; i < 16 && dd + i < D; ++i) dst[i] = tile[t][kr][16 * piece + i];
+            }
         }
     }
 }
@@ -538,11 +546,25 @@ void cooc_padding(int64_t D, int32_t K, int64_t *Dp, int32_t *Kp) {
     *Kp = (K + CP_TN - 1) / CP_TN * CP_TN;   // rows padded to the larger tile edge (256)
 }
 
-void threshold_bytes(const double *S_DxK, int64_t D, int32_t K, double threshold, uint8_t *Bm, int64_t Dp, int64_t col0,
-                     cudaStream_t s) {
+template <int T>
+static void launch_threshold_bytes(dim3 grid, cudaStream_t s, const double *S_DxK, int64_t D, int32_t K, const ThresholdSet &thr,
+                                   uint8_t *Bm, int64_t Dp, int64_t plane, int64_t col0) {
+    EAST_LAUNCH_AS("k_threshold_bytes", k_threshold_bytes<T>, grid, 256, 0, s, S_DxK, D, K, thr, Bm, Dp, plane, col0);
+}
+
+void threshold_bytes(const double *S_DxK, int64_t D, int32_t K, const double *thresholds, int32_t T, uint8_t *Bm, int64_t Dp,
+                     int64_t plane, int64_t col0, cudaStream_t s) {
+    using Launch = void (*)(dim3, cudaStream_t, const double *, int64_t, int32_t, const ThresholdSet &, uint8_t *, int64_t,
+                            int64_t, int64_t);
+    static const Launch launch[MAX_THRESHOLDS] = {launch_threshold_bytes<1>, launch_threshold_bytes<2>, launch_threshold_bytes<3>,
+                                                  launch_threshold_bytes<4>, launch_threshold_bytes<5>, launch_threshold_bytes<6>,
+                                                  launch_threshold_bytes<7>, launch_threshold_bytes<8>};
+    if (T < 1 || T > MAX_THRESHOLDS) throw Error(-1, "threshold_bytes: 1 to 8 thresholds");
+    ThresholdSet thr{};
+    for (int32_t t = 0; t < T; ++t) thr.v[t] = thresholds[t];
     dim3 tg((unsigned)((D + TB_D - 1) / TB_D), (unsigned)((K + TB_K - 1) / TB_K));
-    EAST_BYTES(8.0 * (double)D * K + (double)K * D);
-    EAST_LAUNCH(k_threshold_bytes, tg, 256, 0, s, S_DxK, D, K, threshold, Bm, Dp, col0);
+    EAST_BYTES(8.0 * (double)D * K + (double)T * K * D);
+    launch[T - 1](tg, s, S_DxK, D, K, thr, Bm, Dp, plane, col0);
 }
 
 void cooc_counts_tc(const double *S_DxK, int64_t D, int32_t K, double threshold, int32_t *C, cudaStream_t s, int simple) {
@@ -551,7 +573,7 @@ void cooc_counts_tc(const double *S_DxK, int64_t D, int32_t K, double threshold,
     cooc_padding(D, K, &Dp, &Kp);
     DevBuf<uint8_t> Bm((size_t)Kp * (size_t)Dp, s);
     EAST_CUDA(cudaMemsetAsync(Bm.p, 0, (size_t)Kp * (size_t)Dp, s));  // padding rows / columns are zero
-    threshold_bytes(S_DxK, D, K, threshold, Bm.p, Dp, 0, s);
+    threshold_bytes(S_DxK, D, K, &threshold, 1, Bm.p, Dp, 0, 0, s);
     cooc_counts_bytes(Bm.p, Dp, Kp, K, C, s, simple);
 }
 

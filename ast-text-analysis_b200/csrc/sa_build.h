@@ -230,9 +230,13 @@ void cooc_counts_tc(const double *S_DxK, int64_t D, int32_t K, double threshold,
                     int simple = 0 /* 0: TMA-fed cluster kernel, 1: the non-pipelined 128 x 128 kernel, 2: the cp.async pipeline */);
 // the relevance bytes of D documents x K keyphrases: Bm[Kp][Dp], Dp = D rounded up to 128, Kp = K rounded up to 256
 void cooc_padding(int64_t D, int32_t K, int64_t *Dp, int32_t *Kp);
-// Bm[k][col0 + d] = (S[d][k] >= threshold) for d < D, k < K (S: D x K doc-major); nothing else of Bm is written
-void threshold_bytes(const double *S_DxK, int64_t D, int32_t K, double threshold, uint8_t *Bm, int64_t Dp, int64_t col0,
-                     cudaStream_t s);
+// up to MAX_THRESHOLDS relevance thresholds, passed to k_threshold_bytes by value
+constexpr int MAX_THRESHOLDS = 8;
+struct ThresholdSet { double v[MAX_THRESHOLDS]; };
+// Bm[t * plane + k * Dp + col0 + d] = (S[d][k] >= thresholds[t]) for d < D, k < K, t < T (S: D x K doc-major, read once;
+// 1 <= T <= MAX_THRESHOLDS planes `plane` bytes apart); nothing else of Bm is written
+void threshold_bytes(const double *S_DxK, int64_t D, int32_t K, const double *thresholds, int32_t T, uint8_t *Bm, int64_t Dp,
+                     int64_t plane, int64_t col0, cudaStream_t s);
 // C = Bm Bm^T (K x K int32) from a prepared, zero-padded Kp x Dp matrix
 void cooc_counts_bytes(const uint8_t *Bm, int64_t Dp, int32_t Kp, int32_t K, int32_t *C, cudaStream_t s, int simple = 0);
 

@@ -37,6 +37,7 @@ EXPORTED_SYMBOLS = [
     "east_score_groups_host", "east_score_groups_dev",
     "east_table_groups_host", "east_table_groups_dev", "east_table_texts_groups_host",
     "east_graph_host", "east_graph_dev", "east_graph_texts_host",
+    "east_graph_index_host", "east_graph_index_dev",
 ]
 
 _lib = None
@@ -107,6 +108,10 @@ def load():
                                  ctypes.c_int32, ctypes.c_int, ctypes.c_double, _vp, _vp, ctypes.POINTER(_vp)]
     L.east_graph_texts_host.argtypes = [_u8p, _i64p, ctypes.c_int32, ctypes.c_int, _u32p, _i64p, ctypes.c_int32, _i64p,
                                         ctypes.c_int32, ctypes.c_int, ctypes.c_double, _i32p, _i64p, _i32p, ctypes.POINTER(_vp)]
+    L.east_graph_index_host.argtypes = [_vp, _u32p, _i64p, ctypes.c_int32, _i64p, ctypes.c_int32, ctypes.c_int, _f64p,
+                                        ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, _i32p]
+    L.east_graph_index_dev.argtypes = [_vp, _vp, _u32p, _i64p, ctypes.c_int32, _i64p, ctypes.c_int32, ctypes.c_int, _f64p,
+                                       ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, _vp, _vp]
     L.east_score_probes_dev.argtypes = [_vp, _vp, _i64p, ctypes.c_int32, _vp, _vp, _i64p]
     L.east_score_one.argtypes = [_vp, ctypes.c_int32, _u32p, ctypes.c_int32, ctypes.c_int, _f64p, _f64p]
     L.east_cooc_dev.argtypes = [_vp, ctypes.c_int64, ctypes.c_int32, ctypes.c_double, _vp, ctypes.c_int, _vp]
@@ -618,6 +623,42 @@ class DeviceIndex(object):
         _check(load().east_score_groups_dev(self._h, _vp(kp_devptr), _ptr(kp_off, _i64p), len(kp_off) - 1,
                                             _ptr(group_off, _i64p), len(group_off) - 1, int(doc_begin), int(doc_count),
                                             _vp(out_devptr), _vp(stream)))
+        self.score_timings = last_timings()
+
+    def _graph_args(self, kp_codes, kp_off, thresholds, group_off, doc_begin, doc_count):
+        """(keyphrase, group, threshold and range arguments of east_graph_index_*, cols, T, scalar threshold?)"""
+        scalar = np.ndim(thresholds) == 0
+        thr = np.ascontiguousarray(np.atleast_1d(np.asarray(thresholds, dtype=np.float64)).ravel())
+        kp_codes, kp_off, K = _keyphrases_args(kp_codes, kp_off)
+        group_off, gp, G = _groups_arg(group_off)
+        if doc_count is None:
+            doc_count = self.n_docs - doc_begin
+        args = (_ptr(kp_off, _i64p), K, gp, G)
+        rest = (_ptr(thr, _f64p) if thr.size else None, int(thr.size), int(doc_begin), int(doc_count))
+        return kp_codes, args, rest, max(_columns(K, group_off), 0), int(thr.size), scalar
+
+    def graph(self, kp_codes, kp_off, thresholds, normalized=True, group_off=None, doc_begin=0, doc_count=None):
+        """Keyphrase-graph counts of documents [doc_begin, doc_begin + doc_count) of this index, without a score table
+        (east_graph_index_host): C[i][j] = number of documents in which columns i and j both score >= the threshold.
+        thresholds: a number -> int32 [cols, cols]; a sequence of 1 to 8 -> int32 [T, cols, cols], all from one scoring
+        pass.  cols = K, or G with group_off (pack_variant_groups: the best variant per group, always normalized).
+        Counts of disjoint ranges add up."""
+        kp_codes, args, rest, cols, T, scalar = self._graph_args(kp_codes, kp_off, thresholds, group_off, doc_begin, doc_count)
+        if kp_codes.size == 0:
+            kp_codes = np.zeros(1, dtype=np.uint32)
+        C = np.empty((T, cols, cols), dtype=np.int32)
+        _check(load().east_graph_index_host(self._h, _ptr(kp_codes, _u32p), *args, 1 if normalized else 0, *rest,
+                                            _ptr(C, _i32p) if C.size else None))
+        self.score_timings = last_timings()
+        return C[0] if scalar else C
+
+    def graph_dev(self, kp_devptr, kp_codes, kp_off, thresholds, C_devptr, normalized=True, group_off=None, doc_begin=0,
+                  doc_count=None, stream=0):
+        """graph() with the code points and the int32 [T, cols, cols] counts on the device (east_graph_index_dev), queued
+        on `stream`.  kp_codes: host copy of the code points (or None)."""
+        kp_codes, args, rest, _, _, _ = self._graph_args(kp_codes, kp_off, thresholds, group_off, doc_begin, doc_count)
+        _check(load().east_graph_index_dev(self._h, _vp(kp_devptr), _kp_host_arg(kp_codes), *args, 1 if normalized else 0,
+                                           *rest, _vp(C_devptr), _vp(stream)))
         self.score_timings = last_timings()
 
     def score_probes_dev(self, kp_devptr, kp_off, out_devptr, stream=0):

@@ -225,7 +225,9 @@ class ASTRelevanceMeasure(RelevanceMeasure):
     @classmethod
     def load_index(cls, directory, device=0):
         """A measure over the collection saved by save_index(): relevance(), relevance_table() and the asts' attributes
-        work as after set_text_collection()."""
+        work as after set_text_collection().  cooccurrence() counts on the loaded index without a score table: with
+        applications.graph_from_cooccurrence it gives a keyphrase graph, at one or several relevance thresholds, without
+        rebuilding the collection."""
         import json
         import os
         with open(os.path.join(directory, "layout.json")) as f:
@@ -275,18 +277,46 @@ class ASTRelevanceMeasure(RelevanceMeasure):
 
     def cooccurrence(self, prepared_keyphrases, relevance_threshold, synonimizer=None):
         """int32 [K, K] co-occurrence counts: C[i][j] = number of texts in which prepared keyphrases i and j both score
-        >= relevance_threshold (with a synonimizer: their best synonym variants), C[k][k] the support of k.  The counts
-        of the graph calls made while indexing (set_text_collection with relevance_threshold) when they were made for
-        these keyphrases, variants, threshold and normalization; otherwise those of relevance_table()."""
+        >= relevance_threshold (with a synonimizer: their best synonym variants), C[k][k] the support of k.
+        relevance_threshold may also be a sequence of 1 to 8 thresholds: the result is then int32 [T, K, K], one plane
+        per threshold, from one scoring pass.
+        Where the counts come from:
+          * the graph calls made while indexing (set_text_collection with relevance_threshold), for a scalar threshold
+            equal to theirs and the same keyphrases, variants and normalization: the stored counts themselves;
+          * a measure without a device index, or one that holds the table of these keyphrases and variants (scored while
+            indexing): cooc_host of relevance_table(), per threshold;
+          * otherwise one graph call per device batch on the existing index (DeviceIndex.graph), which forms no score
+            table.  This is what a measure from load_index() does: load_index(dir).cooccurrence(prepared, r), then
+            applications.graph_from_cooccurrence, gives the graph without building an index or scoring a table.
+        Counts computed on the index are returned, not kept."""
         K = len(prepared_keyphrases)
-        if self._cooc is not None:
-            groups = _capi.pack_variant_groups(prepared_keyphrases, synonimizer.get_synonyms()) if synonimizer else None
+        scalar = np.ndim(relevance_threshold) == 0
+        thresholds = [float(relevance_threshold)] if scalar else [float(r) for r in relevance_threshold]
+        groups = _capi.pack_variant_groups(prepared_keyphrases, synonimizer.get_synonyms()) if synonimizer else None
+        if self._cooc is not None and scalar:
             kps, kgroups, kthr, knorm = self._cooc_key
-            same_groups = (groups is None) == (kgroups is None) and (
-                groups is None or all(np.array_equal(a, b) for a, b in zip(groups, kgroups)))
-            if (list(prepared_keyphrases) == kps and same_groups and float(relevance_threshold) == kthr
+            if (list(prepared_keyphrases) == kps and self._same_groups(groups, kgroups) and thresholds[0] == kthr
                     and bool(self.normalized) == knorm):
                 return self._cooc
         if not K or not self.asts:
-            return np.zeros((K, K), dtype=np.int32)
-        return _capi.cooc_host(self.relevance_table(prepared_keyphrases, synonimizer), relevance_threshold)
+            return np.zeros((K, K) if scalar else (len(thresholds), K, K), dtype=np.int32)
+        if self._index is None or self._has_table(prepared_keyphrases, groups):
+            table = self.relevance_table(prepared_keyphrases, synonimizer)
+            planes = [_capi.cooc_host(table, r) for r in thresholds]
+            return planes[0] if scalar else np.stack(planes)
+        codes, off, group_off = groups if groups else (*_capi.pack_keyphrases(prepared_keyphrases), None)
+        counts = None
+        for index, _ in self._batches:
+            part = index.graph(codes, off, thresholds, normalized=self.normalized, group_off=group_off)
+            counts = part if counts is None else counts + part   # int32: exact (counts <= number of texts)
+        return counts[0] if scalar else counts
+
+    @staticmethod
+    def _same_groups(groups, kept):
+        return (groups is None) == (kept is None) and (groups is None or all(np.array_equal(a, b) for a, b in zip(groups, kept)))
+
+    def _has_table(self, prepared_keyphrases, groups):
+        """the table scored while indexing is the one relevance_table(prepared_keyphrases, the synonimizer of groups) returns"""
+        if self._table is None or list(prepared_keyphrases) != self._table_keyphrases:
+            return False
+        return self._table_groups is None if groups is None else self._same_groups(groups, self._table_groups)

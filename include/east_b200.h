@@ -18,9 +18,10 @@
  *   - *_host entry points take host buffers and do their own H<->D copies;
  *     *_dev entry points take device pointers that live on the index's device;
  *   - there is no CPU fallback: without a usable CUDA device every entry point fails;
- *   - the build-and-score entries (east_table_*, east_graph_*) and the score entries (east_score_*) check their
- *     arguments before they touch the device, in one order, and report the first failure: the output (and the peer
- *     list, text_width); the documents (raw texts: their offsets; a score entry: the index and the document range);
+ *   - the build-and-score entries (east_table_*, east_graph_*) and the entries on an index (east_score_*,
+ *     east_graph_index_*) check their arguments before they touch the device, in one order, and report the first
+ *     failure: the output (and the peer list, text_width, the thresholds of a graph); the documents (raw texts: their
+ *     offsets; an entry on an index: the index and the document range);
  *     the groups; the keyphrases (EAST_ERR_ZERODIV for an empty one).
  */
 #ifndef EAST_B200_H
@@ -164,6 +165,30 @@ int east_score_groups_host(const east_index *idx, const uint32_t *kp, const int6
 int east_score_groups_dev(const east_index *idx, const uint32_t *kp_dev, const int64_t *kp_off, int32_t V,
                           const int64_t *group_off, int32_t G, int32_t doc_begin, int32_t doc_count,
                           double *out_dev, void *stream);
+/* keyphrase graphs on an existing index (built, returned by a table or graph entry, or loaded): replaces the pair loop
+ * of applications.keyphrases_graph (applications.py:111-147) for a collection that is already indexed, at several
+ * relevance thresholds in one scoring pass.  C[t][i][j] (int32, n_thresholds x cols x cols, row-major) = the number of
+ * documents d in [doc_begin, doc_begin + doc_count) with score(d, i) >= thresholds[t] and score(d, j) >= thresholds[t];
+ * every plane equals east_cooc_host(table, thresholds[t]) of east_score_table_host / east_score_groups_host of the same
+ * documents, element for element.  group_off NULL: kp holds V plain keyphrases, space-stripped as for
+ * east_score_table_host, scored with `normalized`, and cols = V; otherwise the variants of east_score_groups_*, always
+ * normalized, and cols = G.  thresholds: a host array of 1 <= n_thresholds <= 8 doubles in any order (a NaN counts
+ * nothing).  The documents x columns table is never formed: tiles of documents are scored into an fp64 scratch bounded
+ * by option "score_tmp_doubles" and each tile is read once to write one relevance-byte plane per threshold.  Counts of
+ * disjoint ranges add up.  Checked before the first CUDA call, in the order of the score entries: the output (NULL C,
+ * n_thresholds outside 1..8, NULL thresholds), the index and the range, the groups, the keyphrases (EAST_ERR_ZERODIV
+ * for an empty one).
+ *   east_graph_index_host: host keyphrases, C_host on the host.
+ *   east_graph_index_dev: device keyphrases (kp_host: optional host copy; kp_off, group_off and thresholds stay on the
+ *     host), C_dev on the index's device, queued on `stream` (the call returns once C_dev is written). */
+int east_graph_index_host(const east_index *idx, const uint32_t *kp, const int64_t *kp_off, int32_t V,
+                          const int64_t *group_off, int32_t G, int normalized,
+                          const double *thresholds, int32_t n_thresholds,
+                          int32_t doc_begin, int32_t doc_count, int32_t *C_host);
+int east_graph_index_dev(const east_index *idx, const uint32_t *kp_dev, const uint32_t *kp_host, const int64_t *kp_off,
+                         int32_t V, const int64_t *group_off, int32_t G, int normalized,
+                         const double *thresholds, int32_t n_thresholds,
+                         int32_t doc_begin, int32_t doc_count, int32_t *C_dev, void *stream);
 /* same table through an instrumented scorer that also counts the algorithmic bytes it reads:
  * 8 per (SA word, text word) probe (SURVEY 8(d)); on the fast path 5 per (SA word, text byte)
  * probe and 8 per 2-gram bucket lookup.  *probes receives that byte count. */
