@@ -1924,6 +1924,55 @@ int east_cooc_host(const double *S_DxK, int64_t D, int32_t K, double threshold, 
     EAST_API_END
 }
 
+// the graph assembled from the counts (graph_edges.cu); checked before the first CUDA call: the outputs, the counts, the nodes
+static void check_graph_edges(const int32_t *C, int32_t cols, int32_t n_planes, const int32_t *node_col, int32_t n_nodes,
+                              const int32_t *support_host, const int64_t *n_edges_host, int64_t edge_cap, const int32_t *src_host,
+                              const int32_t *dst_host, const double *conf_host) {
+    if (!support_host || !n_edges_host || edge_cap < 0 || (edge_cap > 0 && (!src_host || !dst_host || !conf_host)))
+        throw Error(EAST_ERR_INVALID, "bad output (supports, edge counts, or edge arrays for edge_cap entries)");
+    if (!C || cols < 1 || n_planes < 1 || n_planes > MAX_THRESHOLDS)
+        throw Error(EAST_ERR_INVALID, "bad counts: C must hold 1 to 8 planes of cols x cols, cols >= 1");
+    if (n_nodes < 0 || (n_nodes > 0 && !node_col)) throw Error(EAST_ERR_INVALID, "bad nodes");
+    for (int32_t n = 0; n < n_nodes; ++n)
+        if (node_col[n] < 0 || node_col[n] >= cols) throw Error(EAST_ERR_INVALID, "node column out of range");
+}
+
+static void graph_edges_call(const int32_t *C_dev, int32_t cols, int32_t n_planes, const int32_t *node_col, int32_t n_nodes,
+                             double referral_confidence, double support_threshold, cudaStream_t s, int32_t *support_host,
+                             int64_t *n_edges_host, int64_t edge_cap, int32_t *src_host, int32_t *dst_host, double *conf_host) {
+    const int64_t total = graph_edges(C_dev, cols, n_planes, node_col, n_nodes, referral_confidence, support_threshold, s,
+                                      support_host, n_edges_host, edge_cap, src_host, dst_host, conf_host);
+    ktime_collect();   // the stream is synchronized: fold the launches' event pairs into east_kernel_stats
+    if (total > edge_cap)
+        throw Error(EAST_ERR_RANGE, "edge_cap is too small: " + std::to_string(total) + " edges (n_edges_host holds them per plane)");
+}
+
+int east_graph_edges_dev(const int32_t *C_dev, int32_t cols, int32_t n_planes, const int32_t *node_col, int32_t n_nodes,
+                         double referral_confidence, double support_threshold, int device, void *stream, int32_t *support_host,
+                         int64_t *n_edges_host, int64_t edge_cap, int32_t *src_host, int32_t *dst_host, double *conf_host) {
+    EAST_API_BEGIN
+    check_graph_edges(C_dev, cols, n_planes, node_col, n_nodes, support_host, n_edges_host, edge_cap, src_host, dst_host, conf_host);
+    use_device(device);
+    graph_edges_call(C_dev, cols, n_planes, node_col, n_nodes, referral_confidence, support_threshold, (cudaStream_t)stream,
+                     support_host, n_edges_host, edge_cap, src_host, dst_host, conf_host);
+    EAST_API_END
+}
+
+int east_graph_edges_host(const int32_t *C_host, int32_t cols, int32_t n_planes, const int32_t *node_col, int32_t n_nodes,
+                          double referral_confidence, double support_threshold, int device, int32_t *support_host,
+                          int64_t *n_edges_host, int64_t edge_cap, int32_t *src_host, int32_t *dst_host, double *conf_host) {
+    EAST_API_BEGIN
+    check_graph_edges(C_host, cols, n_planes, node_col, n_nodes, support_host, n_edges_host, edge_cap, src_host, dst_host, conf_host);
+    use_device(device);
+    cudaStream_t s = 0;
+    const size_t cells = (size_t)n_planes * (size_t)cols * (size_t)cols;
+    DevBuf<int32_t> d_C(cells, s);
+    EAST_CUDA(cudaMemcpyAsync(d_C.p, C_host, sizeof(int32_t) * cells, cudaMemcpyHostToDevice, s));
+    graph_edges_call(d_C.p, cols, n_planes, node_col, n_nodes, referral_confidence, support_threshold, s, support_host,
+                     n_edges_host, edge_cap, src_host, dst_host, conf_host);
+    EAST_API_END
+}
+
 // ---- persistence --------------------------------------------------------------------------
 // One file per index (= one device batch of documents): header, then the arrays in a fixed order.  The reference
 // rebuilds every AST on every run (relevance.py:38-47); a saved index is loaded at PCIe speed instead.

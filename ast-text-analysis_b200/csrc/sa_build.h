@@ -240,4 +240,11 @@ void threshold_bytes(const double *S_DxK, int64_t D, int32_t K, const double *th
 // C = Bm Bm^T (K x K int32) from a prepared, zero-padded Kp x Dp matrix
 void cooc_counts_bytes(const uint8_t *Bm, int64_t Dp, int32_t Kp, int32_t K, int32_t *C, cudaStream_t s, int simple = 0);
 
+// the keyphrase graph of every plane of C (T x cols x cols int32, device) for nodes reading columns node_col_host[N]
+// (graph_edges.cu): supports to support_host[T][N], edges per plane to n_edges_host[T]; returns the number of edges of all
+// planes and writes them (src, dst: node positions; conf) to the host arrays only when it is <= edge_cap
+int64_t graph_edges(const int32_t *C, int64_t cols, int32_t T, const int32_t *node_col_host, int32_t N, double c, double p,
+                    cudaStream_t s, int32_t *support_host, int64_t *n_edges_host, int64_t edge_cap, int32_t *src_host,
+                    int32_t *dst_host, double *conf_host);
+
 }  // namespace east

@@ -20,6 +20,7 @@ SUFTAB, LCPTAB, CHILDTAB_UP, CHILDTAB_DOWN, CHILDTAB_NEXT_L_INDEX, ANNTAB, PACKE
 TEXT_DEVPTR = 100
 
 EAST_ERR_ZERODIV = -4
+EAST_ERR_RANGE = -5
 EAST_ERR_UNSUPPORTED = -6
 
 
@@ -37,7 +38,7 @@ EXPORTED_SYMBOLS = [
     "east_score_groups_host", "east_score_groups_dev",
     "east_table_groups_host", "east_table_groups_dev", "east_table_texts_groups_host",
     "east_graph_host", "east_graph_dev", "east_graph_texts_host",
-    "east_graph_index_host", "east_graph_index_dev",
+    "east_graph_index_host", "east_graph_index_dev", "east_graph_edges_host", "east_graph_edges_dev",
 ]
 
 _lib = None
@@ -112,6 +113,10 @@ def load():
                                         ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, _i32p]
     L.east_graph_index_dev.argtypes = [_vp, _vp, _u32p, _i64p, ctypes.c_int32, _i64p, ctypes.c_int32, ctypes.c_int, _f64p,
                                        ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, _vp, _vp]
+    L.east_graph_edges_dev.argtypes = [_vp, ctypes.c_int32, ctypes.c_int32, _i32p, ctypes.c_int32, ctypes.c_double,
+                                       ctypes.c_double, ctypes.c_int, _vp, _i32p, _i64p, ctypes.c_int64, _i32p, _i32p, _f64p]
+    L.east_graph_edges_host.argtypes = [_i32p, ctypes.c_int32, ctypes.c_int32, _i32p, ctypes.c_int32, ctypes.c_double,
+                                        ctypes.c_double, ctypes.c_int, _i32p, _i64p, ctypes.c_int64, _i32p, _i32p, _f64p]
     L.east_score_probes_dev.argtypes = [_vp, _vp, _i64p, ctypes.c_int32, _vp, _vp, _i64p]
     L.east_score_one.argtypes = [_vp, ctypes.c_int32, _u32p, ctypes.c_int32, ctypes.c_int, _f64p, _f64p]
     L.east_cooc_dev.argtypes = [_vp, ctypes.c_int64, ctypes.c_int32, ctypes.c_double, _vp, ctypes.c_int, _vp]
@@ -692,3 +697,40 @@ def cooc_host(S, threshold, device=0):
 def cooc_dev(S_devptr, D, K, threshold, C_devptr, device=0, stream=0):
     _check(load().east_cooc_dev(_vp(S_devptr), int(D), int(K), float(threshold), _vp(C_devptr), int(device),
                                 _vp(stream)))
+
+
+def graph_edges(C, node_col, referral_confidence, support_threshold):
+    """The keyphrase graphs of the co-occurrence counts C, assembled where C is (east_graph_edges_*): only the supports
+    and the edges come back.  C: int32 [K, K] or [T, K, K] (T <= 8 threshold planes), a numpy array (east_graph_edges_host)
+    or a CUDA torch tensor (east_graph_edges_dev on its device and current stream).  node_col: the column of every node
+    (a position in the caller's keyphrases).  Returns (int32 supports [T, N], int64 edges per plane [T], int32 src [E],
+    int32 dst [E], float64 confidence [E]): the edges of plane 0, then of plane 1, ..., each in row-major order over the
+    kept nodes.  When the first guess of the edge count is too small the call is repeated with the count it reports."""
+    L = load()
+    node_col = np.ascontiguousarray(node_col, dtype=np.int32)
+    N = len(node_col)
+    if isinstance(C, np.ndarray):
+        assert C.dtype == np.int32 and C.ndim in (2, 3)
+        C = np.ascontiguousarray(C)
+        entry, lead, tail = L.east_graph_edges_host, (_ptr(C, _i32p),), (0,)
+    else:
+        import torch
+        assert C.is_cuda and C.dtype == torch.int32 and C.dim() in (2, 3)
+        C = C.contiguous()
+        stream = torch.cuda.current_stream(C.device).cuda_stream
+        entry, lead, tail = L.east_graph_edges_dev, (_vp(C.data_ptr()),), (int(C.device.index), _vp(stream))
+    T, cols = (1 if C.ndim == 2 else int(C.shape[0])), int(C.shape[-1])
+    support = np.empty((T, max(N, 1)), dtype=np.int32)
+    n_edges = np.zeros(T, dtype=np.int64)
+    cap = 16 * max(N, 1) * T   # a sparse graph's edges; a denser one takes a second call with the exact count
+    while True:
+        src, dst = np.empty(max(cap, 1), dtype=np.int32), np.empty(max(cap, 1), dtype=np.int32)
+        conf = np.empty(max(cap, 1), dtype=np.float64)
+        rc = entry(*lead, cols, T, _ptr(node_col, _i32p) if N else None, N, float(referral_confidence), float(support_threshold),
+                   *tail, _ptr(support, _i32p), _ptr(n_edges, _i64p), cap, _ptr(src, _i32p), _ptr(dst, _i32p), _ptr(conf, _f64p))
+        total = int(n_edges.sum())
+        if rc == EAST_ERR_RANGE and total > cap:
+            cap = total
+            continue
+        _check(rc)
+        return support[:, :N], n_edges, src[:total], dst[:total], conf[:total]

@@ -87,13 +87,59 @@ def keyphrases_graph(keyphrases, texts, referral_confidence=0.6, relevance_thres
             cooc = similarity_measure.cooccurrence(prepared, relevance_threshold, synonimizer)
         else:
             cooc = np.zeros((len(kept), len(kept)), dtype=np.int32)
-        return graph_from_cooccurrence(keyphrases, kept, cooc, referral_confidence, relevance_threshold, support_threshold)
+        return graph_on_device(keyphrases, kept, cooc, referral_confidence, relevance_threshold, support_threshold)
     kept, titles, scores = _score_matrix(keyphrases, texts, similarity_measure, synonimizer, language)
     if scores.size:
         cooc = _capi.cooc_host(scores, relevance_threshold)
     else:
         cooc = np.zeros((len(kept), len(kept)), dtype=np.int32)
-    return graph_from_cooccurrence(keyphrases, kept, cooc, referral_confidence, relevance_threshold, support_threshold)
+    return graph_on_device(keyphrases, kept, cooc, referral_confidence, relevance_threshold, support_threshold)
+
+
+def graph_on_device(keyphrases, kept, cooc, referral_confidence, relevance_threshold, support_threshold):
+    """graph_from_cooccurrence assembled where the counts are (east_graph_edges_*): the same graph dict, and only the
+    supports and the edges come back from the device.  cooc: int32 [K, K], or [T, K, K] with T relevance thresholds
+    (relevance_threshold then a sequence of T: a list of T graphs comes back); a numpy array or a CUDA torch tensor.
+    The one difference from graph_from_cooccurrence: no node is paired with itself, whatever referral_confidence (the
+    host function pairs every node with itself at referral_confidence <= -1; the reference never does)."""
+    planes = np.ndim(relevance_threshold) != 0
+    thresholds = list(relevance_threshold) if planes else [relevance_threshold]
+    node_col = _node_columns(keyphrases, kept)
+    if len(keyphrases):
+        support, n_edges, src, dst, conf = _capi.graph_edges(cooc, node_col, referral_confidence, support_threshold)
+        bounds = np.concatenate([[0], np.cumsum(n_edges)]).tolist()
+    else:   # no node, nothing to count
+        support, bounds = np.zeros((len(thresholds), 0), dtype=np.int32), [0] * (len(thresholds) + 1)
+        src = dst = conf = np.zeros(0)
+    graphs = [graph_from_edges(keyphrases, support[t], src[bounds[t]:bounds[t + 1]], dst[bounds[t]:bounds[t + 1]],
+                               conf[bounds[t]:bounds[t + 1]], referral_confidence, r, support_threshold)
+              for t, r in enumerate(thresholds)]
+    return graphs if planes else graphs[0]
+
+
+def _node_columns(keyphrases, kept):
+    """the column of every keyphrase, as graph_from_cooccurrence picks it"""
+    column_of = {}
+    for k, kp in enumerate(kept):
+        column_of[kp] = k  # duplicate keyphrases share one table row (last wins, like a dict)
+    for kp in keyphrases:
+        if kp not in column_of:
+            raise KeyError(kp)  # the reference indexes table[keyphrase] for skipped empty keyphrases
+    return np.array([column_of[kp] for kp in keyphrases], dtype=np.int32)
+
+
+def graph_from_edges(keyphrases, support, src, dst, conf, referral_confidence, relevance_threshold, support_threshold):
+    """The graph dict of graph_from_cooccurrence from one plane of _capi.graph_edges: support[n] of every keyphrase,
+    the edges (node positions src -> dst, their confidences) in permutations order."""
+    support = support.tolist()
+    return {
+        "nodes": [{"id": i, "label": kp, "support": support[i]} for i, kp in enumerate(keyphrases)
+                  if support[i] >= support_threshold],
+        "edges": [{"source": s, "target": d, "confidence": c} for s, d, c in zip(src.tolist(), dst.tolist(), conf.tolist())],
+        "referral_confidence": referral_confidence,
+        "relevance_threshold": relevance_threshold,
+        "support_threshold": support_threshold,
+    }
 
 
 def graph_from_cooccurrence(keyphrases, kept, cooc, referral_confidence, relevance_threshold, support_threshold):

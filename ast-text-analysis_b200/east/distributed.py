@@ -17,7 +17,8 @@ join them:
 Graph.  Co-occurrence counts are additive over documents: every rank indexes its own documents and counts
 C_r = B_r B_r^T of their relevance bytes on the tensor cores (east_graph_dev: the scoring kernel writes the bytes, no
 score table is formed), and ONE all_reduce(int32 sum) of the K x K counts joins them (east/applications.py:111-147;
-SURVEY 5.8).  There is no other exchange on the path.
+SURVEY 5.8).  There is no other exchange on the path; every rank then assembles the graph from its copy of the counts on
+its GPU (east_graph_edges_dev), so the K x K counts never come to the host.
 """
 import numpy as np
 
@@ -273,5 +274,5 @@ def keyphrases_graph_sharded(keyphrases, texts, referral_confidence=0.6, relevan
                 cooc += part   # int32: exact
     if world > 1:
         dist.all_reduce(cooc, op=dist.ReduceOp.SUM, group=group)
-    return applications.graph_from_cooccurrence(keyphrases, kept, cooc.cpu().numpy(), referral_confidence,
-                                                relevance_threshold, support_threshold)
+    # the graph is assembled on the device from the all-reduced counts: only the supports and the edges come to the host
+    return applications.graph_on_device(keyphrases, kept, cooc, referral_confidence, relevance_threshold, support_threshold)

@@ -311,6 +311,16 @@ class ASTRelevanceMeasure(RelevanceMeasure):
             counts = part if counts is None else counts + part   # int32: exact (counts <= number of texts)
         return counts[0] if scalar else counts
 
+    def graphs(self, keyphrases, referral_confidence=0.6, relevance_thresholds=(0.25,), support_threshold=1, synonimizer=None):
+        """applications.keyphrases_graph of the indexed or loaded collection at 1 to 8 relevance thresholds: a list of
+        graph dicts, one per threshold.  The counts come from cooccurrence() (on a loaded index: one scoring pass for all
+        thresholds) and the graphs are assembled from them on the device (applications.graph_on_device)."""
+        from east import applications
+        kept = [kp for kp in keyphrases if kp]
+        thresholds = list(relevance_thresholds)
+        counts = self.cooccurrence([utils.prepare_text(kp) for kp in kept], thresholds, synonimizer)
+        return applications.graph_on_device(keyphrases, kept, counts, referral_confidence, thresholds, support_threshold)
+
     @staticmethod
     def _same_groups(groups, kept):
         return (groups is None) == (kept is None) and (groups is None or all(np.array_equal(a, b) for a, b in zip(groups, kept)))

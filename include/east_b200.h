@@ -207,6 +207,36 @@ int east_cooc_dev(const double *S_DxK_dev, int64_t D, int32_t K, double threshol
 int east_cooc_host(const double *S_DxK, int64_t D, int32_t K, double threshold,
                    int32_t *C_KxK, int device);
 
+/* ---- the keyphrase graph from the counts: replaces the graph assembly of applications.keyphrases_graph
+ * (applications.py:115-149) where the counts are, so that only O(nodes + edges) comes back instead of cols x cols.
+ *   C         : n_planes x cols x cols int32 counts, row-major (1 <= n_planes <= 8: the planes of east_graph_index_*, one
+ *               per relevance threshold); on the device for _dev, on the host for _host (staged through the library's
+ *               own device memory)
+ *   node_col  : host, n_nodes columns: node n (a position in the caller's keyphrases, duplicates included) reads column
+ *               node_col[n] of C
+ * Per plane t: support_host[t * n_nodes + n] = C[t][node_col[n]][node_col[n]]; node n is kept iff (double)support >=
+ * support_threshold (a NaN keeps nothing); kept nodes i1 != i2 -- positions, not columns: two kept nodes of one column
+ * are two nodes, confidence 1.0, or 0.0 at support 0 -- give the edge (i1, i2) iff conf = (double)C[t][col_i1][col_i2]
+ * / (double)max(support_i1, 1) (IEEE division) >= referral_confidence.  The edges of plane t come in row-major order
+ * over the kept positions (the reference's permutations order), after those of plane t - 1: src_host / dst_host hold
+ * node positions, conf_host the confidences; n_edges_host[t] counts plane t's.  A node is never paired with itself.
+ * Sizing: when the edges of all planes exceed edge_cap, the call fails with EAST_ERR_RANGE and support_host and
+ * n_edges_host are filled; a retry with edge_cap >= their sum succeeds (on device counts it costs one more count pass).
+ * edge_cap = 0 is a valid way to ask for the sizes; the edge arrays may then be NULL.
+ * Checked before the first CUDA call, in this order (EAST_ERR_INVALID): the outputs (support_host, n_edges_host,
+ * edge_cap >= 0, the edge arrays when edge_cap > 0); the counts (C, cols >= 1, 1 <= n_planes <= 8); the nodes
+ * (n_nodes >= 0, node_col, every node_col in [0, cols)).
+ *   east_graph_edges_dev: C_dev on `device`, queued on `stream`; returns when the host arrays are written.
+ *   east_graph_edges_host: C_host on the host. */
+int east_graph_edges_dev(const int32_t *C_dev, int32_t cols, int32_t n_planes, const int32_t *node_col, int32_t n_nodes,
+                         double referral_confidence, double support_threshold, int device, void *stream,
+                         int32_t *support_host, int64_t *n_edges_host, int64_t edge_cap, int32_t *src_host,
+                         int32_t *dst_host, double *conf_host);
+int east_graph_edges_host(const int32_t *C_host, int32_t cols, int32_t n_planes, const int32_t *node_col, int32_t n_nodes,
+                          double referral_confidence, double support_threshold, int device, int32_t *support_host,
+                          int64_t *n_edges_host, int64_t edge_cap, int32_t *src_host, int32_t *dst_host,
+                          double *conf_host);
+
 /* ---- measurement hooks (bench.py): per-stage device time of the last build/score call on
  * this thread, measured with CUDA events on the launching stream.
  * names: NUL-separated list written to buf; returns the number of stages. */
