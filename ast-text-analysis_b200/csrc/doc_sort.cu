@@ -31,10 +31,13 @@
 //      ties go to a byte-wise SWAR comparison of the shared-memory text (or to the position)
 //   7  LCP of neighbouring suffixes (SWAR on the staged text), 16-bit copy + min-pyramid in the freed scratch,
 //      per-rank key bytes for the scorer
-//   8  child table and annotation: every warp zero-fills the slices of its 32 chunks (phase 8 stores sparsely; filled
-//      right before they are walked the lines reach HBM once), per-thread chunks walked with the reference's stack
-//      discipline, what lies outside a chunk searched in the pyramid afterwards (farthest first, so that the lanes' long
-//      searches coincide)
+//   8  child table and annotation from PSE / NSV (previous smaller-or-equal, next smaller LCP value) in closed form: a
+//      warp takes tiles of 32 ranks, one lane per rank; bit-plane ballots resolve PSE and NSV inside the tile, the
+//      neighbouring tiles (in registers) or the min-pyramid (one ballot per level) the rest, one query at a time.  Every
+//      warp zero-fills up / down / next of its range right before its tiles store sparsely into it (the lines reach HBM
+//      once) and stores ann densely; stores into other warps' ranges are queued and made after a barrier.
+//      (EAST_DOC_SORT_STACK_WALK=1: per-thread chunks walked with the reference's stack discipline, what lies outside a
+//      chunk searched in the pyramid afterwards, farthest first)
 //   9  (optional: east_table_host / east_table_dev) score every distinct query suffix against the document
 //      (easa.py:91-139; walks of score_walk.cuh) from a copy of text + suffix array in the freed shared memory,
 //      then add the results up per keyphrase: the CTA writes its row of the score table (k_doc_suffix_sort_groups: the
@@ -80,7 +83,7 @@ struct DocSortParams {
     int text_cap;             // bytes reserved for the staged text
     int bits_words;           // words of the bucket-start bitmap
     int doc_begin;            // first document of this launch (CTA x sorts document doc_begin + x)
-    unsigned long long *phase_clk;  // optional (profiling): SM cycles per phase, summed over the CTAs
+    unsigned long long *phase_clk;  // optional (profiling, 17 counters): SM cycles per phase, summed over the CTAs; phase-8 counts
     // optional fused tables (all or none): LCP (easa.py:247-266), child table (:268-304), annotation (:306-331);
     // every entry of the documents of the launch is written (the kernel zero-fills what phase 8 does not set)
     int32_t *lcp, *up, *down, *next, *ann;
@@ -98,6 +101,7 @@ struct DocSortParams {
     const uint8_t *text8;
     uint32_t *text_out;
     int fill_early;           // tuning / A-B: zero-fill the child and annotation slices at the start of phase 7 (round 1)
+    int stack_walk;           // A-B / tests: phase 8 by per-thread stack walks over chunks (round 2) instead of tiles of 32 ranks
 };
 
 // 8 bytes of shared memory at an arbitrary byte offset from a 16-byte aligned base: three aligned
@@ -493,6 +497,52 @@ found:
     return j;
 }
 
+// The same two searches by a whole warp for the lane-per-rank path of phase 8 (level, idx and l uniform): every level,
+// on the way up and on the way down, is one coalesced load of 32 entries and one ballot instead of a scan by one lane.
+// They start above level 0 (the tile itself is resolved by the caller).  cnt (profiling, else nullptr): queries
+// counted by the level at which they found their block, cnt[levels] = not found.
+// largest q with lcp[q] <= l before entry idx of `level` (0 if none)
+__device__ __forceinline__ int ds_warp_prev_le(const SPyr &M, int level, int idx, uint32_t l, int lane, uint32_t *cnt) {
+    int j;
+    while (true) {
+        const int g0 = idx & ~31;
+        const uint32_t v = lane < (idx & 31) ? M.lv(level)[g0 + lane] : 0xffffffffu;
+        const uint32_t B = __ballot_sync(0xffffffffu, v <= l);
+        if (B) { j = g0 + 31 - __clz(B); break; }
+        idx >>= 5;
+        if (++level >= M.levels) { if (cnt && lane == 0) atomicAdd(&cnt[level], 1u); return 0; }
+    }
+    if (cnt && lane == 0) atomicAdd(&cnt[level], 1u);
+    while (level > 0) {   // the block holds such an entry: the last one of its 32 children that does
+        --level;
+        const int i = j * 32 + lane;
+        const uint32_t v = i < M.size(level) ? M.lv(level)[i] : 0xffffffffu;
+        j = j * 32 + 31 - __clz(__ballot_sync(0xffffffffu, v <= l));
+    }
+    return j;
+}
+
+// smallest e with lcp[e] < l after entry idx of `level`, or n
+__device__ __forceinline__ int ds_warp_next_lt(const SPyr &M, int level, int idx, uint32_t l, int n, int lane, uint32_t *cnt) {
+    int j;
+    while (true) {
+        const int g0 = idx & ~31, i = g0 + lane;
+        const uint32_t v = (lane > (idx & 31) && i < M.size(level)) ? M.lv(level)[i] : 0xffffffffu;
+        const uint32_t B = __ballot_sync(0xffffffffu, v < l);
+        if (B) { j = g0 + __ffs(B) - 1; break; }
+        idx >>= 5;
+        if (++level >= M.levels) { if (cnt && lane == 0) atomicAdd(&cnt[level], 1u); return n; }
+    }
+    if (cnt && lane == 0) atomicAdd(&cnt[level], 1u);
+    while (level > 0) {   // the first of the block's children that holds such an entry
+        --level;
+        const int i = j * 32 + lane;
+        const uint32_t v = i < M.size(level) ? M.lv(level)[i] : 0xffffffffu;
+        j = j * 32 + __ffs(__ballot_sync(0xffffffffu, v < l)) - 1;
+    }
+    return j;
+}
+
 // empty 2-gram / 3-gram bucket tables of a document the kernel gives up on
 __device__ __forceinline__ void ds_clear_tables(const DocSortParams &p, int doc, int b, int tid) {
     if (p.bkt) {
@@ -650,11 +700,11 @@ __device__ __forceinline__ void doc_suffix_sort(const DocSortParams &p) {
     const uint32_t term_bucket = p.term << ((G - 1) * b);   // the suffixes that ARE a terminator
     int32_t *sa_doc = p.sa + base;    // plain pointer: written and re-read by this CTA
 
-    long long t_prev = clock64();
+    uint32_t t_prev = (uint32_t)clock();   // 32 bits (one register for the whole kernel): a phase takes < 2^32 cycles
 #define DS_STAMP(k)                                                                     \
     do {                                                                                \
         if (p.phase_clk && tid == 0) {                                                  \
-            const long long t_now = clock64();                                          \
+            const uint32_t t_now = (uint32_t)clock();                                   \
             atomicAdd(&p.phase_clk[k], (unsigned long long)(t_now - t_prev));           \
             t_prev = t_now;                                                             \
         }                                                                               \
@@ -1080,6 +1130,9 @@ __device__ __forceinline__ void doc_suffix_sort(const DocSortParams &p) {
     __syncthreads();
     uint16_t *s_lcp = reinterpret_cast<uint16_t *>(s_scr);
     __shared__ int s_pyr_off[4], s_pyr_size[4], s_pyr_levels;
+    __shared__ uint32_t s_qcnt[7];   // profiling: phase-8 queries by the level that answers them (0: the neighbouring tile,
+                                     // 4: none), 5: tiles redone, 6: stores queued
+    if (tid < 7) s_qcnt[tid] = 0u;
     if (tid == 0) {
         int off = 0, sz = n, levels = 1;
         s_pyr_off[0] = 0; s_pyr_size[0] = n;
@@ -1150,7 +1203,125 @@ __device__ __forceinline__ void doc_suffix_sort(const DocSortParams &p) {
     }
     DS_STAMP(6);
 
-    // ---- phase 8: child table and annotation.  Thread t walks C consecutive ranks with the reference's
+    // ---- phase 8: child table and annotation in closed form (as in tables.cu): for rank r with l = lcp[r],
+    // q = PSE(r) = largest q < r with lcp[q] <= l, e = NSV(r) = smallest e > r with lcp[e] < l (or n).
+    // lcp[q] == l -> next[q] = r; else r is the first l-index of [q .. e-1]: ann[r] = e - q, up[e] = r if
+    // lcp[q] <= lcp[e], down[q] = r if lcp[e] <= lcp[q] (e inside the document); ann[0] = n - m (easa.py:329).
+    // Values are ranks local to the document, 0 = none.
+    // A warp takes a tile of 32 ranks, one lane per rank: bit-plane ballots give every lane the masks of the lanes with
+    // a smaller and with an equal LCP value, and from them PSE and NSV inside the tile.  What the tile does not resolve
+    // (its prefix and suffix minima) the whole warp answers one query at a time: first from the neighbouring tile (its
+    // LCP values are in registers: the warp walks its tiles in order and carries them), then from the min-pyramid,
+    // whose level 1 is the tiles' minima: one load and one ballot per level, up and down.  NSV is only searched for
+    // first l-indices.  Ranks past the end count as LCP 0, so that the first of them is NSV = n.
+    // The tiles of a warp are contiguous; the warp zero-fills up / down / next of its range right before its tiles store
+    // into it (the lines are still in L2 and reach HBM once), ann is stored for every rank.  A store into another warp's
+    // range would race with that warp's fill: such stores (only prefix and suffix minima of the warp's range have them,
+    // a handful per warp) are queued as (target, rank) in the warp's share of the free text area and made after a block
+    // barrier.  Should the queue be full, the tile is noted in a 64-bit mask and its outside stores are computed again
+    // after the barrier.  (EAST_DOC_SORT_STACK_WALK=1: the stack walk below; both measured in DESIGN section 4.)
+    if (!p.stack_walk) {
+        const int T = (n + 31) >> 5, TW = (T + DS_WARPS - 1) / DS_WARPS;   // T <= 2048: TW <= 64
+        const int t0 = min(T, warp * TW), t1 = min(T, t0 + TW);
+        const int w0 = 32 * t0, w1 = min(n, 32 * t1);
+        const int cap = p.text_cap / (4 * DS_WARPS);   // queue entries per warp: target << 16 | rank (both < 65 535)
+        uint32_t *const queue = reinterpret_cast<uint32_t *>(s_raw) + warp * cap;
+        int queued = 0;   // warp-uniform; > cap: the queue overflowed
+        if (!p.fill_early) {
+            for (int x = w0 + lane; x < w1; x += 32) { p.up[base + x] = 0; p.down[base + x] = 0; p.next[base + x] = 0; }
+            __syncwarp();
+        }
+        auto lcp_at = [&](int r) -> uint32_t { return r < n ? (uint32_t)s_lcp[r] : 0u; };
+        // tile t with the LCP values lp / l / ln of the tiles t - 1 / t / t + 1 (lp unused for t = 0: lane 0 has LCP 0).
+        // outside == false: every store inside [w0, w1), the others queued; returns whether the queue overflowed.
+        // outside == true: only the stores outside [w0, w1)
+        auto tile = [&](int t, uint32_t lp, uint32_t l, uint32_t ln, bool outside) -> bool {
+            const int r = 32 * t + lane;
+            const bool valid = r < n;
+            uint32_t lt = 0u, eq = 0xffffffffu;
+            const uint32_t mx = __reduce_max_sync(0xffffffffu, l);   // 16 bits at most (deep-LCP inputs reach 65 534)
+            for (int k = 31 - __clz(mx); k >= 0; --k) {
+                const bool bit = (l >> k) & 1u;
+                const uint32_t B = __ballot_sync(0xffffffffu, bit);
+                if (bit) { lt |= eq & ~B; eq &= B; } else eq &= ~B;
+            }
+            const uint32_t below = (1u << lane) - 1u, above = ~((2u << lane) - 1u);
+            const uint32_t pb = (lt | eq) & below;
+            int q = pb ? 32 * t + 31 - __clz(pb) : -1;
+            // PSE before the tile: the lanes smaller than every lane below them (strictly decreasing values)
+            uint32_t U = __ballot_sync(0xffffffffu, q < 0 && valid && r > 0);
+            while (U) {
+                const int x = __ffs(U) - 1;
+                U &= U - 1u;
+                const uint32_t lx = __shfl_sync(0xffffffffu, l, x);
+                const uint32_t B = __ballot_sync(0xffffffffu, lp <= lx);
+                int f;
+                if (B) { f = 32 * (t - 1) + 31 - __clz(B); if (p.phase_clk && lane == 0) atomicAdd(&s_qcnt[0], 1u); }
+                else f = ds_warp_prev_le(M, 1, t - 1, lx, lane, p.phase_clk ? s_qcnt : nullptr);
+                if (lane == x) q = f;
+            }
+            const bool inner = valid && r > 0;   // rank 0 has neither PSE nor NSV
+            const uint32_t lq = inner ? (uint32_t)s_lcp[q] : 0u;
+            const bool first = inner && lq != l;   // first l-index of [q .. e-1]
+            const uint32_t na = lt & above;
+            int e = na ? 32 * t + __ffs(na) - 1 : -1;
+            U = __ballot_sync(0xffffffffu, e < 0 && first);
+            while (U) {
+                const int x = __ffs(U) - 1;
+                U &= U - 1u;
+                const uint32_t lx = __shfl_sync(0xffffffffu, l, x);
+                const uint32_t B = __ballot_sync(0xffffffffu, ln < lx);   // lx > 0: a rank past the end stops it
+                int f;
+                if (B) { f = 32 * (t + 1) + __ffs(B) - 1; if (p.phase_clk && lane == 0) atomicAdd(&s_qcnt[0], 1u); }
+                else f = ds_warp_next_lt(M, 1, t + 1, lx, n, lane, p.phase_clk ? s_qcnt : nullptr);
+                if (lane == x) e = f;
+            }
+            bool dq = false, de = false;   // the store into down / next [q], into up[e] lies outside [w0, w1)
+            if (inner) {
+                if (!first) {
+                    dq = q < w0;
+                    if (dq == outside) p.next[base + q] = r;
+                } else if (e < n) {
+                    const uint32_t le = s_lcp[e];
+                    if (lq <= le) { de = e >= w1; if (de == outside) p.up[base + e] = r; }
+                    if (le <= lq) { dq = q < w0; if (dq == outside) p.down[base + q] = r; }
+                }
+            }
+            if (outside) return false;
+            if (valid) p.ann[base + r] = r == 0 ? n - p.doc_m[doc] : (first ? e - q : 0);
+            const uint32_t mq = __ballot_sync(0xffffffffu, dq), me = __ballot_sync(0xffffffffu, de);
+            if ((mq | me) == 0u) return false;
+            const int iq = queued + __popc(mq & below), ie = queued + __popc(mq) + __popc(me & below);
+            if (dq && iq < cap) queue[iq] = ((uint32_t)q << 16) | (uint32_t)r;
+            if (de && ie < cap) queue[ie] = ((uint32_t)e << 16) | (uint32_t)r;
+            queued += __popc(mq) + __popc(me);
+            return queued > cap;   // what did fit is stored twice: the same values
+        };
+        uint64_t redo = 0ull;
+        uint32_t lp = t0 > 0 ? lcp_at(32 * t0 - 32 + lane) : 0u, l = lcp_at(32 * t0 + lane);
+        for (int t = t0; t < t1; ++t) {
+            const uint32_t ln = lcp_at(32 * t + 32 + lane);
+            if (tile(t, lp, l, ln, false)) redo |= 1ull << (t - t0);
+            lp = l;
+            l = ln;
+        }
+        __syncthreads();   // every warp has filled its range: from here on the stores may land in other warps' ranges
+        DS_STAMP(7);
+        if (p.phase_clk && lane == 0) { atomicAdd(&s_qcnt[5], (uint32_t)__popcll(redo)); atomicAdd(&s_qcnt[6], (uint32_t)queued); }
+        for (int i = lane; i < min(queued, cap); i += 32) {
+            const uint32_t ent = queue[i];
+            const int x = (int)(ent >> 16), r = (int)(ent & 0xffffu);
+            if (x > r) p.up[base + x] = r;                          // NSV side
+            else if (s_lcp[x] == s_lcp[r]) p.next[base + x] = r;    // PSE side
+            else p.down[base + x] = r;
+        }
+        while (redo) {
+            const int t = t0 + __ffsll((long long)redo) - 1;
+            redo &= redo - 1ull;
+            tile(t, t > 0 ? lcp_at(32 * t - 32 + lane) : 0u, lcp_at(32 * t + lane), lcp_at(32 * t + 32 + lane), true);
+        }
+    } else
+    // ---- phase 8, stack walk (EAST_DOC_SORT_STACK_WALK=1).  Thread t walks C consecutive ranks with the reference's
     // own stack discipline (easa.py:268-331): the stack holds the ranks whose next smaller LCP value
     // has not been met yet, LCP values non-decreasing from bottom to top.  Pushing rank r: the top is
     // q = PSE(r) (largest q < r with lcp[q] <= lcp[r]); popping t because of r: r = NSV(t) (smallest
@@ -1271,6 +1442,7 @@ __device__ __forceinline__ void doc_suffix_sort(const DocSortParams &p) {
     }
     if (p.phase_clk) __syncthreads();
     DS_STAMP(8);
+    if (p.phase_clk && tid < 7) atomicAdd(&p.phase_clk[10 + tid], (unsigned long long)s_qcnt[tid]);
     ds_score_document<GROUPS, GRAPH>(p, ds_smem, p.text_cap + DS_SCR_BYTES + 4 * p.bits_words + 2 * (int)sizeof(uint2) * DS_LIST_CAP, doc, base, n, tid);
     if (p.phase_clk) __syncthreads();
     DS_STAMP(9);
@@ -1336,6 +1508,8 @@ void doc_sort_launch(const DocSortPlan &plan, const uint8_t *t8, const uint32_t 
     p.text8 = p.code_table ? text8 : nullptr; p.text_out = const_cast<uint32_t *>(text);
     static const bool fill_early = getenv("EAST_DOC_SORT_FILL_EARLY") != nullptr;
     p.fill_early = fill_early ? 1 : 0;
+    static const bool stack_walk = getenv("EAST_DOC_SORT_STACK_WALK") != nullptr;
+    p.stack_walk = stack_walk ? 1 : 0;
     p.lcp = p.up = p.down = p.next = p.ann = nullptr;
     if (tables && plan.tables_fit) { p.lcp = tables->lcp; p.up = tables->up; p.down = tables->down; p.next = tables->next; p.ann = tables->ann; }
     // algorithmic bytes per code point: 1 (byte text in) + 4 (suffix array out), with the fused tables + 5 x 4

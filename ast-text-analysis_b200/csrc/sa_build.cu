@@ -1412,8 +1412,8 @@ void build_suffix_array(const SaInput &in, SaOutput &out, StageTimer &tm, cudaSt
             static const bool profile = getenv("EAST_DOC_SORT_PROFILE") != nullptr;
             DevBuf<unsigned long long> clk;
             if (profile) {
-                clk = DevBuf<unsigned long long>(16, s);
-                EAST_CUDA(cudaMemsetAsync(clk.p, 0, 16 * sizeof(unsigned long long), s));
+                clk = DevBuf<unsigned long long>(17, s);
+                EAST_CUDA(cudaMemsetAsync(clk.p, 0, 17 * sizeof(unsigned long long), s));
             }
             DocSortTables tables{in.lcp, in.up, in.down, in.next, in.ann};
             const bool fuse = in.lcp != nullptr && plan.tables_fit;
@@ -1429,12 +1429,19 @@ void build_suffix_array(const SaInput &in, SaOutput &out, StageTimer &tm, cudaSt
             const uint32_t overflow = h_flag[0];
             const bool missed = sampled && h_flag[1] != 0u;   // the sampled alphabet lacks a code point of the text
             if (profile) {
-                unsigned long long h[16];
+                unsigned long long h[17];
                 EAST_CUDA(cudaMemcpy(h, clk.p, sizeof(h), cudaMemcpyDeviceToHost));
-                static const char *names[10] = {"load", "hist", "scan", "scatter", "refine", "windows", "lcp", "stack_walk", "beyond_chunk", "score"};
+                // phase 8: "child" = stack walk or tiles, "child_outside" = outside-chunk searches or redone tiles
+                static const char *names[10] = {"load", "hist", "scan", "scatter", "refine", "windows", "lcp", "child", "child_outside", "score"};
                 fprintf(stderr, "[east] doc_sort phases, kilo-cycles per document:");
                 for (int k = 0; k < 10; ++k) fprintf(stderr, " %s %.1f", names[k], (double)h[k] / D / 1e3);
                 fprintf(stderr, "\n");
+                // tile path of phase 8 only (zero for the stack walk): queries that leave their tile, by the pyramid level
+                // that answers them, the stores into other warps' ranges queued for after the barrier and the tiles redone
+                // because that queue was full
+                fprintf(stderr, "[east] doc_sort phase 8 per document: queries answered by the next tile %.1f, at level 1 %.1f, "
+                        "level 2 %.1f, level 3 %.1f, none %.1f; stores queued %.1f, tiles redone %.1f\n", (double)h[10] / D,
+                        (double)h[11] / D, (double)h[12] / D, (double)h[13] / D, (double)h[14] / D, (double)h[16] / D, (double)h[15] / D);
             }
             if (missed) {
                 // nothing of this pass is kept: the same build with the alphabet of the whole text

@@ -148,7 +148,7 @@ bool doc_sort_plan(int sigma, int32_t max_doc_n, DocSortPlan &plan);
 void doc_sort_launch(const DocSortPlan &plan, const uint8_t *t8, const uint32_t *text, const int32_t *doc_off,
                      const int32_t *doc_m, int doc_begin, int n_docs,
                      int64_t n_total /* code points of these documents */, uint32_t term, int32_t *sa, uint32_t *bkt, uint32_t *bkt3, uint32_t *overflow, cudaStream_t s,
-                     unsigned long long *phase_clk = nullptr /* profiling: 8 cycle counters */,
+                     unsigned long long *phase_clk = nullptr /* profiling: 17 counters */,
                      const DocSortTables *tables = nullptr /* also produce LCP, child table, annotation */,
                      uint32_t *sk = nullptr /* also produce the scorer's per-rank key bytes */,
                      const DocScore *score = nullptr /* also score keyphrases (needs bkt and sk) */,
